@@ -19,7 +19,9 @@ concatenates blocks in order.  A "step" encodes every block of the rank's shard 
 from __future__ import annotations
 
 import argparse
+import atexit
 import ctypes as C
+import functools
 import json
 import lzma
 import os
@@ -44,10 +46,16 @@ METRIC = "TSV->ZDW encode GB/s (decode GB/s alongside) on synthetic analytics-hi
 
 
 # --------------------------------------------------------------------------------------- generator
+@functools.lru_cache(maxsize=1)
 def _build_synth() -> Path:
+    """The generator library: tools/libsynth_gen.so when it is up to date, else compiled once per process into a
+    temporary directory that is removed at exit (the tree may be read-only)."""
     so = ROOT / "tools" / "libsynth_gen.so"
     src = ROOT / "tools" / "synth_gen.c"
     if not so.exists() or so.stat().st_mtime < src.stat().st_mtime:
+        tmp = tempfile.mkdtemp(prefix="zdwsynth_")
+        atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+        so = Path(tmp) / "libsynth_gen.so"
         subprocess.run(["gcc", "-O2", "-fPIC", "-shared", "-o", str(so), str(src)], check=True)
     return so
 
@@ -435,6 +443,57 @@ def bind_to_gpu_node(torch, index: int):
         return f"unchanged ({type(ex).__name__})"
 
 
+DUMP_ELEMENTS = 15 << 20  # float32 samples over all dumped arrays: 60 MiB
+
+
+class _DeviceBytes:
+    """n bytes at a device address, for torch.as_tensor (no copy, no stream synchronisation)."""
+
+    def __init__(self, ptr: int, n: int):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "|u1", "data": (ptr, False), "version": 3, "stream": None}
+
+
+class OutputSampler:
+    """--dump-outputs.  Before the timed steps: seeded positions into every block's result (from its length in the untimed
+    pass) and a buffer for the bytes there, both on the device.  In the last timed step: each call enqueues one gather
+    of those positions on its lane's stream, before the lane's next call reuses the result buffer.  After the timed
+    steps: the samples go to the host and into DIR/<name>.npy (float32), the per-block numbers into <name>_blocks.npy."""
+
+    def __init__(self, torch, dev, block_ids, lengths: dict, per_block: int):
+        self.torch, self.dev, self.block_ids, self.per_block = torch, dev, block_ids, per_block
+        self.lengths = {name: list(ns) for name, ns in lengths.items()}
+        self.idx = {name: [self._positions(name, j, n) for j, n in enumerate(ns)] for name, ns in lengths.items()}
+        self.buf = {name: [torch.empty(len(i), dtype=torch.uint8, device=dev) for i in idx] for name, idx in self.idx.items()}
+        self.numbers = {name: [None] * len(ns) for name, ns in lengths.items()}
+
+    def _positions(self, name: str, j: int, n: int):
+        import numpy as np
+        if n <= self.per_block:
+            idx = np.arange(n)
+        else:
+            seed = [SEED, self.block_ids[j], sorted(self.lengths).index(name)]
+            idx = np.sort(np.random.default_rng(seed).integers(0, n, self.per_block))
+        return self.torch.from_numpy(idx).to(self.dev)
+
+    def take(self, stream, name: str, j: int, ptr: int, n: int, numbers):
+        torch = self.torch
+        self.numbers[name][j] = numbers
+        if n != self.lengths[name][j]:  # a result longer or shorter than in the untimed pass: positions drawn here
+            self.lengths[name][j] = n
+            self.idx[name][j] = self._positions(name, j, n)
+            self.buf[name][j] = torch.empty(len(self.idx[name][j]), dtype=torch.uint8, device=self.dev)
+        view = torch.as_tensor(_DeviceBytes(ptr, n), device=self.dev)
+        with torch.cuda.stream(stream):
+            torch.index_select(view, 0, self.idx[name][j], out=self.buf[name][j])
+
+    def write(self, out_dir: str, prefix: str):
+        import numpy as np
+        os.makedirs(out_dir, exist_ok=True)
+        for name, bufs in self.buf.items():
+            np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), np.concatenate([b.cpu().numpy() for b in bufs]).astype(np.float32))
+            np.save(os.path.join(out_dir, f"{prefix}{name}_blocks.npy"), np.array(self.numbers[name], dtype=np.float64))
+
+
 def run_cuda(args):
     import torch
 
@@ -546,11 +605,29 @@ def run_cuda(args):
     enc_items = list(zip(dev_tsv, host_lens))
     dec_items = list(zip(dev_zdw, zdw_lens))
 
-    def encode_pass():
-        _res_pass(lambda c, it: c.encode_block(types, it[0].data_ptr(), it[1], input_on_device=True, output_on_device=True), enc_items)
+    # --dump-outputs: the samples of all ranks together stay within DUMP_ELEMENTS
+    sampler_out = None
+    if args.dump_outputs:
+        sampler_out = OutputSampler(torch, dev, my_blocks, {"encode_zdw": zdw_lens, "decode_tsv": host_lens},
+                                    DUMP_ELEMENTS // 2 // max(1, nb))
+        torch.cuda.synchronize(dev)
+    lane_stream = {id(c): s for c, s in zip(res_lanes, res_streams)}
 
-    def decode_pass():
-        _res_pass(lambda c, it: c.decode_block(types, it[0].data_ptr(), it[1], input_on_device=True, output_on_device=True), dec_items)
+    def encode_pass(sample=None):
+        def one(c, j):
+            t, n = enc_items[j]
+            blk = c.encode_block(types, t.data_ptr(), n, input_on_device=True, output_on_device=True)
+            if sample is not None:
+                sample.take(lane_stream[id(c)], "encode_zdw", j, blk.dev_ptr, blk.length, (blk.length, blk.nrows, blk.longest_line))
+        _res_pass(one, range(len(enc_items)))
+
+    def decode_pass(sample=None):
+        def one(c, j):
+            z, n = dec_items[j]
+            d = c.decode_block(types, z.data_ptr(), n, input_on_device=True, output_on_device=True)
+            if sample is not None:
+                sample.take(lane_stream[id(c)], "decode_tsv", j, d.dev_ptr, d.length, (d.length, d.nrows, d.line_length))
+        _res_pass(one, range(len(dec_items)))
 
     def barrier():
         if world > 1:
@@ -636,11 +713,12 @@ def run_cuda(args):
     barrier()
     t_wall0 = time.perf_counter()
     t_epoch0 = time.time()
-    for _ in range(args.steps):
+    for step in range(args.steps):
+        sample = sampler_out if step == args.steps - 1 else None
         ev[0].record(stream)
-        encode_pass()
+        encode_pass(sample)
         ev[1].record(stream)
-        decode_pass()
+        decode_pass(sample)
         ev[2].record(stream)
         ev[2].synchronize()
         enc_ms.append(ev[0].elapsed_time(ev[1]))
@@ -649,6 +727,8 @@ def run_cuda(args):
     t_wall = time.perf_counter() - t_wall0
     launches = sum(c.kernel_launches() for c in res_lanes) - launches0
     clocks = sampler.stop(t_epoch0, time.time())
+    if sampler_out is not None:
+        sampler_out.write(args.dump_outputs, f"rank{rank}_" if world > 1 else "")
 
     # ---- end to end through the C ABI with HOST buffers (H2D + kernels + D2H inside the timed region).  Blocks are
     # independent, so E2E_LANES contexts (one host thread + stream each) work on different blocks at the same time: the
@@ -816,6 +896,7 @@ def run_cuda(args):
                     "decode_value": e2e_dec_tsv / t_e2e_dec / 1e9, "decode_blocks_timed": len(e2e_dec_items), "pinned_decode_input": bool(dec_pinned) and not dec_keep,
                     "decode_d2h_bytes": int(d2h_dec_all)},
             "gpu_launches": int(launches_all),
+            "dump_outputs": args.dump_outputs,
             "parity": parity,
             "clocks": clocks,
             "tsv_bytes": int(tot_tsv), "zdw_bytes": int(tot_zdw),
@@ -933,6 +1014,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C2 / C3 / C5 timings of the N=1 line")
     ap.add_argument("--no-parity", action="store_true", help="skip the comparison with oracle/_ref (diagnostic runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/*.npy: a seeded sample of every block's ZDW bytes "
+                         "and decoded TSV bytes (float32, %d MiB in all) and per block its length, rows and longest "
+                         "line (float64); the timed calls only enqueue a gather of positions drawn beforehand" % (DUMP_ELEMENTS * 4 >> 20))
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "cuda":
         args.warmup = 3

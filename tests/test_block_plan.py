@@ -6,6 +6,8 @@ all it takes to reproduce such a file: the oracle restatement takes them as an e
 the plan from a file the compiled reference cut on its own (--mem-limit) and checks that the restatement then writes
 the same bytes.  The GPU twin of this test (test_gpu_encode.py) holds the CUDA encoder to the same files."""
 import functools
+import hashlib
+import json
 import os
 import subprocess
 import tempfile
@@ -16,7 +18,7 @@ import c5_check
 import corpus
 import oracle as O
 
-pytestmark = pytest.mark.skipif(not O.have_ref(), reason="compiled reference (oracle/_ref) not available")
+needs_ref = pytest.mark.skipif(not O.have_ref(), reason="compiled reference (oracle/_ref) not available")
 
 
 @functools.lru_cache(maxsize=2)
@@ -31,6 +33,18 @@ def reference_mem_limit_file(rows: int, mem_limit_mb: int):
                            capture_output=True, timeout=600)
         assert p.returncode == 0, p.stderr[-500:]
         return tsv, open(os.path.join(d, "x.zdw.gz"), "rb").read()
+
+
+@functools.lru_cache(maxsize=1)
+def memory_cut_file():
+    """(tsv, image): the rows of tests/golden/memory_cut.json and the file the restatement writes for them with the cut
+    kept there (its heap-block model at K = 2, the reference's cut under --mem-limit=140: test_stored_cut_is_the_references),
+    checked against the stored SHA-256."""
+    cut = json.loads((O.GOLDEN / "memory_cut.json").read_text())
+    tsv = c5_check.make_rows(cut["rows"])
+    image = O.encode(O.parse_desc(c5_check.DESC), tsv, plan=[tuple(b) for b in cut["plan"]]).data
+    assert hashlib.sha256(image).hexdigest() == cut["sha256"]
+    return tsv, image
 
 
 def recover_plan(sch, tsv: bytes, image: bytes):
@@ -51,6 +65,12 @@ def recover_plan(sch, tsv: bytes, image: bytes):
     return plan
 
 
+@needs_ref
+def test_stored_cut_is_the_references():
+    assert memory_cut_file() == reference_mem_limit_file(600_000, 140)
+
+
+@needs_ref
 def test_restatement_reproduces_a_memory_cut_file():
     sch = O.parse_desc(c5_check.DESC)
     tsv, image = reference_mem_limit_file(600_000, 140)
@@ -62,6 +82,7 @@ def test_restatement_reproduces_a_memory_cut_file():
     assert ref.tsv == tsv
 
 
+@needs_ref
 def test_heap_block_model_places_the_references_cut():
     """SURVEY 8f-1 / App. B-14: where the reference cuts a file is a function of the input and ONE number - the
     string-heap allocation at which its process is found over --mem-limit.  The restatement packs new strings into

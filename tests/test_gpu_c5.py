@@ -30,12 +30,13 @@ def test_c5_decode_through_unconvert_api(tmp_path):
     tsv = c5_check.make_rows(50000)
     z = O.encode(O.parse_desc(c5_check.DESC), tsv, rows_per_block=20000).data  # three blocks
     (tmp_path / "c5.zdw").write_bytes(z)
-    outs = []
-    for tool in (ROOT / "zdw_b200" / "bin" / "test_unconvert_api", ROOT / "oracle" / "_ref" / "test_unconvert_api"):
-        p = subprocess.run([str(tool), "c5.zdw"], cwd=tmp_path, capture_output=True, timeout=300)
-        assert p.returncode == 0, p.stderr[-500:]
-        outs.append(p.stdout)
-    assert outs[0] == outs[1] == tsv
+    import recorded_runs as RR
+    p = subprocess.run([str(ROOT / "zdw_b200" / "bin" / "test_unconvert_api"), "c5.zdw"], cwd=tmp_path, capture_output=True,
+                       timeout=300)
+    assert p.returncode == 0, p.stderr[-500:]
+    rc, ref_out, ref_err, _ = RR.run("test_unconvert_api", ["c5.zdw"], tmp_path)
+    assert rc == 0, ref_err
+    assert p.stdout == ref_out == tsv
 
 
 @pytest.mark.gpu
@@ -71,9 +72,12 @@ def test_api_rowloop_twins_agree_on_goldens(tmp_path, name):
     sys.path.insert(0, str(ROOT / "tests"))
     import oracle as O
     (tmp_path / "g.zdw").write_bytes(O.golden(f"{name}.zdw"))
+    import recorded_runs as RR
+    p = subprocess.run([str(ROOT / "zdw_b200" / "bin" / "api_rowloop"), "--checksum", "g.zdw"], cwd=tmp_path,
+                       capture_output=True, timeout=300)
+    rc, ref_out, ref_err, _ = RR.run("api_rowloop", ["--checksum", "g.zdw"], tmp_path)
     res = []
-    for tool in (ROOT / "zdw_b200" / "bin" / "api_rowloop", ROOT / "oracle" / "_ref" / "api_rowloop"):
-        p = subprocess.run([str(tool), "--checksum", "g.zdw"], cwd=tmp_path, capture_output=True, text=True, timeout=300)
-        assert p.returncode == 0, p.stderr[-500:]
-        res.append(json.loads(p.stdout.strip().splitlines()[-1]))
+    for code, out, err in ((p.returncode, p.stdout, p.stderr), (rc, ref_out, ref_err)):
+        assert code == 0, err[-500:]
+        res.append(json.loads(out.decode().strip().splitlines()[-1]))
     assert (res[0]["rows"], res[0]["tsv_bytes"], res[0]["fnv1a"]) == (res[1]["rows"], res[1]["tsv_bytes"], res[1]["fnv1a"])

@@ -157,13 +157,12 @@ def test_explicit_block_plan_with_spill(ctx, plan):
 
 def test_reproduces_a_file_the_reference_cut_on_its_own(ctx):
     """The compiled reference splits a dictionary-heavy input when it runs low on memory (--mem-limit); with the block
-    plan recovered from its output the CUDA encoder writes the same bytes, spilled strings included."""
+    plan recovered from that file (test_block_plan.memory_cut_file: the restatement's file for the reference's cut) the
+    CUDA encoder writes the same bytes, spilled strings included."""
     import c5_check
     import test_block_plan as BP
-    if not O.have_ref():
-        pytest.skip("compiled reference (oracle/_ref) not available")
     sch = O.parse_desc(c5_check.DESC)
-    tsv, image = BP.reference_mem_limit_file(600_000, 140)
+    tsv, image = BP.memory_cut_file()
     plan = BP.recover_plan(sch, tsv, image)
     assert plan and any(spill for _, spill in plan)
     got = G.encode_file_with_product(ctx, sch, tsv, plan=plan)

@@ -1,5 +1,6 @@
-"""Host layer (zdw_b200/host): the reference-shaped CLIs and C++ API, differential against the compiled reference
-(oracle/_ref) run on the same inputs with the same flags.  The `gpu` tests exercise the CUDA path end to end through
+"""Host layer (zdw_b200/host): the reference-shaped CLIs and C++ API, differential on the same inputs with the same
+flags against recorded runs (recorded_runs.py: written against the compiled reference, replayed from a snapshot of
+this project's tools where the reference is not built).  The `gpu` tests exercise the CUDA path end to end through
 the binaries; the others cover what needs no device (help text, .desc.sql emission, loud failure without a GPU)."""
 import os
 import shutil
@@ -11,23 +12,22 @@ import pytest
 
 import corpus
 import oracle as O
+import recorded_runs as RR
 
 ROOT = Path(__file__).resolve().parent.parent
 BIN = ROOT / "zdw_b200" / "bin"
-REF = ROOT / "oracle" / "_ref"
 
 pytestmark = pytest.mark.skipif(not (BIN / "convertDWfile").exists(), reason="host binaries not built (run __graft_entry__.build())")
 
 
-def _env():
-    env = dict(os.environ)
-    env["PATH"] = f"{REF / 'nocomp'}:{env.get('PATH', '')}"  # gzip/zcat pass-through: compressor stage out of scope
-    return env
-
-
 def run(tool_dir: Path, tool: str, args, cwd, stdin: bytes | None = None, timeout=300):
-    p = subprocess.run([str(tool_dir / tool), *args], cwd=cwd, env=_env(), input=stdin, capture_output=True, timeout=timeout)
+    p = subprocess.run([str(tool_dir / tool), *args], cwd=cwd, env=RR.env(), input=stdin, capture_output=True, timeout=timeout)
     return p.returncode, p.stdout, p.stderr
+
+
+def ours(tool: str, args, cwd, stdin: bytes | None = None, timeout=300):
+    """-> (exit code, stdout, stderr, {path under cwd: bytes}) like reference_runs.run"""
+    return (*run(BIN, tool, args, cwd, stdin, timeout), RR.files_under(cwd))
 
 
 class Work:
@@ -39,56 +39,67 @@ class Work:
         shutil.rmtree(self.d, ignore_errors=True)
 
 
-def encode_both(tsv: bytes, desc: bytes, args=(), metadata: bytes | None = None):
-    """-> ((rc, zdw, out) ours, (rc, zdw, out) reference)"""
+def encode_both(tsv: bytes, desc: bytes, args=(), metadata: bytes | None = None, runners=(ours, RR.run)):
+    """-> ((rc, zdw, out, files) ours, (rc, zdw, out, files) recorded)"""
     res = []
-    for tool_dir in (BIN, REF):
+    for runner in runners:
         with Work() as d:
             (d / "x.sql").write_bytes(tsv)
             (d / "x.desc.sql").write_bytes(desc)
             if metadata is not None:
                 (d / "x.metadata").write_bytes(metadata)
-            rc, out, err = run(tool_dir, "convertDWfile", [*args, "x.sql"], d)
-            f = d / "x.zdw.gz"
-            res.append((rc, f.read_bytes() if f.exists() else None, (out + err).decode("latin1"),
-                        sorted(p.name for p in d.iterdir())))
+            rc, out, err, files = runner("convertDWfile", [*args, "x.sql"], d)
+            res.append((rc, files.get("x.zdw.gz"), (out + err).decode("latin1"), sorted(files)))
     return res
 
 
-def decode_both(zdw: bytes, args=(), name="x.zdw"):
+def decode_both(zdw: bytes, args=(), name="x.zdw", runners=(ours, RR.run)):
     res = []
-    for tool_dir in (BIN, REF):
+    for runner in runners:
         with Work() as d:
             (d / name).write_bytes(zdw)
-            rc, out, err = run(tool_dir, "unconvertDWfile", [*args, name], d)
-            files = {p.name: p.read_bytes() for p in d.iterdir() if p.name != name}
+            rc, out, err, files = runner("unconvertDWfile", [*args, name], d)
+            files.pop(name, None)
             res.append((rc, out, err.decode("latin1"), files))
     return res
 
 
+def encode_ours(*a, **k):
+    """encode_both for our tool alone (flags of this build, which the reference does not know)"""
+    return encode_both(*a, runners=(ours,), **k)[0]
+
+
+def decode_ours(*a, **k):
+    return decode_both(*a, runners=(ours,), **k)[0]
+
+
+def decode_recorded(*a, **k):
+    return decode_both(*a, runners=(RR.run,), **k)[0]
+
+
 # ------------------------------------------------------------------------------------------------ no GPU needed
 def test_help_text_matches_reference_except_additions():
-    for tool in ("convertDWfile", "unconvertDWfile"):
-        ours = subprocess.run([str(BIN / tool), "--help"], capture_output=True).stdout.decode()
-        ref = subprocess.run([str(REF / tool), "--help"], capture_output=True).stdout.decode()
-        kept = [ln for ln in ours.splitlines() if "(B200 build)" not in ln]
-        # the additions are listed in one extra paragraph of the encoder help
-        assert [ln for ln in kept if ln.strip()] == [ln for ln in ref.splitlines() if ln.strip()]
-    assert subprocess.run([str(BIN / "convertDWfile"), "--version"], capture_output=True).stdout == \
-        subprocess.run([str(REF / "convertDWfile"), "--version"], capture_output=True).stdout
+    with Work() as d:
+        for tool in ("convertDWfile", "unconvertDWfile"):
+            mine = run(BIN, tool, ["--help"], d)[1].decode()
+            ref = RR.run(tool, ["--help"], d)[1].decode()
+            kept = [ln for ln in mine.splitlines() if "(B200 build)" not in ln]
+            # the additions are listed in one extra paragraph of the encoder help
+            assert [ln for ln in kept if ln.strip()] == [ln for ln in ref.splitlines() if ln.strip() and "(B200 build)" not in ln]
+        assert run(BIN, "convertDWfile", ["--version"], d)[1] == RR.run("convertDWfile", ["--version"], d)[1]
 
 
 def test_cli_argument_errors_match_reference():
-    with Work() as d:
-        for tool, args in (("convertDWfile", ["--bogus"]), ("convertDWfile", ["-q"]), ("convertDWfile", ["-d"]),
-                           ("unconvertDWfile", ["-x", "f"]), ("unconvertDWfile", ["-c"]), ("unconvertDWfile", ["-qq", "f"]),
-                           ("unconvertDWfile", ["-c", "a", "-ci", "b", "f"]), ("unconvertDWfile", ["-o", "--metadata", "f"]),
-                           ("unconvertDWfile", ["--metadata-values=a,a", "f"]), ("unconvertDWfile", ["nonexistent.zdw"])):
+    for tool, args in (("convertDWfile", ["--bogus"]), ("convertDWfile", ["-q"]), ("convertDWfile", ["-d"]),
+                       ("unconvertDWfile", ["-x", "f"]), ("unconvertDWfile", ["-c"]), ("unconvertDWfile", ["-qq", "f"]),
+                       ("unconvertDWfile", ["-c", "a", "-ci", "b", "f"]), ("unconvertDWfile", ["-o", "--metadata", "f"]),
+                       ("unconvertDWfile", ["--metadata-values=a,a", "f"]), ("unconvertDWfile", ["nonexistent.zdw"])):
+        with Work() as d:  # each run in a directory of its own: nothing left by one run keys or changes the other
             a = run(BIN, tool, args, d)
-            b = run(REF, tool, args, d)
-            assert a[0] == b[0], (tool, args, a, b)
-            norm = lambda s, td: s.replace(str(td).encode(), b"BIN")
-            assert norm(a[2], BIN) == norm(b[2], REF), (tool, args)
+        with Work() as d:
+            b = RR.run(tool, args, d)
+        assert a[0] == b[0], (tool, args, a, b)
+        assert a[2].replace(str(BIN).encode(), RR.TOOL_DIR) == b[2], (tool, args)
 
 
 def test_desc_only_needs_no_gpu_and_matches_reference():
@@ -102,15 +113,20 @@ def test_desc_only_needs_no_gpu_and_matches_reference():
 
 
 def test_missing_files_and_desc_errors_match_reference():
-    with Work() as d:
-        (d / "a.sql").write_bytes(b"1\t2\n")
-        for args in (["a.sql"], ["a.txt"], ["nofile.sql"]):
-            a, b = run(BIN, "convertDWfile", args, d), run(REF, "convertDWfile", args, d)
-            assert a[0] == b[0] == 2
-            assert a[2].split(b"\n")[-2] == b[2].split(b"\n")[-2]
-        (d / "a.desc.sql").write_bytes(b"col_without_type\n")
-        a, b = run(BIN, "convertDWfile", ["a.sql"], d), run(REF, "convertDWfile", ["a.sql"], d)
-        assert a[0] == b[0] == 2 and b"DESC_FILE_MISSING_TYPE_INFO" in a[2]
+    def both(args, files):
+        res = []
+        for runner in (ours, RR.run):
+            with Work() as d:  # each run in a directory of its own, holding only the inputs
+                for name, data in files.items():
+                    (d / name).write_bytes(data)
+                res.append(runner("convertDWfile", args, d))
+        return res
+    for args in (["a.sql"], ["a.txt"], ["nofile.sql"]):
+        a, b = both(args, {"a.sql": b"1\t2\n"})
+        assert a[0] == b[0] == 2
+        assert a[2].split(b"\n")[-2] == b[2].split(b"\n")[-2]
+    a, b = both(["a.sql"], {"a.sql": b"1\t2\n", "a.desc.sql": b"col_without_type\n"})
+    assert a[0] == b[0] == 2 and b"DESC_FILE_MISSING_TYPE_INFO" in a[2]
 
 
 def _gpu_present():
@@ -168,7 +184,7 @@ def test_metadata_sources_and_precedence():
     assert ours[0] == ref[0] == 2 and ours[1] is None
     ours, ref = encode_both(tsv, desc, [], b"no equals sign\n")
     assert ours[0] == ref[0] == 2
-    z = encode_both(tsv, desc, ["--metadata:b=2", "--metadata:a=1"])[0][1]
+    z = encode_ours(tsv, desc, ["--metadata:b=2", "--metadata:a=1"])[1]
     for args in (["--metadata", "-"], ["--metadata", "--metadata-keys", "-"], ["--metadata", "--metadata-values=a", "-"],
                  ["--metadata", "--metadata-values=zz", "-"], ["--metadata", "--metadata-values-allow-missing=zz,a", "-"], []):
         a, b = decode_both(z, ["-q", *args])
@@ -178,7 +194,7 @@ def test_metadata_sources_and_precedence():
 @pytest.mark.gpu
 def test_streaming_stdin_encode_matches_file_mode():
     tsv, desc = O.golden("test.sql") * 50, O.golden("test.desc.sql")
-    want = encode_both(tsv, desc)[0][1]
+    want = encode_ours(tsv, desc)[1]
     with Work() as d:
         (d / "x.desc.sql").write_bytes(desc)
         rc, out, err = run(BIN, "convertDWfile", ["-i", "-v", "x.sql"], d, stdin=tsv)
@@ -224,20 +240,20 @@ def test_decode_column_selection_and_virtual_columns():
 @pytest.mark.gpu
 def test_decode_stdin_and_output_dir():
     z = O.golden_to_v11(O.golden("test.zdw"))
-    for tool_dir in (BIN, REF):
+    for runner in (ours, RR.run):
         with Work() as d:
             (d / "o").mkdir()
-            rc, out, err = run(tool_dir, "unconvertDWfile", ["-q", "-i"], d, stdin=z)
+            rc, out, err, files = runner("unconvertDWfile", ["-q", "-i"], d, stdin=z)
             assert rc == 0 and out == O.golden("test.sql")
-            rc, out, err = run(tool_dir, "unconvertDWfile", ["-q", "-i", "-d", "o/", "named"], d, stdin=z)
-            assert rc == 0 and (d / "o" / "named.sql").read_bytes() == O.golden("test.sql")
-            assert (d / "o" / "named.desc.sql").exists()
+            rc, out, err, files = runner("unconvertDWfile", ["-q", "-i", "-d", "o/", "named"], d, stdin=z)
+            assert rc == 0 and files["o/named.sql"] == O.golden("test.sql")
+            assert "o/named.desc.sql" in files
 
 
 @pytest.mark.gpu
 def test_multi_block_files_and_statistics():
     tsv, desc = O.golden("movie_tickets.sql"), O.golden("movie_tickets.desc.sql")
-    ours = encode_both(tsv, desc, ["--rows-per-block=100000"])[0]
+    ours = encode_ours(tsv, desc, ["--rows-per-block=100000"])
     assert ours[0] == 0 and "block 6 of" in ours[2]
     z = ours[1]
     want = O.encode(O.parse_desc(desc), tsv, rows_per_block=100000)
@@ -250,7 +266,7 @@ def test_multi_block_files_and_statistics():
     assert a[0] == b[0] == 0
     a, b = decode_both(z, ["-q", "-c", "virtual_export_row", "-"])
     assert a[1] == b[1]                            # row numbers run on across blocks
-    small = encode_both(tsv[: 1 << 20].rsplit(b"\n", 1)[0] + b"\n", desc, ["--block-bytes=70000"])[0]
+    small = encode_ours(tsv[: 1 << 20].rsplit(b"\n", 1)[0] + b"\n", desc, ["--block-bytes=70000"])
     assert small[0] == 0
     back = decode_both(small[1], ["-q", "-"])
     assert back[0][1] == back[1][1] == tsv[: 1 << 20].rsplit(b"\n", 1)[0] + b"\n"
@@ -278,7 +294,7 @@ def test_block_bytes_windows_cut_like_the_sequential_loop(window):
     the restatement writes for those cuts."""
     tsv = O.golden("movie_tickets.sql")[: 1 << 20].rsplit(b"\n", 1)[0] + b"\n"
     desc = O.golden("movie_tickets.desc.sql")
-    ours = encode_both(tsv, desc, [f"--block-bytes={window}"])[0]
+    ours = encode_ours(tsv, desc, [f"--block-bytes={window}"])
     assert ours[0] == 0, ours[2]
     plan = _window_plan(tsv, window)
     want = O.encode(O.parse_desc(desc), tsv, plan=plan)
@@ -296,7 +312,7 @@ def test_truncated_and_trailing_garbage():
     a, b = decode_both(z[: len(z) // 2], ["-q"])   # cut inside the dictionary: the short read throws GZREAD_FAILED,
     assert a[0] == b[0] == -6                       # which neither CLI catches (reference UnconvertFromZDW.cpp:294-300)
     assert "failed" in a[2] and "failed" in b[2]
-    a = decode_both(z[: len(z) - 1000], ["-q"])[0]  # cut inside the rows
+    a = decode_ours(z[: len(z) - 1000], ["-q"])  # cut inside the rows
     assert a[0] == 8  # ROW_COUNT_ERR (the reference dies on the short read here as well)
 
 
@@ -304,29 +320,30 @@ def test_truncated_and_trailing_garbage():
 @pytest.mark.parametrize("name", ["test", "analytics-hits", "movie_tickets"])
 def test_unconvert_api_matches_reference(name):
     z = O.golden(f"{name}.zdw")
-    for tool_dir in (BIN, REF):
+    for runner in (ours, RR.run):
         with Work() as d:
             (d / "x.zdw").write_bytes(z)
-            rc, out, err = run(tool_dir, "test_unconvert_api", ["x.zdw"], d)
+            rc, out, err, _ = runner("test_unconvert_api", ["x.zdw"], d)
             assert rc == 0, err
             assert out == O.golden(f"{name}.sql")
     names = [ln.split(b"\t")[0].decode() for ln in O.golden(f"{name}.desc.sql").splitlines()]
     sel = ",".join([names[-1], "nope", names[0]])
     outs = []
-    for tool_dir in (BIN, REF):
+    for runner in (ours, RR.run):
         with Work() as d:
             (d / "x.zdw").write_bytes(z)
-            outs.append(run(tool_dir, "test_unconvert_api", ["-ci", sel, "x.zdw"], d)[:2])
+            outs.append(runner("test_unconvert_api", ["-ci", sel, "x.zdw"], d)[:2])
     assert outs[0] == outs[1]
 
 
 @pytest.mark.gpu
 def test_block_plan_flag_reproduces_the_references_memory_cut():
-    """convertDWfile --block-plan=rows:spill with the plan recovered from a file the reference cut under --mem-limit."""
+    """convertDWfile --block-plan=rows:spill with the plan recovered from the memory-cut file (test_block_plan.memory_cut_file:
+    the restatement's file for the cut the reference makes under --mem-limit=140)."""
     import c5_check
     import test_block_plan as BP
     sch = O.parse_desc(c5_check.DESC)
-    tsv, image = BP.reference_mem_limit_file(600_000, 140)
+    tsv, image = BP.memory_cut_file()
     plan = BP.recover_plan(sch, tsv, image)
     with Work() as d:
         (d / "x.sql").write_bytes(tsv)
@@ -354,7 +371,7 @@ def test_encode_workers_write_the_sequential_file(flags):
     (--lanes-per-gpu=1) and as the restatement for those cuts."""
     tsv = O.golden("movie_tickets.sql")[: 3 << 20].rsplit(b"\n", 1)[0] + b"\n"
     desc = O.golden("movie_tickets.desc.sql")
-    ours = encode_both(tsv, desc, ["--block-bytes=131072", *flags])[0]
+    ours = encode_ours(tsv, desc, ["--block-bytes=131072", *flags])
     assert ours[0] == 0, ours[2]
     plan = _window_plan(tsv, 131072)
     want = O.encode(O.parse_desc(desc), tsv, plan=plan)
@@ -371,7 +388,7 @@ def test_encode_workers_report_the_first_bad_row():
     tsv = b"\n".join(rows) + b"\n"
     desc = corpus.desc([("a", "int(11)"), ("b", "varchar(8)"), ("c", "int(11)")])
     for flags in (["--lanes-per-gpu=1"], ["--gpus=0,0"]):
-        ours = encode_both(tsv, desc, ["--block-bytes=65536", *flags])[0]
+        ours = encode_ours(tsv, desc, ["--block-bytes=65536", *flags])
         assert ours[0] == 2, ours[2]
         assert "had the problem" in ours[2] and "WRONG_NUM_OF_COLUMNS_ON_A_ROW" in ours[2]
         assert "x.creating.zdw.gz" in ours[3] and "x.zdw.gz" not in ours[3]
@@ -395,14 +412,16 @@ def test_c4_file_on_two_gpus_equals_one_gpu_and_the_oracle():
     tsv = b"".join(parts)
     window = len(tsv) // 17
     two = "--gpus=2" if _gpu_count() >= 2 else "--gpus=0,0"
-    one = encode_both(tsv, synth.desc, [f"--block-bytes={window}", "--gpus=1", "--lanes-per-gpu=1"])[0]
-    par = encode_both(tsv, synth.desc, [f"--block-bytes={window}", two])[0]
+    one = encode_ours(tsv, synth.desc, [f"--block-bytes={window}", "--gpus=1", "--lanes-per-gpu=1"])
+    par = encode_ours(tsv, synth.desc, [f"--block-bytes={window}", two])
     assert one[0] == 0 and par[0] == 0, one[2] + par[2]
     assert one[1] == par[1]
     plan = _window_plan(tsv, window)
     want = O.encode(O.parse_desc(synth.desc), tsv, plan=plan)
     assert want.nblocks >= 16 and par[1] == want.data
-    rc, ref_tsv, err = O.ref_decode(par[1], timeout=600)
+    with Work() as d:
+        (d / "x.zdw").write_bytes(par[1])
+        rc, ref_tsv, err, _ = RR.run("unconvertDWfile", ["-q", "-", "x.zdw"], d, timeout=600)
     assert rc == 0 and ref_tsv == tsv, err
 
 
@@ -416,8 +435,8 @@ def test_decode_workers_write_the_sequential_rows(flags):
     desc = O.golden("movie_tickets.desc.sql")
     img = O.encode(O.parse_desc(desc), tsv, rows_per_block=2500)
     assert img.nblocks >= 15
-    a = decode_both(img.data, ["-q", *flags])[0]
-    b = decode_both(img.data, ["-q"])[1]
+    a = decode_ours(img.data, ["-q", *flags])
+    b = decode_recorded(img.data, ["-q"])
     assert a[0] == b[0] == 0, a[2]
     assert a[3]["x.sql"] == b[3]["x.sql"] == tsv
     with Work() as d:
@@ -425,7 +444,7 @@ def test_decode_workers_write_the_sequential_rows(flags):
         rc, out, err = run(BIN, "unconvertDWfile", ["-q", *flags, "-", "x.zdw"], d)
         assert rc == 0 and out == tsv, err
         rc, out, err = run(BIN, "unconvertDWfile", ["-q", *flags, "-c", "revenue,virtual_export_row,movie", "--non-empty-column-header", "-", "x.zdw"], d)
-        rc2, out2, err2 = run(REF, "unconvertDWfile", ["-q", "-c", "revenue,virtual_export_row,movie", "--non-empty-column-header", "-", "x.zdw"], d)
+        rc2, out2, err2, _ = RR.run("unconvertDWfile", ["-q", "-c", "revenue,virtual_export_row,movie", "--non-empty-column-header", "-", "x.zdw"], d)
         assert rc == rc2 == 0 and out == out2, err
 
 
@@ -465,8 +484,8 @@ def test_c4_file_decodes_on_two_gpus():
     img = O.encode(O.parse_desc(synth.desc), tsv, rows_per_block=rows)
     assert img.nblocks == 17
     two = "--gpus=2" if _gpu_count() >= 2 else "--gpus=0,0"
-    a = decode_both(img.data, ["-q", two])[0]
-    b = decode_both(img.data, ["-q"])[1]
+    a = decode_ours(img.data, ["-q", two])
+    b = decode_recorded(img.data, ["-q"])
     assert a[0] == 0, a[2]
     assert a[3]["x.sql"] == tsv == b[3]["x.sql"]
 
@@ -485,24 +504,25 @@ def test_streaming_validation_compares_normalised_rows(flags):
             rows.append(b"\n\n")
     tsv = b"".join(rows) + b"tail\t1"
     outs = []
-    for tool_dir in (BIN, REF):
+    for runner in (ours, RR.run):
         with Work() as d:
             (d / "x.desc.sql").write_bytes(desc)
-            extra = ["--block-bytes=20000"] if tool_dir == BIN else []
-            rc, out, err = run(tool_dir, "convertDWfile", [*flags, *extra, "x.sql"], d, stdin=tsv)
-            outs.append((rc, b"GOOD" in out, sorted(p.name for p in d.iterdir()), (out + err).decode("latin1")))
+            extra = ["--block-bytes=20000"] if runner is ours else []
+            rc, out, err, files = runner("convertDWfile", [*flags, *extra, "x.sql"], d, stdin=tsv)
+            outs.append((rc, b"GOOD" in out, sorted(files), (out + err).decode("latin1")))
     assert outs[0][:3] == outs[1][:3], outs
     assert outs[0][0] == 0 and outs[0][1], outs[0][3]
 
 
 @pytest.mark.gpu
 def test_heap_blocks_flag_reproduces_the_references_memory_cut_without_a_plan():
-    """convertDWfile --heap-blocks=2 writes the file the compiled reference cut on its own under --mem-limit=140 (K = 2 is
+    """convertDWfile --heap-blocks=2 writes the memory-cut file (the restatement's file for the cut the compiled reference
+    makes on its own under --mem-limit=140, test_block_plan.memory_cut_file; K = 2 is
     the allocation at which that process was over its limit, tests/test_block_plan.py) - no explicit plan given.
     --mem-limit itself is accepted and changes nothing."""
     import c5_check
     import test_block_plan as BP
-    tsv, image = BP.reference_mem_limit_file(600_000, 140)
+    tsv, image = BP.memory_cut_file()
     with Work() as d:
         (d / "x.sql").write_bytes(tsv)
         (d / "x.desc.sql").write_bytes(c5_check.DESC)
