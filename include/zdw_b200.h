@@ -80,9 +80,8 @@ int zdwb_ctx_set_stream(zdwb_ctx* ctx, void* cuda_stream);
  * in the radix passes: 4 or 16, 0 = by size), "ht_initial_log2" (first-try size of the string hash set).  Decode:
  * "dec_delta" (0/1: rows of wide schemas are assembled from the row before), "dec_strip_rows" (rows per strip of the row
  * kernels, 0 = automatic), "dec_group_lanes" (lanes per row in the narrow-schema kernels: 8, 16, 32, 0 = by schema
- * width), "dec_emit_words" (0/1: cached texts leave as aligned words), "dec_tile_bytes" (row-stream bytes per CTA in the
- * row-boundary discovery), "dec_readback_kernel" (0/1: small results reach the host through a kernel's stores into
- * mapped memory instead of the copy engine).  Both: "copy_gate" (0/1, default 1: host<->device copies of 8 MiB and more
+ * width), "dec_tile_bytes" (row-stream bytes per CTA in the row-boundary discovery).  Both: "copy_gate" (0/1, default
+ * 1: host<->device copies of 8 MiB and more
  * take turns with those of the process's other contexts on the same device instead of sharing the link),
  * "kernel_timing" (0/1).  Returns ZDWB_ERR_BAD_ARG for unknown names. */
 int zdwb_ctx_set_tuning(zdwb_ctx* ctx, const char* name, long long value);

@@ -193,13 +193,17 @@ def test_roundtrip_property_large_random(ctx):
     assert img == O.encode(sch, tsv).data
 
 
-@pytest.mark.parametrize("emit_words,delta,lanes,strip", [(0, 0, 0, 0), (1, 0, 8, 0), (1, 0, 16, 0), (1, 1, 32, 0), (1, 1, 32, 3), (0, 1, 0, 1)])
-def test_row_writer_variants_forced(ctx, emit_words, delta, lanes, strip):
-    """The row writer has variants: cached texts stored byte by byte or as aligned words (dec_emit_words), and for wide
-    schemas rows assembled from the row before (dec_delta: unchanged stretches copied 16 bytes at a time, only changed
-    items rendered).  Every combination must write the oracle's rows: the whole corpus, the goldens, projections, the
-    in-memory layout; short strips make the delta writer start over often."""
-    ctx.set_tuning("dec_emit_words", emit_words)
+@pytest.mark.parametrize("delta,lanes,strip", [(0, 0, 0), (0, 8, 0), (0, 16, 0), (1, 32, 0), (1, 32, 3), (1, 0, 1)])
+def test_row_writer_variants_forced(ctx, delta, lanes, strip):
+    """The row writer has variants: for wide schemas rows assembled from the row before (dec_delta: unchanged stretches
+    copied 16 bytes at a time, only changed items rendered), 8, 16 or 32 lanes per row, the strip length.  Every
+    combination must write the oracle's rows: the whole corpus, the goldens, projections, the in-memory layout; short
+    strips make the delta writer start over often.  The knobs of removed variants are unknown names."""
+    from zdw_b200 import ZdwError
+    for removed in ("dec_emit_words", "dec_readback_kernel"):
+        with pytest.raises(ZdwError) as ei:
+            ctx.set_tuning(removed, 1)
+        assert ei.value.code == 4  # ZDWB_ERR_BAD_ARG
     ctx.set_tuning("dec_delta", delta)
     ctx.set_tuning("dec_group_lanes", lanes)
     ctx.set_tuning("dec_strip_rows", strip)
@@ -214,7 +218,6 @@ def test_row_writer_variants_forced(ctx, emit_words, delta, lanes, strip):
         test_column_projection(ctx)
         test_in_memory_layout_and_row_offsets(ctx)
     finally:
-        ctx.set_tuning("dec_emit_words", 1)
         ctx.set_tuning("dec_delta", 1)
         ctx.set_tuning("dec_group_lanes", 0)
         ctx.set_tuning("dec_strip_rows", 0)

@@ -8,6 +8,8 @@
 #pragma once
 #include <stdint.h>
 
+#include "common.cuh"
+
 namespace zdwb {
 namespace {
 
@@ -54,6 +56,22 @@ __global__ void k_carry_apply(const unsigned long long* __restrict__ sval, const
     cin[(size_t)s * U + u] = v;
     if (shas[(size_t)s * U + u]) v = sval[(size_t)s * U + u];
   }
+}
+
+// cin of nstrips strips of U used columns from their sval / shas: reduce, scan and apply over segments of S strips
+int carry_prefix(Ctx* ctx, const unsigned long long* sval, const uint8_t* shas, uint32_t nstrips, uint32_t U,
+                 unsigned long long* cin) {
+  const uint32_t S = std::max<uint32_t>((nstrips + 255) / 256, 4);  // (the scan over segments is a serial loop: at least 4 per segment)
+  const uint32_t nseg = (nstrips + S - 1) / S;
+  DevBuf seg_val, seg_has;
+  ZDWB_TRY(seg_val.alloc(ctx, (size_t)nseg * U * 8));
+  ZDWB_TRY(seg_has.alloc(ctx, (size_t)nseg * U));
+  const dim3 g2((U + 127) / 128, nseg);
+  ZDWB_TRY(launch(ctx, "k_carry_reduce", k_carry_reduce, g2, 128, 0, sval, shas, nstrips, U, S, seg_val.as<unsigned long long>(),
+                  seg_has.as<uint8_t>()));
+  ZDWB_TRY(launch(ctx, "k_carry_scan", k_carry_scan, (U + 127) / 128, 128, 0, seg_val.as<unsigned long long>(),
+                  seg_has.as<uint8_t>(), nseg, U));
+  return launch(ctx, "k_carry_apply", k_carry_apply, g2, 128, 0, sval, shas, seg_val.as<unsigned long long>(), nstrips, U, S, cin);
 }
 
 }  // namespace

@@ -39,9 +39,7 @@ struct Ctx {
   long long dec_group_lanes = 0;     // lanes per strip in the row kernels: 8, 16, 32 (0 = by schema width)
   long long dec_strip_rows = 0;      // rows per strip of the row kernels (0 = automatic)
   long long copy_gate = 1;           // large H2D / D2H copies of different contexts take turns (0 = off)
-  long long dec_emit_words = 1;      // the row writer stores cached texts as aligned words (k_dec_rows<.., true>; measured: 0.98 -> 0.90 ms)
   long long dec_delta = 1;           // wide schemas: rows are assembled from the row before (k_dec_write_delta)
-  long long dec_readback_kernel = 1; // small decode results reach the host through a kernel's stores, not the copy engine (decode.cu)
   long long dec_tile_bytes = 8192;   // row-stream bytes per CTA in the decoder's row-boundary discovery
   unsigned long long last_out_per_row = 0;  // decoded bytes per row of the previous block (sizes the next output)
   unsigned long long last_unique = 0;  // dictionary size of the previous block (seeds the next hash set)
@@ -85,30 +83,6 @@ struct Ctx {
   std::vector<Timed> timed;
 };
 
-// Brackets one kernel launch with events when Ctx::timing is on (zero cost otherwise).
-struct KernelScope {
-  Ctx* c;
-  const char* name;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  KernelScope(Ctx* ctx, const char* n) : c(ctx), name(n) {
-    if (c->timing) {
-      cudaEventCreate(&e0);
-      cudaEventCreate(&e1);
-      cudaEventRecord(e0, c->stream);
-    }
-  }
-  ~KernelScope() {
-    if (e0) {
-      cudaEventRecord(e1, c->stream);
-      c->timed.push_back(Ctx::Timed{name, e0, e1});
-    }
-  }
-};
-
-struct Status {
-  int code;
-};
-
 #define ZDWB_CUDA_TRY(ctx, expr)                                                                   \
   do {                                                                                             \
     cudaError_t _e = (expr);                                                                       \
@@ -128,12 +102,31 @@ struct Status {
     if (_rc != ZDWB_OK) return _rc;       \
   } while (0)
 
-// count a launch and check for launch-configuration errors
-#define ZDWB_LAUNCH_CHECK(ctx)                                                                     \
-  do {                                                                                             \
-    (ctx)->launches++;                                                                             \
-    ZDWB_CUDA_TRY(ctx, cudaGetLastError());                                                        \
-  } while (0)
+#ifdef __CUDACC__
+// Launches kernel k on the context's stream: bracketed by events when Ctx::timing is on, counted in Ctx::launches, and
+// checked for launch errors, which name the kernel in Ctx::err.
+template <class... P, class... A>
+int launch(Ctx* c, const char* name, void (*k)(P...), dim3 grid, dim3 block, size_t smem, A... args) {
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  if (c->timing) {
+    cudaEventCreate(&e0);
+    cudaEventCreate(&e1);
+    cudaEventRecord(e0, c->stream);
+  }
+  k<<<grid, block, smem, c->stream>>>(args...);
+  if (e0) {
+    cudaEventRecord(e1, c->stream);
+    c->timed.push_back(Ctx::Timed{name, e0, e1});
+  }
+  ++c->launches;
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    c->err = std::string("launch of ") + name + " failed: " + cudaGetErrorString(e);
+    return e == cudaErrorMemoryAllocation ? ZDWB_ERR_OOM : ZDWB_ERR_CUDA;
+  }
+  return ZDWB_OK;
+}
+#endif
 
 // Device memory of a call comes from a per-context stack arena: a few big cudaMalloc'd chunks that every call re-uses
 // from the bottom, so a call in steady state makes no driver-level memory-management call at all (those serialise with

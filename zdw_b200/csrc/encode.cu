@@ -2550,25 +2550,17 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     const uint32_t ntiles = (uint32_t)((span + tile_bytes - 1) / tile_bytes);
     const uint32_t tile_ctas = (ntiles + ENC_WARPS - 1) / ENC_WARPS;
     ZDWB_TRY(agg.alloc(ctx, (size_t)ntiles * sizeof(TileAgg)));
-    if (delta) {
-      KernelScope _ks(ctx, "k_row_census");
-      k_row_census<<<tile_ctas, ENC_THREADS, 0, st>>>(buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>());
-    } else {
-      KernelScope _ks(ctx, "k_tile_count");
-      k_tile_count<<<tile_ctas, ENC_THREADS, 0, st>>>(buf, n, lo, ntiles, agg.as<TileAgg>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    if (delta)
+      ZDWB_TRY(launch(ctx, "k_row_census", k_row_census, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>()));
+    else
+      ZDWB_TRY(launch(ctx, "k_tile_count", k_tile_count, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, agg.as<TileAgg>()));
     {
       const uint32_t nparts = (ntiles + TS_THREADS - 1) / TS_THREADS;
       DevBuf part;
       ZDWB_TRY(part.alloc(ctx, (size_t)nparts * sizeof(TileAgg)));
-      KernelScope _ks(ctx, "k_tile_scan");
-      k_tile_scan_local<<<nparts, TS_THREADS, 0, st>>>(agg.as<TileAgg>(), ntiles, part.as<TileAgg>());
-      ZDWB_LAUNCH_CHECK(ctx);
-      k_tile_scan<<<1, TS_THREADS, 0, st>>>(part.as<TileAgg>(), nparts, meta);
-      ZDWB_LAUNCH_CHECK(ctx);
-      k_tile_scan_add<<<nparts, TS_THREADS, 0, st>>>(agg.as<TileAgg>(), ntiles, part.as<TileAgg>());
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_local, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
+      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan, 1, TS_THREADS, 0, part.as<TileAgg>(), nparts, meta));
+      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_add, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
     }
     ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
     ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
@@ -2605,11 +2597,7 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
         out->tsv_consumed = tail_start;  // the unterminated tail belongs to the next window
       }
     } else {
-      {
-        KernelScope _ks(ctx, "k_find_cut");
-        k_find_cut<<<1, 32, 0, st>>>(buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>(), nrows - 1, meta);
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_find_cut", k_find_cut, 1, 32, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>(), nrows - 1, meta));
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
       ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
       limit = hmeta->cut_end_p1;
@@ -2617,11 +2605,7 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       {
         // the row behind the block has been read in full when the block is closed - the row buffer has grown with it
         // (getnextrow.cpp:57-65), so its length counts for longestLine - and its first spill_cols columns have been parsed
-        {
-          KernelScope _ks(ctx, "k_find_spill");
-          k_find_spill<<<1, 1, 0, st>>>(buf, n, hmeta->next_start, opts->spill_cols, meta);
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
+        ZDWB_TRY(launch(ctx, "k_find_spill", k_find_spill, 1, 1, 0, buf, n, hmeta->next_start, opts->spill_cols, meta));
         ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
         ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
         if (hmeta->spill_row_len) {
@@ -2675,12 +2659,8 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(slots.p, 0, cap * 8, st));
       ht.slots = slots.as<unsigned long long>();
       ht.mask = (uint32_t)(cap - 1);
-      {
-        KernelScope _ks(ctx, "k_init_minmax");
-        k_init_minmax<<<(ncols + 255) / 256, 256, 0, st>>>(colmin.as<unsigned long long>(), colmax.as<unsigned long long>(),
-                                                         colset.as<uint32_t>(), ncols);
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_init_minmax", k_init_minmax, (ncols + 255) / 256, 256, 0, colmin.as<unsigned long long>(),
+                      colmax.as<unsigned long long>(), colset.as<uint32_t>(), ncols));
       P1Args A;
       A.buf = buf;
       A.n = n;
@@ -2709,29 +2689,19 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
         D.row_cnt = row_cnt.as<uint32_t>();
         D.chg_start = chg_start.as<uint32_t>();
         D.chg_len = chg_len.as<uint32_t>();
-        {
-          KernelScope _ks(ctx, "k_pass1d");
-          k_pass1d<<<(p1_tiles + D1_WARPS - 1) / D1_WARPS, D1_THREADS, 0, st>>>(D);
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
+        ZDWB_TRY(launch(ctx, "k_pass1d", k_pass1d, (p1_tiles + D1_WARPS - 1) / D1_WARPS, D1_THREADS, 0, D));
         D1List L;
         L.start = chg_start.as<uint32_t>();
         L.len = chg_len.as<uint32_t>();
         L.col = rec_col.as<uint32_t>();
-        KernelScope _ks(ctx, "k_pass1d_values");
-        k_pass1d_values<<<ctx->sm_count * 4, ENC_THREADS, 0, st>>>(A, L, (uint32_t)rec_cap);
+        ZDWB_TRY(launch(ctx, "k_pass1d_values", k_pass1d_values, ctx->sm_count * 4, ENC_THREADS, 0, A, L, (uint32_t)rec_cap));
       } else {
-        KernelScope _ks(ctx, "k_pass1");
-        k_pass1<<<(p1_tiles + ENC_WARPS - 1) / ENC_WARPS, ENC_THREADS, 0, st>>>(A);
+        ZDWB_TRY(launch(ctx, "k_pass1", k_pass1, (p1_tiles + ENC_WARPS - 1) / ENC_WARPS, ENC_THREADS, 0, A));
       }
-      ZDWB_LAUNCH_CHECK(ctx);
-      {  // writeLookupColumnStats (ConvertToZDW.cpp:417-483) needs nothing from the host: it runs before the read-back
-        KernelScope _ks(ctx, "k_col_stats");
-        k_col_stats<<<1, ENC_THREADS, 0, st>>>(types_d.as<uint8_t>(), ncols, colset.as<uint32_t>(), colmin.as<unsigned long long>(),
-                                             colmax.as<unsigned long long>(), csize.as<uint8_t>(), cbase.as<unsigned long long>(),
-                                             used_idx.as<int32_t>(), used_cols.as<uint32_t>(), meta);
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      // writeLookupColumnStats (ConvertToZDW.cpp:417-483) needs nothing from the host: it runs before the read-back
+      ZDWB_TRY(launch(ctx, "k_col_stats", k_col_stats, 1, ENC_THREADS, 0, types_d.as<uint8_t>(), ncols, colset.as<uint32_t>(),
+                      colmin.as<unsigned long long>(), colmax.as<unsigned long long>(), csize.as<uint8_t>(),
+                      cbase.as<unsigned long long>(), used_idx.as<int32_t>(), used_cols.as<uint32_t>(), meta));
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
       ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
       if (hmeta->delta_bail) {
@@ -2793,26 +2763,14 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       ZDWB_TRY(pre.alloc(ctx, (size_t)nrec * 8));
       ZDWB_TRY(cut_d.alloc(ctx, sizeof(HeapCut)));
       ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(first_ord.p, 0xff, cap * 4, st));
-      {
-        KernelScope _ks(ctx, "k_heap_first_ord");
-        k_heap_first_ord<<<(nrec + 255) / 256, 256, 0, st>>>(rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
-                                                           types_d.as<uint8_t>(), nrec, first_ord.as<uint32_t>());
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
-      {
-        KernelScope _ks(ctx, "k_heap_new_len");
-        k_heap_new_len<<<(nrec + 255) / 256, 256, 0, st>>>(rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
-                                                         types_d.as<uint8_t>(), nrec, first_ord.as<uint32_t>(), ht.slots,
-                                                         new_len.as<uint64_t>());
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_heap_first_ord", k_heap_first_ord, (nrec + 255) / 256, 256, 0, rec_col.as<uint32_t>(),
+                      rec_val.as<unsigned long long>(), types_d.as<uint8_t>(), nrec, first_ord.as<uint32_t>()));
+      ZDWB_TRY(launch(ctx, "k_heap_new_len", k_heap_new_len, (nrec + 255) / 256, 256, 0, rec_col.as<uint32_t>(),
+                      rec_val.as<unsigned long long>(), types_d.as<uint8_t>(), nrec, first_ord.as<uint32_t>(), ht.slots,
+                      new_len.as<uint64_t>()));
       ZDWB_TRY(exclusive_scan_u64(ctx, new_len.as<uint64_t>(), pre.as<uint64_t>(), nrec, nullptr));
-      {
-        KernelScope _ks(ctx, "k_heap_cut");
-        k_heap_cut<<<1, 1, 0, st>>>(pre.as<uint64_t>(), new_len.as<uint64_t>(), nrec, 0, probe->K, row_rec.as<uint32_t>(),
-                                    nrows, rec_col.as<uint32_t>(), cut_d.as<HeapCut>());
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_heap_cut", k_heap_cut, 1, 1, 0, pre.as<uint64_t>(), new_len.as<uint64_t>(), nrec, 0, probe->K,
+                      row_rec.as<uint32_t>(), nrows, rec_col.as<uint32_t>(), cut_d.as<HeapCut>()));
       HeapCut* hc = reinterpret_cast<HeapCut*>(reinterpret_cast<uint8_t*>(ctx->meta_host) + 2048);
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hc, cut_d.p, sizeof(HeapCut), cudaMemcpyDeviceToHost, st));
       ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
@@ -2852,25 +2810,14 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ZDWB_TRY(order.alloc(ctx, (size_t)nu * 4));
     ZDWB_TRY(offs.alloc(ctx, (size_t)nu * 4));
     const uint32_t cap = ht.mask + 1;
-    {
-      KernelScope _ks(ctx, "k_ht_compact");
-      k_ht_compact<<<(cap + ENC_THREADS - 1) / ENC_THREADS, ENC_THREADS, 0, st>>>(ht.slots, cap, ustart.as<uint32_t>(),
-                                                                               ulen.as<uint32_t>(), uslot.as<uint32_t>(), meta);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_ht_compact", k_ht_compact, (cap + ENC_THREADS - 1) / ENC_THREADS, ENC_THREADS, 0, ht.slots, cap,
+                    ustart.as<uint32_t>(), ulen.as<uint32_t>(), uslot.as<uint32_t>(), meta));
     ZDWB_TRY(sort_strings(ctx, buf, ustart.as<uint32_t>(), ulen.as<uint32_t>(), nu, hmeta->max_str_len, order.as<uint32_t>()));
-    {
-      KernelScope _ks(ctx, "k_sorted_lens");
-      k_sorted_lens<<<(nu + 255) / 256, 256, 0, st>>>(order.as<uint32_t>(), ulen.as<uint32_t>(), nu, offs.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_sorted_lens", k_sorted_lens, (nu + 255) / 256, 256, 0, order.as<uint32_t>(), ulen.as<uint32_t>(), nu,
+                    offs.as<uint32_t>()));
     ZDWB_TRY(exclusive_scan_u32(ctx, offs.as<uint32_t>(), offs.as<uint32_t>(), nu, nullptr));
-    {
-      KernelScope _ks(ctx, "k_dict_slots");
-      k_dict_slots<<<(nu + 255) / 256, 256, 0, st>>>(order.as<uint32_t>(), uslot.as<uint32_t>(), offs.as<uint32_t>(), nu,
-                                                   slot_off.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_dict_slots", k_dict_slots, (nu + 255) / 256, 256, 0, order.as<uint32_t>(), uslot.as<uint32_t>(),
+                    offs.as<uint32_t>(), nu, slot_off.as<uint32_t>()));
   }
 
   // ---- pass 2 into the staging buffer
@@ -2901,12 +2848,8 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ZDWB_TRY(tile_off.alloc(ctx, (size_t)tiles2 * 8));
     ZDWB_TRY(rows_total_d.alloc(ctx, 8));
     ZDWB_TRY(colinfo.alloc(ctx, (size_t)ncols * sizeof(ColInfo)));
-    {
-      KernelScope _ks(ctx, "k_col_info");
-      k_col_info<<<(ncols + 255) / 256, 256, 0, st>>>(types_d.as<uint8_t>(), used_idx.as<int32_t>(), cbase.as<unsigned long long>(), ncols,
-                                                    colinfo.as<ColInfo>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_col_info", k_col_info, (ncols + 255) / 256, 256, 0, types_d.as<uint8_t>(), used_idx.as<int32_t>(),
+                    cbase.as<unsigned long long>(), ncols, colinfo.as<ColInfo>()));
     if (delta) {
       P2DArgs A2;
       A2.rec_col = rec_col.as<uint32_t>();
@@ -2922,60 +2865,27 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       A2.used_cols = used_cols.as<uint32_t>();
       A2.csize = csize.as<uint8_t>();
       // the value every used column has where a tile begins
-      DevBuf cin, sval, shas, seg_val, seg_has;
+      DevBuf cin, sval, shas;
       if (tiles2 > 1) {
         ZDWB_TRY(cin.alloc(ctx, (size_t)tiles2 * U * 8));
         ZDWB_TRY(sval.alloc(ctx, (size_t)tiles2 * U * 8));
         ZDWB_TRY(shas.alloc(ctx, (size_t)tiles2 * U));
         const size_t smem_sum = (size_t)U * 4 + (size_t)(2 * rpc2 + 1) * 4 + 16;
         ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_p2d_summary, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-        {
-          KernelScope _ks(ctx, "k_p2d_summary");
-          k_p2d_summary<<<tiles2, ENC_THREADS, smem_sum, st>>>(A2, sval.as<unsigned long long>(), shas.as<uint8_t>());
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
-        const uint32_t S = std::max<uint32_t>((tiles2 + 255) / 256, 4);  // (the scan over segments is a serial loop: at least 4 per segment)
-        const uint32_t nseg = (tiles2 + S - 1) / S;
-        ZDWB_TRY(seg_val.alloc(ctx, (size_t)nseg * U * 8));
-        ZDWB_TRY(seg_has.alloc(ctx, (size_t)nseg * U));
-        dim3 g2((U + 127) / 128, nseg);
-        {
-          KernelScope _ks(ctx, "k_carry_reduce");
-          k_carry_reduce<<<g2, 128, 0, st>>>(sval.as<unsigned long long>(), shas.as<uint8_t>(), tiles2, U, S,
-                                           seg_val.as<unsigned long long>(), seg_has.as<uint8_t>());
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
-        {
-          KernelScope _ks(ctx, "k_carry_scan");
-          k_carry_scan<<<(U + 127) / 128, 128, 0, st>>>(seg_val.as<unsigned long long>(), seg_has.as<uint8_t>(), nseg, U);
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
-        {
-          KernelScope _ks(ctx, "k_carry_apply");
-          k_carry_apply<<<g2, 128, 0, st>>>(sval.as<unsigned long long>(), shas.as<uint8_t>(), seg_val.as<unsigned long long>(),
-                                          tiles2, U, S, cin.as<unsigned long long>());
-        }
-        ZDWB_LAUNCH_CHECK(ctx);
+        ZDWB_TRY(launch(ctx, "k_p2d_summary", k_p2d_summary, tiles2, ENC_THREADS, smem_sum, A2, sval.as<unsigned long long>(),
+                        shas.as<uint8_t>()));
+        ZDWB_TRY(carry_prefix(ctx, sval.as<unsigned long long>(), shas.as<uint8_t>(), tiles2, U, cin.as<unsigned long long>()));
       }
       const size_t smem = (size_t)(rpc2 + 1) * U * 8 + (size_t)(rpc2 + 1) * MW * 4 + (size_t)(3 * rpc2 + 3) * 4 + U + 16;
       ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_pass2d, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-      {
-        KernelScope _ks(ctx, "k_pass2d");
-        k_pass2d<<<tiles2, ENC_THREADS, smem, st>>>(A2, tiles2 > 1 ? cin.as<unsigned long long>() : nullptr, tile_cap,
-                                                  staging.as<uint8_t>(), tile_bytes.as<uint64_t>());
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_pass2d", k_pass2d, tiles2, ENC_THREADS, smem, A2, tiles2 > 1 ? cin.as<unsigned long long>() : nullptr,
+                      tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>()));
     } else {
       const size_t smem = (size_t)(rpc2 + 1) * U * 8 + (size_t)(rpc2 + 1) * 4 + (size_t)(rpc2 + 2) * 4 + U + 16;
       ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_pass2, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-      {
-        KernelScope _ks(ctx, "k_pass2");
-        k_pass2<<<tiles2, ENC_THREADS, smem, st>>>(rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(), row_rec.as<uint32_t>(),
-                                                 nrows, rpc2, colinfo.as<ColInfo>(), slot_off.as<uint32_t>(),
-                                                 used_cols.as<uint32_t>(), csize.as<uint8_t>(), U,
-                                                 nflag, tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>());
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_pass2", k_pass2, tiles2, ENC_THREADS, smem, rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
+                      row_rec.as<uint32_t>(), nrows, rpc2, colinfo.as<ColInfo>(), slot_off.as<uint32_t>(), used_cols.as<uint32_t>(),
+                      csize.as<uint8_t>(), U, nflag, tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>()));
     }
     ZDWB_TRY(exclusive_scan_u64(ctx, tile_bytes.as<uint64_t>(), tile_off.as<uint64_t>(), tiles2, rows_total_d.as<uint64_t>()));
     ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(ctx->meta_host) + 1024, rows_total_d.p, 8, cudaMemcpyDeviceToHost, st));
@@ -2991,27 +2901,16 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ctx->out_dev = ob.detach();
   }
   uint8_t* outp = static_cast<uint8_t*>(ctx->out_dev);
-  {
-    KernelScope _ks(ctx, "k_block_header");
-    k_block_header<<<std::max(1u, std::min((ncols + 255) / 256, 64u)), 256, 0, st>>>(
-      outp, meta, nrows, longest_field, is_last ? 1u : 0u, ncols, csize.as<uint8_t>(), cbase.as<unsigned long long>(),
-      used_cols.as<uint32_t>());
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  ZDWB_TRY(launch(ctx, "k_block_header", k_block_header, std::max(1u, std::min((ncols + 255) / 256, 64u)), 256, 0, outp, meta, nrows,
+                  longest_field, is_last ? 1u : 0u, ncols, csize.as<uint8_t>(), cbase.as<unsigned long long>(), used_cols.as<uint32_t>()));
   if (nu) {
     const uint64_t threads = (uint64_t)nu * 8;
-    KernelScope _ks(ctx, "k_dict_emit");
-    k_dict_emit<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(buf, order.as<uint32_t>(), ustart.as<uint32_t>(),
-                                                                ulen.as<uint32_t>(), offs.as<uint32_t>(), nu,
-                                                                outp + hmeta->dict_base);
+    ZDWB_TRY(launch(ctx, "k_dict_emit", k_dict_emit, (unsigned)((threads + 255) / 256), 256, 0, buf, order.as<uint32_t>(),
+                    ustart.as<uint32_t>(), ulen.as<uint32_t>(), offs.as<uint32_t>(), nu, outp + hmeta->dict_base));
   }
-  if (nu) ZDWB_LAUNCH_CHECK(ctx);
-  if (tiles2) {
-    KernelScope _ks(ctx, "k_gather_tiles");
-    k_gather_tiles<<<tiles2, ENC_THREADS, 0, st>>>(staging.as<uint8_t>(), tile_cap, tile_off.as<uint64_t>(),
-                                                 tile_bytes.as<uint64_t>(), outp + rows_base);
-  }
-  if (tiles2) ZDWB_LAUNCH_CHECK(ctx);
+  if (tiles2)
+    ZDWB_TRY(launch(ctx, "k_gather_tiles", k_gather_tiles, tiles2, ENC_THREADS, 0, staging.as<uint8_t>(), tile_cap,
+                    tile_off.as<uint64_t>(), tile_bytes.as<uint64_t>(), outp + rows_base));
 
   const size_t total_len = (size_t)(rows_base + rows_bytes);
   out->len = total_len;

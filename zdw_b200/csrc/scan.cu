@@ -88,28 +88,12 @@ int exclusive_scan_impl(Ctx* ctx, const T* in, T* out, size_t n, T* total_dev) {
     return ZDWB_OK;
   }
   const size_t nb = (n + SCAN_TILE - 1) / SCAN_TILE;
-  if (nb == 1) {
-    {
-      KernelScope _ks(ctx, "k_scan_down");
-      k_scan_down<T><<<1, SCAN_THREADS, 0, ctx->stream>>>(in, out, n, nullptr, total_dev);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    return ZDWB_OK;
-  }
+  if (nb == 1) return launch(ctx, "k_scan_down", k_scan_down<T>, 1, SCAN_THREADS, 0, in, out, n, nullptr, total_dev);
   DevBuf sums;
   ZDWB_TRY(sums.alloc(ctx, nb * sizeof(T)));
-  {
-    KernelScope _ks(ctx, "k_scan_reduce");
-    k_scan_reduce<T><<<(unsigned)nb, SCAN_THREADS, 0, ctx->stream>>>(in, n, sums.as<T>());
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  ZDWB_TRY(launch(ctx, "k_scan_reduce", k_scan_reduce<T>, (unsigned)nb, SCAN_THREADS, 0, in, n, sums.as<T>()));
   ZDWB_TRY(exclusive_scan_impl<T>(ctx, sums.as<T>(), sums.as<T>(), nb, nullptr));
-  {
-    KernelScope _ks(ctx, "k_scan_down");
-    k_scan_down<T><<<(unsigned)nb, SCAN_THREADS, 0, ctx->stream>>>(in, out, n, sums.as<T>(), total_dev);
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
-  return ZDWB_OK;
+  return launch(ctx, "k_scan_down", k_scan_down<T>, (unsigned)nb, SCAN_THREADS, 0, in, out, n, sums.as<T>(), total_dev);
 }
 
 }  // namespace

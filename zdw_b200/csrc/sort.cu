@@ -235,26 +235,15 @@ int radix_passes(Ctx* ctx, SortBufs& b, uint32_t n, const int* pass_list, int np
   P.n = npass;
   for (int q = 0; q < npass; ++q) P.pass[q] = pass_list[q];
   ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(R.ghist, 0, RS_SMALL_BYTES, ctx->stream));
-  {
-    KernelScope _ks(ctx, "k_radix_ghist");
-    const uint32_t grid = std::min<uint32_t>((n + RS_THREADS - 1) / RS_THREADS, (uint32_t)ctx->sm_count * 8);
-    k_radix_ghist<<<grid, RS_THREADS, 0, ctx->stream>>>(b.key[b.cur], b.seg[b.cur], n, P, R.ghist);
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  const uint32_t grid = std::min<uint32_t>((n + RS_THREADS - 1) / RS_THREADS, (uint32_t)ctx->sm_count * 8);
+  ZDWB_TRY(launch(ctx, "k_radix_ghist", k_radix_ghist, grid, RS_THREADS, 0, b.key[b.cur], b.seg[b.cur], n, P, R.ghist));
   for (int q = 0; q < npass; ++q) {
     const int pass = pass_list[q];
     const int s = b.cur, d = b.cur ^ 1;
     const uint32_t epoch = ++R.epoch;
-    {
-      KernelScope _ks(ctx, "k_radix_onesweep");
-      if (items == 4)
-        k_radix_onesweep<4><<<ntiles, RS_THREADS, 0, ctx->stream>>>(b.key[s], b.seg[s], b.val[s], n, pass, q, epoch, R.ghist, R.tickets,
-                                                                   R.status, b.key[d], b.seg[s] ? b.seg[d] : nullptr, b.val[d]);
-      else
-        k_radix_onesweep<16><<<ntiles, RS_THREADS, 0, ctx->stream>>>(b.key[s], b.seg[s], b.val[s], n, pass, q, epoch, R.ghist, R.tickets,
-                                                                    R.status, b.key[d], b.seg[s] ? b.seg[d] : nullptr, b.val[d]);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_radix_onesweep", items == 4 ? k_radix_onesweep<4> : k_radix_onesweep<16>, ntiles, RS_THREADS, 0,
+                    b.key[s], b.seg[s], b.val[s], n, pass, q, epoch, R.ghist, R.tickets, R.status, b.key[d],
+                    b.seg[s] ? b.seg[d] : nullptr, b.val[d]));
     b.cur = d;
   }
   return ZDWB_OK;
@@ -470,29 +459,13 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
     ZDWB_TRY(rank.alloc(ctx, (size_t)n * 4));
     ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(rank.p, 0, (size_t)n * 4, st));
     const unsigned gi = (n + RK_THREADS - 1) / RK_THREADS, ntile = (n + RK_JTILE - 1) / RK_JTILE;
-    {
-      KernelScope _ks(ctx, "k_rank_keys");
-      k_rank_keys<<<gi, RK_THREADS, 0, st>>>(base, starts, lens, n, keys.as<ulonglong2>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_rank_tile_sort");
-      k_rank_tile_sort<<<ntile, RK_SORT_THREADS, 0, st>>>(keys.as<ulonglong2>(), n, skeys.as<ulonglong2>(), sidx.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_rank_count");
-      const uint32_t ipt = n > 16384 ? 4 : 1;
-      k_rank_count<<<dim3((gi + ipt - 1) / ipt, ntile), RK_THREADS, 0, st>>>(
-        base, starts, lens, keys.as<ulonglong2>(), skeys.as<ulonglong2>(), sidx.as<uint32_t>(), n, ipt, rank.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_rank_scatter");
-      k_rank_scatter<<<gi, RK_THREADS, 0, st>>>(rank.as<uint32_t>(), n, order_out);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    return ZDWB_OK;
+    ZDWB_TRY(launch(ctx, "k_rank_keys", k_rank_keys, gi, RK_THREADS, 0, base, starts, lens, n, keys.as<ulonglong2>()));
+    ZDWB_TRY(launch(ctx, "k_rank_tile_sort", k_rank_tile_sort, ntile, RK_SORT_THREADS, 0, keys.as<ulonglong2>(), n,
+                    skeys.as<ulonglong2>(), sidx.as<uint32_t>()));
+    const uint32_t ipt = n > 16384 ? 4 : 1;
+    ZDWB_TRY(launch(ctx, "k_rank_count", k_rank_count, dim3((gi + ipt - 1) / ipt, ntile), RK_THREADS, 0, base, starts, lens,
+                    keys.as<ulonglong2>(), skeys.as<ulonglong2>(), sidx.as<uint32_t>(), n, ipt, rank.as<uint32_t>()));
+    return launch(ctx, "k_rank_scatter", k_rank_scatter, gi, RK_THREADS, 0, rank.as<uint32_t>(), n, order_out);
   }
 
   // ---- large path
@@ -527,11 +500,7 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
   b.cur = 0;
 
   // round 0: sort everything by the first 8 bytes
-  {
-    KernelScope _ks(ctx, "k_make_keys");
-    k_make_keys<<<g256, 256, 0, st>>>(base, starts, lens, nullptr, n, 0, b.key[0], b.val[0]);
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  ZDWB_TRY(launch(ctx, "k_make_keys", k_make_keys, g256, 256, 0, base, starts, lens, nullptr, n, 0, b.key[0], b.val[0]));
   {
     const int passes[8] = {0, 1, 2, 3, 4, 5, 6, 7};
     ZDWB_TRY(radix_passes(ctx, b, n, passes, 8, RSc));
@@ -539,11 +508,8 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
   ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(order_out, b.val[b.cur], (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
 
   // tie groups of round 0
-  {
-    KernelScope _ks(ctx, "k_mark_groups");
-    k_mark_groups<<<g256, 256, 0, st>>>(b.key[b.cur], nullptr, n, head.as<uint32_t>(), unres.as<uint32_t>());
-  }
-  ZDWB_LAUNCH_CHECK(ctx);
+  ZDWB_TRY(launch(ctx, "k_mark_groups", k_mark_groups, g256, 256, 0, b.key[b.cur], nullptr, n, head.as<uint32_t>(),
+                  unres.as<uint32_t>()));
   ZDWB_TRY(exclusive_scan_u32(ctx, unres.as<uint32_t>(), unres_scan.as<uint32_t>(), n, total.as<uint32_t>()));
   uint32_t m = 0;
   ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->meta_host, total.p, 4, cudaMemcpyDeviceToHost, st));
@@ -561,18 +527,9 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
     DevBuf head_scan;
     ZDWB_TRY(head_scan.alloc(ctx, (size_t)n * 4));
     ZDWB_TRY(exclusive_scan_u32(ctx, head.as<uint32_t>(), head_scan.as<uint32_t>(), n, nullptr));
-    {
-      KernelScope _ks(ctx, "k_group_ids");
-      k_group_ids<<<g256, 256, 0, st>>>(head.as<uint32_t>(), head_scan.as<uint32_t>(), n);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
-    {
-      KernelScope _ks(ctx, "k_compact_unresolved");
-      k_compact_unresolved<<<g256, 256, 0, st>>>(unres.as<uint32_t>(), unres_scan.as<uint32_t>(), head_scan.as<uint32_t>(),
-                                               b.val[b.cur], nullptr, n, ids.as<uint32_t>(), segA.as<uint32_t>(),
-                                               pos.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_group_ids", k_group_ids, g256, 256, 0, head.as<uint32_t>(), head_scan.as<uint32_t>(), n));
+    ZDWB_TRY(launch(ctx, "k_compact_unresolved", k_compact_unresolved, g256, 256, 0, unres.as<uint32_t>(), unres_scan.as<uint32_t>(),
+                    head_scan.as<uint32_t>(), b.val[b.cur], nullptr, n, ids.as<uint32_t>(), segA.as<uint32_t>(), pos.as<uint32_t>()));
   }
   uint32_t* pos_cur = pos.as<uint32_t>();
   uint32_t* pos_nxt = pos2.as<uint32_t>();
@@ -592,11 +549,7 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
     b.seg[1] = segB.as<uint32_t>();
     // the current group ids live in segA; make sure the record set starts in slot 0
     b.cur = 0;
-    {
-      KernelScope _ks(ctx, "k_make_keys");
-      k_make_keys<<<gm, 256, 0, st>>>(base, starts, lens, ids.as<uint32_t>(), m, off, b.key[0], b.val[0]);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_make_keys", k_make_keys, gm, 256, 0, base, starts, lens, ids.as<uint32_t>(), m, off, b.key[0], b.val[0]));
     int passes[12];
     int np = 0;
     for (int p = 0; p < 8; ++p) passes[np++] = p;
@@ -604,17 +557,10 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
     for (uint32_t p = 0; p < seg_bytes; ++p) passes[np++] = 8 + (int)p;
     ZDWB_TRY(radix_passes(ctx, b, m, passes, np, RSc));
     // write the refined order back to the positions these records occupy
-    {
-      KernelScope _ks(ctx, "k_scatter_order");
-      k_scatter_order<<<gm, 256, 0, st>>>(pos_cur, b.val[b.cur], m, order_out);
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_scatter_order", k_scatter_order, gm, 256, 0, pos_cur, b.val[b.cur], m, order_out));
     // new tie groups
-    {
-      KernelScope _ks(ctx, "k_mark_groups");
-      k_mark_groups<<<gm, 256, 0, st>>>(b.key[b.cur], b.seg[b.cur], m, head.as<uint32_t>(), unres.as<uint32_t>());
-    }
-    ZDWB_LAUNCH_CHECK(ctx);
+    ZDWB_TRY(launch(ctx, "k_mark_groups", k_mark_groups, gm, 256, 0, b.key[b.cur], b.seg[b.cur], m, head.as<uint32_t>(),
+                    unres.as<uint32_t>()));
     ZDWB_TRY(exclusive_scan_u32(ctx, unres.as<uint32_t>(), unres_scan.as<uint32_t>(), m, total.as<uint32_t>()));
     ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->meta_host, total.p, 4, cudaMemcpyDeviceToHost, st));
     ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
@@ -624,19 +570,11 @@ int sort_strings(Ctx* ctx, const uint8_t* base, const uint32_t* starts, const ui
       DevBuf head_scan;
       ZDWB_TRY(head_scan.alloc(ctx, (size_t)m * 4));
       ZDWB_TRY(exclusive_scan_u32(ctx, head.as<uint32_t>(), head_scan.as<uint32_t>(), m, nullptr));
-      {
-        KernelScope _ks(ctx, "k_group_ids");
-        k_group_ids<<<gm, 256, 0, st>>>(head.as<uint32_t>(), head_scan.as<uint32_t>(), m);
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_group_ids", k_group_ids, gm, 256, 0, head.as<uint32_t>(), head_scan.as<uint32_t>(), m));
       // compact into (ids, segA, pos_nxt).  The kernel reads none of the seg arrays (k_mark_groups, the last
       // reader of the sorted segs, is already ordered before it), so the new group ids go straight to segA.
-      {
-        KernelScope _ks(ctx, "k_compact_unresolved");
-        k_compact_unresolved<<<gm, 256, 0, st>>>(unres.as<uint32_t>(), unres_scan.as<uint32_t>(), head_scan.as<uint32_t>(),
-                                               b.val[b.cur], pos_cur, m, ids.as<uint32_t>(), segA.as<uint32_t>(), pos_nxt);
-      }
-      ZDWB_LAUNCH_CHECK(ctx);
+      ZDWB_TRY(launch(ctx, "k_compact_unresolved", k_compact_unresolved, gm, 256, 0, unres.as<uint32_t>(), unres_scan.as<uint32_t>(),
+                      head_scan.as<uint32_t>(), b.val[b.cur], pos_cur, m, ids.as<uint32_t>(), segA.as<uint32_t>(), pos_nxt));
     }
     uint32_t* t = pos_cur;
     pos_cur = pos_nxt;
