@@ -1248,7 +1248,8 @@ __device__ __forceinline__ bool warp_differ(const uint8_t* __restrict__ a, const
   return false;
 }
 
-// The open row is complete (n fields in the lists of `cur`): bitmap + rank prefix; unless it is the reference row,
+// The open row is complete (n fields in the lists of `cur`, their columns' bits in BM[cur], set while they were
+// extracted): rank prefix of the bitmap; unless it is the reference row,
 // compare with the row before (lists of cur ^ 1), hand out the records and queue the changed fields.
 // r = row number, or >= A.nrows for the spilled row (no row entry: its records only feed the dictionary and the column
 // ranges).  The changed fields are only LISTED here (record slot, column, position, length); k_pass1d_values works the
@@ -1259,7 +1260,9 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
   const unsigned lane = lane_id();
   const uint32_t BW = (P.ncols + 31u) >> 5, prv = cur ^ 1u;
   // ---- -t: trailing spaces do not belong to a field; a field of spaces only is an empty one (ConvertToZDW.cpp:295-313)
-  if (P.trim) {
+  if (P.trim) {  // (the bitmap is rebuilt from the fields that stay)
+    for (uint32_t w = lane; w < BW; w += 32u) W.BM[cur][w] = 0u;
+    __syncwarp();
     uint32_t kept = 0;
     for (uint32_t k0 = 0; k0 < n; k0 += 32u) {
       const uint32_t k = k0 + lane;
@@ -1277,30 +1280,12 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
         W.S[cur][d] = (uint16_t)s;
         W.E[cur][d] = (uint16_t)e;
         W.C[d] = (uint16_t)c;
+        atomicOr(&W.BM[cur][c >> 5], 1u << (c & 31u));
       }
       kept += (uint32_t)__popc(m);
       __syncwarp();
     }
     n = kept;
-  }
-  // ---- bitmap of the non-empty columns: the fields are in column order, so fields of one bitmap word sit side by
-  // side; a segmented OR along the lanes leaves the word's bits in the last lane of its run
-  for (uint32_t w = lane; w < BW; w += 32u) W.BM[cur][w] = 0u;
-  __syncwarp();
-  for (uint32_t k0 = 0; k0 < n; k0 += 32u) {
-    const uint32_t k = k0 + lane;
-    const bool valid = k < n;
-    const uint32_t col = valid ? (uint32_t)W.C[k] : 0xffffffffu;
-    const uint32_t w = col >> 5;
-    uint32_t v = valid ? 1u << (col & 31u) : 0u;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t uv = __shfl_up_sync(0xffffffffu, v, o), uw = __shfl_up_sync(0xffffffffu, w, o);
-      if (lane >= (unsigned)o && uw == w) v |= uv;
-    }
-    const uint32_t nw = __shfl_down_sync(0xffffffffu, w, 1);
-    if (valid && (lane == 31u || nw != w)) W.BM[cur][w] |= v;  // one lane per word and batch; batches run in turn
-    __syncwarp();
   }
   // ---- rank prefix: fields in front of every bitmap word
   {
@@ -1590,6 +1575,8 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
       row_no = pre.rows + rows_seen;
       n_ne = tabs = 0;
       cursor = pos;
+      for (uint32_t w = lane; w < BW; w += 32u) W.BM[cur][w] = 0u;  // (filled while the fields are extracted)
+      __syncwarp();
     }
     int32_t seg_end = (int32_t)DSTEP - 1;
     bool ends = false;
@@ -1646,7 +1633,9 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
           const uint32_t lowb = bj & bits_below(i);
           const int32_t fs = (lowb ? j * 32 + (31 - __clz(lowb)) : lbj) + 1;
           W.S[cur][k] = (uint16_t)(rel_sb + fs);
-          W.C[k] = (uint16_t)min(tbj + (uint32_t)__popc(tj & bits_below(i)), P.ncols - 1u);
+          const uint32_t col = min(tbj + (uint32_t)__popc(tj & bits_below(i)), P.ncols - 1u);
+          W.C[k] = (uint16_t)col;
+          atomicOr(&W.BM[cur][col >> 5], 1u << (col & 31u));
         }
       }
       n_ne += nf;
