@@ -17,6 +17,8 @@
  *        UnconvertFromZDW_Base::parseBlockHeader   UnconvertFromZDW.cpp:758-1000
  *        UnconvertFromZDW<T>::readNextRow          UnconvertFromZDW.cpp:1270-1464 (+GetWord :359-371,
  *        llutoa/lltoa :318-356, outputDefault :1224-1266) for all rows of the block
+ *   zdwb_decode_columns (no counterpart in the reference) decodes a block into typed device columns instead
+ *        of text: one int64 per cell, text as codes into the block's sorted dictionary
  *
  * Plain C types only; int status codes; no exceptions and no C++ types cross the boundary.  Outputs
  * are owned by the context and stay valid until the next call on the same context.  One context per
@@ -33,7 +35,7 @@
 extern "C" {
 #endif
 
-#define ZDWB_ABI_VERSION 4
+#define ZDWB_ABI_VERSION 5
 
 /* status codes (mapped to the reference's ERR_CODE enums by the host classes) */
 enum {
@@ -213,6 +215,52 @@ typedef struct {
  * version word (9, 10 or 11: the block layout is identical). */
 int zdwb_decode_block(zdwb_ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail,
                       const zdwb_decode_opts* opts, zdwb_rows_out* out);
+
+/* ---- columnar decode (ABI 5) -----------------------------------------------------------------
+ * zdwb_decode_columns decodes one block, like zdwb_decode_block, into an n_cols x nrows int64 matrix on the device: row k
+ * of the matrix (values + k * nrows) is file column cols[k].  A cell holds what readNextRow would print for it
+ * (UnconvertFromZDW.cpp:1349-1453), as a number.  With v the column's stored value and base its columnBase:
+ *   text-like (VARCHAR, TEXT, TINY/MEDIUM/LONGTEXT, DATETIME, CHAR_2, DECIMAL): the code of the string, i.e. the 0-based
+ *       index of the dictionary entry at offset v + base; -1 when v == 0 (the empty string; "0.000000000000" for DECIMAL).
+ *   unsigned integers: the bits of (v ? v + base : 0) (read them as uint64).
+ *   signed integers: (int64)(v ? v + base : 0).  INT64_MIN is INT64_MIN (its text is the reference's quirky one).
+ *   CHAR: the stored tuple (v ? v + base : 0): the low byte is the character, bits 8-15 the escaped one when the low byte
+ *       is '\\'; no character when the low byte is 0.
+ *   a column that is not used in the block (columnSize 0): -1 for text-like types, 0 for the others.
+ * The dictionary of a block is sorted bytewise (the reference's strcmp order), so within a block codes compare like the
+ * strings they stand for.  Codes belong to their block.  When a text-like column is selected the call also returns the
+ * dictionary: `dict` (dict_bytes bytes, the origin NUL byte included) and `entry_off` (dict_entries + 1 offsets; entry i
+ * is dict[entry_off[i] .. entry_off[i+1] - 1), entry_off[dict_entries] = dict_bytes).  Otherwise both are NULL and
+ * dict_entries is 0.
+ * Errors are those of zdwb_decode_block (ZDWB_ERR_TRUNCATED / ROW_COUNT / CORRUPT, with the same at_end_of_file rule),
+ * plus ZDWB_ERR_CORRUPT for a selected text-like column whose offset is not the start of a dictionary entry (past the
+ * dictionary, or the byte in front is not NUL: the TSV decoder prints the string's tail then, which no code expresses),
+ * and ZDWB_ERR_BAD_ARG for an empty column list, an index >= ncols or an index listed twice.
+ * Every output is device memory owned by the context, valid until the next call on it. */
+typedef struct {
+  int32_t input_on_device;   /* `zdw` is a device pointer */
+  int32_t at_end_of_file;    /* `avail` reaches the end of the file (as zdwb_decode_opts.at_end_of_file) */
+  const uint32_t* cols;      /* host memory: the file columns to decode, in the order of the output rows */
+  uint32_t n_cols;
+  uint32_t reserved;
+} zdwb_columns_opts;
+
+typedef struct {
+  const int64_t* values;     /* device: n_cols x nrows */
+  const uint8_t* dict;       /* device: the block's dictionary (NULL when no text-like column is selected) */
+  const uint64_t* entry_off; /* device: dict_entries + 1 offsets into dict (NULL when dict is) */
+  uint64_t dict_entries;
+  uint64_t dict_bytes;       /* the dictionary's size, origin byte included */
+  uint64_t consumed;         /* bytes of `zdw` this block occupied: the next block starts at zdw + consumed */
+  uint32_t nrows;            /* numRows of the block header */
+  uint32_t line_length;      /* exportFileLineLength of the block header */
+  uint8_t is_last;           /* isLastBlock */
+  uint8_t reserved[3];
+  uint32_t ncols_used;       /* columns with columnSize != 0 */
+} zdwb_columns_out;
+
+int zdwb_decode_columns(zdwb_ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail,
+                        const zdwb_columns_opts* opts, zdwb_columns_out* out);
 
 /* ---- pinned host staging (used by the host classes and the end-to-end bench) ------------------ */
 void* zdwb_host_alloc(size_t bytes);   /* cudaHostAlloc'd (pinned, usable from every device) memory, NULL on failure */

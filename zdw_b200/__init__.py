@@ -1,11 +1,14 @@
 """zdw_b200 -- B200 (sm_100a) implementation of the adobe/zdw hot path.
 
 The product is native: `libzdw_b200.so` (hand-written CUDA kernels behind the C ABI declared in
-include/zdw_b200.h) plus the C++ host classes/CLIs under zdw_b200/host.  This Python package only
-holds the ctypes binding the test-suite and bench.py use to call that ABI; it contains no compute
-and no CPU fallback.
+include/zdw_b200.h) plus the C++ host classes/CLIs under zdw_b200/host.  This Python package holds
+the ctypes binding of that ABI (capi: Context, used by the test-suite and bench.py) and a reader
+that decodes ZDW files into typed CUDA tensors (reader: read_header, read_columns; one ColumnBlock
+per block, decoded on the GPU by zdwb_decode_columns).  It contains no compute of its own and no
+CPU fallback; torch is only imported by the columnar calls.
 """
 from .capi import (  # noqa: F401
+    ColumnBlock,
     Context,
     EncodedBlock,
     DecodedBlock,
@@ -13,5 +16,7 @@ from .capi import (  # noqa: F401
     lib_path,
     load_library,
 )
+from .reader import FileHeader, read_columns, read_header  # noqa: F401
 
-__all__ = ["Context", "EncodedBlock", "DecodedBlock", "ZdwError", "lib_path", "load_library"]
+__all__ = ["Context", "EncodedBlock", "DecodedBlock", "ColumnBlock", "ZdwError", "FileHeader", "lib_path", "load_library",
+           "read_columns", "read_header"]

@@ -18,7 +18,7 @@ STATUS_NAMES = {0: "OK", 1: "ERR_CUDA", 2: "ERR_OOM", 3: "ERR_WRONG_COLUMNS", 4:
 EXPORTED_SYMBOLS = [
     "zdwb_abi_version", "zdwb_device_count", "zdwb_ctx_create", "zdwb_ctx_destroy", "zdwb_last_error", "zdwb_ctx_set_stream",
     "zdwb_ctx_set_tuning", "zdwb_ctx_kernel_launches", "zdwb_ctx_kernel_times", "zdwb_encode_block", "zdwb_decode_block", "zdwb_host_alloc",
-    "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd",
+    "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns",
 ]
 
 
@@ -71,6 +71,17 @@ class _RowsOut(C.Structure):
                 ("reserved2", C.c_uint32), ("flag_counts", C.c_void_p)]
 
 
+class _ColOpts(C.Structure):
+    _fields_ = [("input_on_device", C.c_int32), ("at_end_of_file", C.c_int32), ("cols", C.POINTER(C.c_uint32)),
+                ("n_cols", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class _ColsOut(C.Structure):
+    _fields_ = [("values", C.c_void_p), ("dict", C.c_void_p), ("entry_off", C.c_void_p), ("dict_entries", C.c_uint64),
+                ("dict_bytes", C.c_uint64), ("consumed", C.c_uint64), ("nrows", C.c_uint32), ("line_length", C.c_uint32),
+                ("is_last", C.c_uint8), ("reserved", C.c_uint8 * 3), ("ncols_used", C.c_uint32)]
+
+
 _lib = None
 
 
@@ -108,6 +119,8 @@ def load_library():
                                     C.POINTER(_BlockOut)]
     L.zdwb_decode_block.argtypes = [C.c_void_p, C.POINTER(_Schema), C.c_void_p, C.c_size_t, C.POINTER(_DecOpts),
                                     C.POINTER(_RowsOut)]
+    L.zdwb_decode_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.c_void_p, C.c_size_t, C.POINTER(_ColOpts),
+                                      C.POINTER(_ColsOut)]
     L.zdwb_host_alloc.argtypes = [C.c_size_t]
     L.zdwb_host_alloc.restype = C.c_void_p
     L.zdwb_host_free.argtypes = [C.c_void_p]
@@ -148,6 +161,65 @@ class DecodedBlock:
     flag_counts: list | None = None
 
 
+@dataclass
+class ColumnBlock:
+    """One block decoded into typed device columns (zdwb_decode_columns): row k of `values` is the k-th requested column.
+
+    values     (K, nrows) int64 CUDA tensor.  Text-like columns hold codes into this block's dictionary (-1 = no value: the
+               empty string, "0.000000000000" for DECIMAL); unsigned integers hold their bits (`.view(torch.uint64)`),
+               signed integers their value, CHAR columns the stored tuple (low byte = the character).
+    dict       uint8 CUDA tensor: the block's dictionary, origin NUL byte included (empty when no text column was asked for).
+    entry_off  int64 CUDA tensor of dict_entries + 1 offsets: entry i is dict[entry_off[i] : entry_off[i + 1] - 1].
+    The entries are sorted bytewise, so within a block codes compare like the strings.
+    """
+    values: object
+    dict: object
+    entry_off: object
+    columns: list            # file column index of every row of `values`
+    nrows: int
+    consumed: int            # bytes the block occupied: the next block starts there
+    is_last: bool
+    line_length: int
+    ncols_used: int
+
+    def strings(self, k: int) -> list:
+        """The texts of row k of `values` (a text-like column) on the host: bytes per row, None for code -1."""
+        codes = self.values[k].cpu().tolist()
+        d = bytes(self.dict.cpu().numpy().tobytes()) if self.dict.numel() else b""
+        eo = self.entry_off.cpu().tolist()
+        return [None if c < 0 else d[eo[c]:eo[c + 1] - 1] for c in codes]
+
+
+class _DeviceArray:
+    """A device range seen through __cuda_array_interface__ (so that torch can copy it)."""
+
+    def __init__(self, ptr: int, shape: tuple, typestr: str):
+        self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 3,
+                                         "strides": None, "stream": None}
+
+
+def _device_tensors(torch, device: int, copy_stream, ranges):
+    """Tensors of their own with the contents of context-owned device ranges [(ptr, shape, typestr, dtype), ...].
+
+    The context re-uses its memory at its next call, so the copies must be complete before this returns.  They run on
+    `copy_stream`, which holds nothing else, and the host waits for them there: work the caller has queued on torch's
+    current stream neither delays them nor runs after them.  The tensors are handed to the current stream afterwards
+    (record_stream), so that the caching allocator does not give their memory to the copy stream while work on the
+    current stream may still read them."""
+    cur = torch.cuda.current_stream(device)
+    out = []
+    with torch.cuda.stream(copy_stream):
+        for ptr, shape, typestr, dtype in ranges:
+            if not ptr or any(n == 0 for n in shape):
+                out.append(torch.empty(shape, dtype=dtype, device=f"cuda:{device}"))
+            else:
+                out.append(torch.as_tensor(_DeviceArray(ptr, shape, typestr), device=f"cuda:{device}").clone())
+    copy_stream.synchronize()
+    for t in out:
+        t.record_stream(cur)
+    return out
+
+
 class Context:
     """One GPU context (zdwb_ctx).  Not thread-safe; one per host thread / GPU."""
 
@@ -158,6 +230,8 @@ class Context:
         if rc != 0:
             raise ZdwError(rc, "zdwb_ctx_create failed (is a CUDA device visible? zdw_b200 has no CPU fallback)")
         self._h = h
+        self.device = device
+        self._copy_stream = None  # torch stream of the decode_columns copies (created at the first call)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -286,3 +360,38 @@ class Context:
             counts = list((C.c_uint64 * out.ncols_used).from_address(out.flag_counts))
         return DecodedBlock(tsv, int(out.tsv or 0), out.len, offs, out.nrows, out.line_length, bool(out.is_last),
                             out.consumed, out.dict_bytes, out.ncols_used, counts)
+
+    # ------------------------------------------------------------------ columnar decode
+    def decode_columns(self, types, zdw, columns, avail: int | None = None, *, input_on_device=False, at_end_of_file=True,
+                       offset: int = 0) -> ColumnBlock:
+        """Decodes the block at zdw[offset:] into typed device columns (see ColumnBlock).  columns: file column indices,
+        in the order of the output rows.  zdw: bytes-like (host) or an int device pointer (input_on_device=True, avail
+        required).  The tensors are copies, complete when this returns: they stay valid after the next call on the context,
+        whatever is queued on torch's current stream."""
+        import torch  # (only needed here: the rest of the binding works without it)
+
+        tarr = (C.c_uint8 * max(len(types), 1))(*types)
+        sch = _Schema(len(types), C.cast(tarr, C.POINTER(C.c_uint8)))
+        if input_on_device:
+            if avail is None:
+                raise ValueError("decode_columns: `avail` is required with input_on_device")
+            ptr = C.c_void_p(int(zdw) + offset)
+        else:
+            keep = zdw if isinstance(zdw, bytes) else bytes(zdw)
+            avail = len(keep) - offset if avail is None else avail
+            ptr = C.c_void_p(C.cast(C.c_char_p(keep), C.c_void_p).value + offset)
+        cols = [int(c) for c in columns]
+        carr = (C.c_uint32 * max(len(cols), 1))(*cols)
+        o = _ColOpts(int(input_on_device), int(at_end_of_file), C.cast(carr, C.POINTER(C.c_uint32)), len(cols), 0)
+        out = _ColsOut()
+        rc = self._L.zdwb_decode_columns(self._h, C.byref(sch), ptr, avail, C.byref(o), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        dev = self.device
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=dev)
+        values, dct, eo = _device_tensors(torch, dev, self._copy_stream, [
+            (out.values or 0, (len(cols), out.nrows), "<i8", torch.int64),
+            (out.dict or 0, (out.dict_bytes if out.dict else 0,), "|u1", torch.uint8),
+            (out.entry_off or 0, (out.dict_entries + 1 if out.entry_off else 0,), "<i8", torch.int64)])
+        return ColumnBlock(values, dct, eo, cols, out.nrows, out.consumed, bool(out.is_last), out.line_length, out.ncols_used)

@@ -14,6 +14,8 @@ int encode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* tsv, size
                       zdwb_block_out* out);
 int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_decode_opts* opts,
                       zdwb_rows_out* out);
+int decode_columns_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_columns_opts* opts,
+                        zdwb_columns_out* out);
 }  // namespace zdwb
 
 using zdwb::Ctx;
@@ -255,6 +257,29 @@ int zdwb_decode_block(zdwb_ctx* c, const zdwb_schema* schema, const void* zdw, s
     return ZDWB_ERR_OOM;
   } catch (...) {
     c->err = "zdwb_decode_block: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_decode_columns(zdwb_ctx* c, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_columns_opts* opts,
+                        zdwb_columns_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!schema || !out || !opts || !zdw) {
+    c->err = "zdwb_decode_columns: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::decode_columns_impl(c, schema, zdw, avail, opts, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_decode_columns: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_decode_columns: unexpected C++ exception";
     return ZDWB_ERR_CUDA;
   }
 }

@@ -19,6 +19,10 @@
 //   k_dec_rows<true>   (k_dec_write_rows) the same walk with the rendered texts kept in shared memory; every row is
 //                      assembled straight in global memory from a static template and the items' texts.
 // The row-walking kernels give a row to 32 lanes, or to 16 / 8 when the schema is narrow (several rows per warp).
+// zdwb_decode_columns shares the row-boundary discovery and the carries (strips of 32 rows), then
+//   k_dict_counts / k_dict_entries   where every dictionary entry starts (a scan over the NUL map's popcounts), so that a
+//                      text offset becomes the entry's rank (its code) in O(1)
+//   k_dec_columns      one warp per strip, one lane per row: the int64 of every selected column in every row.
 #include <algorithm>
 #include <deque>
 #include <string>
@@ -1142,6 +1146,115 @@ __global__ void __launch_bounds__(128, 8)
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// columnar decode (zdwb_decode_columns): the value every selected column holds in every row, as one int64 per cell.
+// Text-like columns become dictionary codes: the rank of the entry among the block's dictionary entries, which are
+// sorted, so codes compare like the strings.
+// ---------------------------------------------------------------------------------------------
+// An entry starts at byte p in [1, dict_total) iff byte p - 1 is NUL.  The NULs that start an entry are those at
+// q < dict_total - 1: word w of the NUL map with the others cleared.
+__device__ __forceinline__ uint32_t entry_nuls(const uint32_t* __restrict__ nulmap, uint64_t dict_total, uint64_t w) {
+  const uint64_t lim = dict_total ? dict_total - 1 : 0, b0 = w * 32;
+  if (b0 >= lim) return 0u;
+  const uint32_t m = __ldg(nulmap + w);
+  return lim - b0 >= 32 ? m : m & ((1u << (uint32_t)(lim - b0)) - 1u);
+}
+
+// cnt[w] = entries whose NUL lies in word w of the NUL map
+__global__ void k_dict_counts(const uint32_t* __restrict__ nulmap, uint64_t dict_total, uint32_t* __restrict__ cnt, uint64_t nwords) {
+  const uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (w < nwords) cnt[w] = __popc(entry_nuls(nulmap, dict_total, w));
+}
+
+// entry_off[e] = first byte of entry e (prefix = exclusive prefix of cnt); the word of the last NUL map word also writes
+// entry_off[entries] = dict_total
+__global__ void k_dict_entries(const uint32_t* __restrict__ nulmap, uint64_t dict_total, const uint32_t* __restrict__ prefix,
+                               uint64_t nwords, unsigned long long* __restrict__ entry_off) {
+  const uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= nwords) return;
+  uint32_t m = entry_nuls(nulmap, dict_total, w);
+  uint32_t e = prefix[w];
+  while (m) {
+    const uint32_t b = (uint32_t)__ffs(m) - 1u;
+    m &= m - 1u;
+    entry_off[e++] = w * 32 + b + 1;
+  }
+  if (w == nwords - 1) entry_off[e] = dict_total;
+}
+
+__device__ __forceinline__ uint32_t low_bits(uint32_t b) { return (1u << b) - 1u; }  // b < 32
+
+// flag word w of a row (flag bytes 4w .. 4w+3; bytes past the F flag bytes read as 0)
+__device__ __forceinline__ uint32_t row_flag_word(const DecParams& P, const uint8_t* __restrict__ rp, uint32_t w) {
+  uint32_t x = 0;
+#pragma unroll
+  for (uint32_t b = 0; b < 4; ++b) {
+    const uint32_t j = 4 * w + b;
+    if (j < P.F) x |= (uint32_t)__ldg(rp + j) << (8 * b);
+  }
+  return x;
+}
+
+// The int64 of a cell of used column u holding stored value v (include/zdw_b200.h, zdwb_decode_columns).  A text offset
+// that is not the start of a dictionary entry sets meta->err.
+__device__ __forceinline__ unsigned long long column_cell(const DecParams& P, uint32_t u, unsigned long long v,
+                                                          const uint32_t* __restrict__ dict_prefix, DecMeta* meta) {
+  if (!is_text_like(P.utype[u])) return v ? v + P.ubase[u] : 0ull;
+  if (v == 0) return ~0ull;  // -1: no value
+  const uint32_t o = (uint32_t)(v + P.ubase[u]);  // ULONG index, UnconvertFromZDW.cpp:1363
+  if (o == 0 || (uint64_t)o >= P.dict_total || !((__ldg(P.nulmap + ((o - 1) >> 5)) >> ((o - 1) & 31u)) & 1u)) {
+    meta->err = 1;
+    return ~0ull;
+  }
+  return (unsigned long long)(__ldg(dict_prefix + (o >> 5)) + __popc(__ldg(P.nulmap + (o >> 5)) & low_bits(o & 31u)) - 1u);
+}
+
+// One warp per strip of 32 rows, one lane per row.  A lane walks the selected used columns in ascending order and keeps
+// the offset of the next value in its row from popcounts of its flag bits against the width bit planes.  A row whose
+// flag bit is clear takes the value of the nearest lane in front that has one (a ballot and one shuffle), or the
+// strip's carry-in.  The warp stores the 32 rows of a column side by side: 256 bytes per column and strip.
+__global__ void __launch_bounds__(DEC_THREADS)
+    k_dec_columns(const DecParams P, const uint32_t* __restrict__ row_off, const unsigned long long* __restrict__ cin,
+                  const uint32_t* __restrict__ sel_u, const uint32_t* __restrict__ sel_k, uint32_t n_sel,
+                  const uint32_t* __restrict__ dict_prefix, unsigned long long* __restrict__ values, DecMeta* __restrict__ meta) {
+  const unsigned lane = lane_id();
+  const uint32_t strip = blockIdx.x * DEC_WARPS + (threadIdx.x >> 5);
+  const uint32_t r0 = strip * 32;
+  if (r0 >= P.nrows) return;  // (the whole warp)
+  const uint32_t r = r0 + lane;
+  const bool live = r < P.nrows;
+  const uint8_t* rp = P.blk + P.rows_base + (live ? row_off[r] : 0u);
+  const unsigned le = lanemask_lt() | (1u << lane);
+  uint32_t voff = P.F;  // offset of the next value in the row
+  uint32_t cw = 0;      // flag word of the walk, its bits below `from` are counted in voff
+  uint32_t from = 0;
+  uint32_t fw = live ? row_flag_word(P, rp, 0) : 0u;
+  uint32_t pl0 = __ldg(P.planes), pl1 = __ldg(P.planes + P.W), pl2 = __ldg(P.planes + 2 * P.W), pl3 = __ldg(P.planes + 3 * P.W);
+  auto widths = [&](uint32_t m) { return __popc(m & pl0) + 2u * __popc(m & pl1) + 4u * __popc(m & pl2) + 8u * __popc(m & pl3); };
+  for (uint32_t j = 0; j < n_sel; ++j) {
+    const uint32_t u = __ldg(sel_u + j);
+    const uint32_t w = u >> 5, b = u & 31u;
+    while (cw < w) {
+      voff += widths(fw & ~low_bits(from));
+      ++cw;
+      from = 0;
+      fw = live ? row_flag_word(P, rp, cw) : 0u;
+      pl0 = __ldg(P.planes + cw);
+      pl1 = __ldg(P.planes + P.W + cw);
+      pl2 = __ldg(P.planes + 2 * P.W + cw);
+      pl3 = __ldg(P.planes + 3 * P.W + cw);
+    }
+    voff += widths(fw & low_bits(b) & ~low_bits(from));
+    from = b;
+    const bool has = (fw >> b) & 1u;
+    unsigned long long v = has ? load_le(rp + voff, P.usz[u]) : 0ull;
+    const unsigned src = __ballot_sync(0xffffffffu, has) & le;
+    v = __shfl_sync(0xffffffffu, v, src ? 31 - __clz(src) : lane);
+    if (!src) v = cin[(size_t)strip * P.U + u];
+    if (live) values[(size_t)__ldg(sel_k + j) * P.nrows + r] = column_cell(P, u, v, dict_prefix, meta);
+  }
+}
+
 struct HostBlockHeader {
   uint32_t nrows = 0, line_len = 0;
   uint8_t last = 0, idx_size = 0;
@@ -1213,13 +1326,29 @@ int with_lanes(uint32_t lanes, F f) {
   return f(std::integral_constant<int, 32>());
 }
 
-}  // namespace
+// ---------------------------------------------------------------------------------------------
+// front end of both decoders (zdwb_decode_block, zdwb_decode_columns): the block header and the used-column tables
+// (dec_read_header), the block on the device with the tables and the dictionary's NUL map (dec_upload), the offset of
+// every row (dec_find_rows)
+// ---------------------------------------------------------------------------------------------
+struct DecFront {
+  HostBlockHeader H;
+  std::vector<uint32_t> used_cols;          // file column of every used column
+  std::vector<uint8_t> usz, utype;          // [U]
+  std::vector<unsigned long long> ubase;    // [U]
+  uint32_t U = 0, F = 0, W = 0, M = 0;
+  uint64_t rows_base = 0;
+  const uint8_t* src = nullptr;             // the caller's block
+  bool in_dev = false;
+  uint64_t avail = 0;
+  uint64_t win = 0;                         // row-stream bytes on the device
+  // (released in reverse order: the buffers a caller allocates afterwards go first)
+  DevBuf blk_dev, d_usz, d_ubase, d_utype, d_planes, d_meta, d_nulmap;
+  DecParams P;
+  DecMeta* meta = nullptr;
+};
 
-int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_decode_opts* opts,
-                      zdwb_rows_out* out) {
-  memset(out, 0, sizeof(*out));
-  ZDWB_TRY(call_begin(ctx));
-  cudaStream_t st = ctx->stream;
+int dec_read_header(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, bool in_dev, DecFront& D) {
   const uint32_t nc = schema->ncols;
   if (nc == 0 || !schema->types) {
     ctx->err = "decode: schema has no columns";
@@ -1231,11 +1360,13 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
       return ZDWB_ERR_UNSUPPORTED;
     }
   }
-  const bool in_dev = opts->input_on_device != 0;
   const uint8_t* src = static_cast<const uint8_t*>(zdw);
+  D.src = src;
+  D.in_dev = in_dev;
+  D.avail = avail;
 
   // ---- block header (readLineLength :782-810, readDictionary :812-846, readColumnFieldStats :966-1000)
-  HostBlockHeader H;
+  HostBlockHeader& H = D.H;
   uint8_t head[16];
   ZDWB_TRY(fetch(ctx, src, in_dev, avail, 0, head, 10));
   memcpy(&H.nrows, head, 4);
@@ -1261,34 +1392,41 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   }
   std::vector<uint8_t> csize(nc);
   ZDWB_TRY(fetch(ctx, src, in_dev, avail, H.stats_base, csize.data(), nc));
-  std::vector<uint32_t> used_cols;
+  std::vector<uint32_t>& used_cols = D.used_cols;
   for (uint32_t c = 0; c < nc; ++c)
     if (csize[c]) used_cols.push_back(c);
   const uint32_t U = (uint32_t)used_cols.size();
-  std::vector<unsigned long long> ubase(U ? U : 1);
-  if (U) ZDWB_TRY(fetch(ctx, src, in_dev, avail, H.stats_base + nc, ubase.data(), (size_t)U * 8));
-  const uint64_t rows_base = H.stats_base + nc + 8ull * U;
-  const uint32_t F = (U + 7) / 8, W = (F + 3) / 4;
-  std::vector<uint8_t> usz(U ? U : 1), utype(U ? U : 1);
-  uint32_t M = F;
+  D.ubase.assign(U ? U : 1, 0ull);
+  if (U) ZDWB_TRY(fetch(ctx, src, in_dev, avail, H.stats_base + nc, D.ubase.data(), (size_t)U * 8));
+  D.rows_base = H.stats_base + nc + 8ull * U;
+  D.U = U;
+  D.F = (U + 7) / 8;
+  D.W = (D.F + 3) / 4;
+  D.usz.assign(U ? U : 1, 0);
+  D.utype.assign(U ? U : 1, 0);
+  D.M = D.F;
   for (uint32_t u = 0; u < U; ++u) {
-    usz[u] = csize[used_cols[u]];
-    if (usz[u] > 8) {
+    D.usz[u] = csize[used_cols[u]];
+    if (D.usz[u] > 8) {
       ctx->err = "decode: column size > 8";
       return ZDWB_ERR_CORRUPT;
     }
-    utype[u] = schema->types[used_cols[u]];
-    M += usz[u];
+    D.utype[u] = schema->types[used_cols[u]];
+    D.M += D.usz[u];
   }
-  out->nrows = H.nrows;
-  out->line_length = H.line_len;
-  out->is_last = H.last;
-  out->dict_bytes = H.dict_total;
-  out->ncols_used = U;
-  const uint32_t nrows = H.nrows;
+  return ZDWB_OK;
+}
+
+int dec_upload(Ctx* ctx, bool at_end_of_file, DecFront& D) {
+  cudaStream_t st = ctx->stream;
+  const HostBlockHeader& H = D.H;
+  const uint32_t U = D.U, F = D.F, W = D.W, M = D.M, nrows = H.nrows;
+  const uint64_t rows_base = D.rows_base, avail = D.avail;
+  const bool in_dev = D.in_dev;
+  const uint8_t* src = D.src;
 
   // zero-byte rows at the very end of the file are never read by the reference (input->eof(), :1577)
-  if (U == 0 && nrows > 0 && opts->at_end_of_file && rows_base >= avail) {
+  if (U == 0 && nrows > 0 && at_end_of_file && rows_base >= avail) {
     ctx->err = "Rows unpacked (0) does not match expected (" + std::to_string(nrows) + ")";
     return ZDWB_ERR_ROW_COUNT;
   }
@@ -1299,23 +1437,23 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
     ctx->err = "decode: a block's row stream must be smaller than 4 GiB";
     return ZDWB_ERR_UNSUPPORTED;
   }
-  DevBuf blk_dev;
+  D.win = win;
   const uint8_t* blk;
   if (in_dev) {
     blk = src;
   } else {
     const uint64_t need = rows_base + win;
-    ZDWB_TRY(blk_dev.alloc(ctx, need + 64));
+    ZDWB_TRY(D.blk_dev.alloc(ctx, need + 64));
     if (need >= ((uint64_t)32 << 20) && is_pageable_host(src)) {  // (see encode_block_impl: pageable memory goes through the pinned ring)
       const uint8_t* from = src;
-      ZDWB_TRY(ring_h2d(ctx, blk_dev.p, (size_t)need, [from](void* dst, size_t off, size_t k) {
+      ZDWB_TRY(ring_h2d(ctx, D.blk_dev.p, (size_t)need, [from](void* dst, size_t off, size_t k) {
         memcpy(dst, from + off, k);
         return true;
       }));
     } else {
-      ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(blk_dev.p, src, need, cudaMemcpyHostToDevice, st));
+      ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(D.blk_dev.p, src, need, cudaMemcpyHostToDevice, st));
     }
-    blk = blk_dev.as<uint8_t>();
+    blk = D.blk_dev.as<uint8_t>();
   }
   const uint64_t dev_avail = in_dev ? avail : rows_base + win;
 
@@ -1323,18 +1461,17 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   std::vector<uint32_t> planes((size_t)4 * (W ? W : 1), 0);
   for (uint32_t u = 0; u < U; ++u) {
     for (uint32_t k = 0; k < 4; ++k)
-      if (usz[u] & (1u << k)) planes[(size_t)k * W + u / 32] |= 1u << (u % 32);
+      if (D.usz[u] & (1u << k)) planes[(size_t)k * W + u / 32] |= 1u << (u % 32);
   }
-  DevBuf d_usz, d_ubase, d_utype, d_planes, d_meta;
-  ZDWB_TRY(upload(ctx, d_usz, usz));
-  ZDWB_TRY(upload(ctx, d_ubase, ubase));
-  ZDWB_TRY(upload(ctx, d_utype, utype));
-  ZDWB_TRY(upload(ctx, d_planes, planes));
-  ZDWB_TRY(d_meta.alloc(ctx, sizeof(DecMeta)));
-  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(d_meta.p, 0, sizeof(DecMeta), st));
-  DecMeta* meta = d_meta.as<DecMeta>();
+  ZDWB_TRY(upload(ctx, D.d_usz, D.usz));
+  ZDWB_TRY(upload(ctx, D.d_ubase, D.ubase));
+  ZDWB_TRY(upload(ctx, D.d_utype, D.utype));
+  ZDWB_TRY(upload(ctx, D.d_planes, planes));
+  ZDWB_TRY(D.d_meta.alloc(ctx, sizeof(DecMeta)));
+  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(D.d_meta.p, 0, sizeof(DecMeta), st));
+  D.meta = D.d_meta.as<DecMeta>();
 
-  DecParams P;
+  DecParams& P = D.P;
   P.blk = blk;
   P.avail = dev_avail;
   P.rows_base = rows_base;
@@ -1345,19 +1482,118 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   P.F = F;
   P.M = M;
   P.W = W;
-  P.usz = d_usz.as<uint8_t>();
-  P.ubase = d_ubase.as<unsigned long long>();
-  P.utype = d_utype.as<uint8_t>();
-  P.planes = d_planes.as<uint32_t>();
+  P.usz = D.d_usz.as<uint8_t>();
+  P.ubase = D.d_ubase.as<unsigned long long>();
+  P.utype = D.d_utype.as<uint8_t>();
+  P.planes = D.d_planes.as<uint32_t>();
   // NUL bitmap of the dictionary: the length of any entry is then one or two word loads
-  DevBuf d_nulmap;
   {
     const uint64_t nwords = (H.dict_total + 31) / 32 + 1;
-    ZDWB_TRY(d_nulmap.alloc(ctx, nwords * 4));
+    ZDWB_TRY(D.d_nulmap.alloc(ctx, nwords * 4));
     ZDWB_TRY(launch(ctx, "k_dict_nulmap", k_dict_nulmap, (unsigned)((nwords + 255) / 256), 256, 0, blk + H.dict_base, H.dict_total,
-                    d_nulmap.as<uint32_t>(), nwords));
+                    D.d_nulmap.as<uint32_t>(), nwords));
   }
-  P.nulmap = d_nulmap.as<uint32_t>();
+  P.nulmap = D.d_nulmap.as<uint32_t>();
+  return ZDWB_OK;
+}
+
+// row_off[r] = offset of row r in the row stream (r <= nrows; nrows > 0), found with GL lanes per tile; *consumed_stream =
+// where the rows end.  ZDWB_ERR_ROW_COUNT / ZDWB_ERR_TRUNCATED when the data ends before nrows rows do.
+int dec_find_rows(Ctx* ctx, const DecFront& D, uint32_t GL, bool at_end_of_file, DevBuf& row_off, uint64_t* consumed_stream) {
+  cudaStream_t st = ctx->stream;
+  const DecParams& P = D.P;
+  const uint32_t nrows = D.H.nrows, U = D.U, M = D.M, W = D.W;
+  const uint64_t win = D.win;
+  ZDWB_TRY(row_off.alloc(ctx, ((size_t)nrows + 1) * 4));
+  *consumed_stream = 0;
+  if (U == 0) {
+    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(row_off.p, 0, ((size_t)nrows + 1) * 4, st));
+    return ZDWB_OK;
+  }
+  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(row_off.p, 0xff, ((size_t)nrows + 1) * 4, st));
+  uint32_t T = (uint32_t)std::max<long long>(256, std::min<long long>(ctx->dec_tile_bytes, 32768));
+  T &= ~3u;
+  // every row occupies at least F bytes, so tiles beyond nrows*M never matter; +1 tile for the end mark
+  const uint32_t ntiles = (uint32_t)(win / T) + 1;
+  DevBuf maps0;
+  ZDWB_TRY(maps0.alloc(ctx, (size_t)ntiles * M * 8));
+  const size_t smem_maps = (size_t)T * 4 + ((T + 4 * W + 8) / 4) * 4 + (size_t)4 * W * 4 + 16;
+  if (smem_maps > 200 * 1024) {
+    ctx->err = "decode: too many used columns for the row-boundary kernel";
+    return ZDWB_ERR_UNSUPPORTED;
+  }
+  ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_dec_tile_maps, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  ZDWB_TRY(launch(ctx, "k_dec_tile_maps", k_dec_tile_maps, ntiles, DEC_THREADS, smem_maps, P, win, T, maps0.as<uint64_t>()));
+  // up-sweep: compose groups of G maps until one remains
+  const uint32_t G = 32;
+  std::deque<DevBuf> owned;     // the levels above the tile maps and the entry states (a deque: they stay in place)
+  std::vector<DevBuf*> levels;  // levels[0] = tile maps
+  std::vector<uint32_t> counts;
+  levels.push_back(&maps0);
+  counts.push_back(ntiles);
+  while (counts.back() > 1) {
+    const uint32_t n_in = counts.back();
+    const uint32_t n_out = (n_in + G - 1) / G;
+    DevBuf& nb = owned.emplace_back();
+    ZDWB_TRY(nb.alloc(ctx, (size_t)n_out * M * 8));
+    ZDWB_TRY(launch(ctx, "k_dec_compose", k_dec_compose, n_out, DEC_THREADS, 0, levels.back()->as<uint64_t>(), n_in, M, G,
+                    nb.as<uint64_t>()));
+    levels.push_back(&nb);
+    counts.push_back(n_out);
+  }
+  // down-sweep: entry state of every node, from the single root (rows = 0, offset = 0) to the tiles
+  DevBuf* ent_parent = &owned.emplace_back();
+  ZDWB_TRY(ent_parent->alloc(ctx, 8));
+  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(ent_parent->p, 0, 8, st));
+  for (int lv = (int)levels.size() - 2; lv >= 0; --lv) {
+    const uint32_t n_in = counts[lv], n_parent = counts[lv + 1];
+    DevBuf& ec = owned.emplace_back();
+    ZDWB_TRY(ec.alloc(ctx, (size_t)n_in * 8));
+    ZDWB_TRY(launch(ctx, "k_dec_descend", k_dec_descend, (n_parent + 127) / 128, 128, 0, levels[lv]->as<uint64_t>(), n_in, M, G,
+                    ent_parent->as<uint64_t>(), n_parent, ec.as<uint64_t>()));
+    ent_parent = &ec;
+  }
+  // with a single tile the root entry is the tile entry
+  const uint32_t per_cta = DEC_WARPS * (32 / GL);
+  const unsigned grid = (ntiles + per_cta - 1) / per_cta;
+  ZDWB_TRY(with_lanes(GL, [&](auto g) {
+    return launch(ctx, "k_dec_row_starts", k_dec_row_starts<decltype(g)::value>, grid, DEC_THREADS, 0, P, T, ntiles,
+                  ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
+  }));
+  ZDWB_CUDA_TRY(ctx, readback_small(ctx, ctx->meta_host, row_off.as<uint32_t>() + nrows, 4));
+  ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  const uint32_t h_end = *static_cast<uint32_t*>(ctx->meta_host);
+  if (h_end == 0xffffffffu || (uint64_t)h_end > win) {
+    // the data ends before `nrows` rows do
+    ctx->err = "decode: block truncated (fewer rows than the header promises)";
+    return at_end_of_file ? ZDWB_ERR_ROW_COUNT : ZDWB_ERR_TRUNCATED;
+  }
+  *consumed_stream = h_end;
+  return ZDWB_OK;
+}
+
+}  // namespace
+
+int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_decode_opts* opts,
+                      zdwb_rows_out* out) {
+  memset(out, 0, sizeof(*out));
+  ZDWB_TRY(call_begin(ctx));
+  cudaStream_t st = ctx->stream;
+  DecFront D;
+  ZDWB_TRY(dec_read_header(ctx, schema, zdw, avail, opts->input_on_device != 0, D));
+  const uint32_t nc = schema->ncols;
+  const HostBlockHeader& H = D.H;
+  const std::vector<uint32_t>& used_cols = D.used_cols;
+  const uint32_t U = D.U, F = D.F;
+  out->nrows = H.nrows;
+  out->line_length = H.line_len;
+  out->is_last = H.last;
+  out->dict_bytes = H.dict_total;
+  out->ncols_used = U;
+  const uint32_t nrows = H.nrows;
+  ZDWB_TRY(dec_upload(ctx, opts->at_end_of_file != 0, D));
+  const DecParams& P = D.P;
+  DecMeta* meta = D.meta;
 
   // ---- output plan: static segments and dynamic items in output order
   const uint8_t sep = opts->separator;
@@ -1459,78 +1695,15 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   ZDWB_TRY(upload(ctx, d_u_item, u_item));
 
   if (nrows == 0) {
-    out->consumed = rows_base;
+    out->consumed = D.rows_base;
     return ZDWB_OK;
   }
 
   // ---- row starts
   DevBuf row_off;
-  ZDWB_TRY(row_off.alloc(ctx, ((size_t)nrows + 1) * 4));
   uint64_t consumed_stream = 0;
-  if (U == 0) {
-    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(row_off.p, 0, ((size_t)nrows + 1) * 4, st));
-  } else {
-    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(row_off.p, 0xff, ((size_t)nrows + 1) * 4, st));
-    uint32_t T = (uint32_t)std::max<long long>(256, std::min<long long>(ctx->dec_tile_bytes, 32768));
-    T &= ~3u;
-    // every row occupies at least F bytes, so tiles beyond nrows*M never matter; +1 tile for the end mark
-    const uint32_t ntiles = (uint32_t)(win / T) + 1;
-    DevBuf maps0;
-    ZDWB_TRY(maps0.alloc(ctx, (size_t)ntiles * M * 8));
-    const size_t smem_maps = (size_t)T * 4 + ((T + 4 * W + 8) / 4) * 4 + (size_t)4 * W * 4 + 16;
-    if (smem_maps > 200 * 1024) {
-      ctx->err = "decode: too many used columns for the row-boundary kernel";
-      return ZDWB_ERR_UNSUPPORTED;
-    }
-    ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_dec_tile_maps, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    ZDWB_TRY(launch(ctx, "k_dec_tile_maps", k_dec_tile_maps, ntiles, DEC_THREADS, smem_maps, P, win, T, maps0.as<uint64_t>()));
-    // up-sweep: compose groups of G maps until one remains
-    const uint32_t G = 32;
-    std::deque<DevBuf> owned;     // the levels above the tile maps and the entry states (a deque: they stay in place)
-    std::vector<DevBuf*> levels;  // levels[0] = tile maps
-    std::vector<uint32_t> counts;
-    levels.push_back(&maps0);
-    counts.push_back(ntiles);
-    while (counts.back() > 1) {
-      const uint32_t n_in = counts.back();
-      const uint32_t n_out = (n_in + G - 1) / G;
-      DevBuf& nb = owned.emplace_back();
-      ZDWB_TRY(nb.alloc(ctx, (size_t)n_out * M * 8));
-      ZDWB_TRY(launch(ctx, "k_dec_compose", k_dec_compose, n_out, DEC_THREADS, 0, levels.back()->as<uint64_t>(), n_in, M, G,
-                      nb.as<uint64_t>()));
-      levels.push_back(&nb);
-      counts.push_back(n_out);
-    }
-    // down-sweep: entry state of every node, from the single root (rows = 0, offset = 0) to the tiles
-    DevBuf* ent_parent = &owned.emplace_back();
-    ZDWB_TRY(ent_parent->alloc(ctx, 8));
-    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(ent_parent->p, 0, 8, st));
-    for (int lv = (int)levels.size() - 2; lv >= 0; --lv) {
-      const uint32_t n_in = counts[lv], n_parent = counts[lv + 1];
-      DevBuf& ec = owned.emplace_back();
-      ZDWB_TRY(ec.alloc(ctx, (size_t)n_in * 8));
-      ZDWB_TRY(launch(ctx, "k_dec_descend", k_dec_descend, (n_parent + 127) / 128, 128, 0, levels[lv]->as<uint64_t>(), n_in, M, G,
-                      ent_parent->as<uint64_t>(), n_parent, ec.as<uint64_t>()));
-      ent_parent = &ec;
-    }
-    // with a single tile the root entry is the tile entry
-    const uint32_t per_cta = DEC_WARPS * (32 / GL);
-    const unsigned grid = (ntiles + per_cta - 1) / per_cta;
-    ZDWB_TRY(with_lanes(GL, [&](auto g) {
-      return launch(ctx, "k_dec_row_starts", k_dec_row_starts<decltype(g)::value>, grid, DEC_THREADS, 0, P, T, ntiles,
-                    ent_parent->as<uint64_t>(), row_off.as<uint32_t>());
-    }));
-    ZDWB_CUDA_TRY(ctx, readback_small(ctx, ctx->meta_host, row_off.as<uint32_t>() + nrows, 4));
-    ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    const uint32_t h_end = *static_cast<uint32_t*>(ctx->meta_host);
-    if (h_end == 0xffffffffu || (uint64_t)h_end > win) {
-      // the data ends before `nrows` rows do
-      ctx->err = "decode: block truncated (fewer rows than the header promises)";
-      return opts->at_end_of_file ? ZDWB_ERR_ROW_COUNT : ZDWB_ERR_TRUNCATED;
-    }
-    consumed_stream = h_end;
-  }
-  out->consumed = rows_base + consumed_stream;
+  ZDWB_TRY(dec_find_rows(ctx, D, GL, opts->at_end_of_file != 0, row_off, &consumed_stream));
+  out->consumed = D.rows_base + consumed_stream;
   if (opts->skim_only) return ZDWB_OK;  // the caller only wanted to know where the next block starts
 
   // ---- strips: one warp walks RS consecutive rows (k_dec_rows); about four waves of warps over the GPU
@@ -1769,6 +1942,144 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
   }
   ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   out->tsv = static_cast<const uint8_t*>(ctx->out_host);
+  return ZDWB_OK;
+}
+
+
+int decode_columns_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_columns_opts* opts,
+                        zdwb_columns_out* out) {
+  memset(out, 0, sizeof(*out));
+  ZDWB_TRY(call_begin(ctx));
+  cudaStream_t st = ctx->stream;
+  const uint32_t nc = schema->ncols, K = opts->n_cols;
+  if (K == 0 || !opts->cols) {
+    ctx->err = "decode_columns: empty column list";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  {
+    std::vector<uint8_t> seen(nc, 0);
+    for (uint32_t k = 0; k < K; ++k) {
+      const uint32_t c = opts->cols[k];
+      if (c >= nc) {
+        ctx->err = "decode_columns: column index " + std::to_string(c) + " out of range (the schema has " + std::to_string(nc) + ")";
+        return ZDWB_ERR_BAD_ARG;
+      }
+      if (seen[c]) {
+        ctx->err = "decode_columns: column " + std::to_string(c) + " listed twice";
+        return ZDWB_ERR_BAD_ARG;
+      }
+      seen[c] = 1;
+    }
+  }
+  DecFront D;
+  ZDWB_TRY(dec_read_header(ctx, schema, zdw, avail, opts->input_on_device != 0, D));
+  const HostBlockHeader& H = D.H;
+  const uint32_t U = D.U, F = D.F, nrows = H.nrows;
+  out->nrows = nrows;
+  out->line_length = H.line_len;
+  out->is_last = H.last;
+  out->dict_bytes = H.dict_total;
+  out->ncols_used = U;
+  ZDWB_TRY(dec_upload(ctx, opts->at_end_of_file != 0, D));
+  const DecParams& P = D.P;
+
+  // ---- the selected used columns in ascending order (sel_u) with their output rows (sel_k); unused ones are filled
+  std::vector<int32_t> used_idx(nc, -1);
+  for (uint32_t u = 0; u < U; ++u) used_idx[D.used_cols[u]] = (int32_t)u;
+  std::vector<std::pair<uint32_t, uint32_t>> sel;
+  bool want_dict = false;
+  for (uint32_t k = 0; k < K; ++k) {
+    const uint32_t c = opts->cols[k];
+    if (is_text_like(schema->types[c])) want_dict = true;
+    if (used_idx[c] >= 0) sel.emplace_back((uint32_t)used_idx[c], k);
+  }
+  std::sort(sel.begin(), sel.end());
+  std::vector<uint32_t> sel_u(sel.size()), sel_k(sel.size());
+  for (size_t j = 0; j < sel.size(); ++j) {
+    sel_u[j] = sel[j].first;
+    sel_k[j] = sel[j].second;
+  }
+
+  // ---- outputs: the values, and with a text-like column the dictionary and where its entries start
+  unsigned long long* values;
+  {
+    DevBuf vb;
+    ZDWB_TRY(vb.alloc(ctx, (size_t)K * nrows * 8 + 16));
+    values = static_cast<unsigned long long*>(vb.detach());
+  }
+  const uint64_t nwords = (H.dict_total + 31) / 32 + 1;  // words of the NUL map
+  DevBuf dict_prefix;
+  uint32_t* h_entries = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(ctx->meta_host) + 2048);
+  if (want_dict) {
+    DevBuf db;
+    ZDWB_TRY(db.alloc(ctx, H.dict_total + 16));
+    if (H.dict_total) ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(db.p, P.blk + H.dict_base, H.dict_total, cudaMemcpyDeviceToDevice, st));
+    out->dict = static_cast<const uint8_t*>(db.detach());
+    DevBuf d_total;
+    ZDWB_TRY(d_total.alloc(ctx, 4));
+    ZDWB_TRY(dict_prefix.alloc(ctx, nwords * 4));
+    ZDWB_TRY(launch(ctx, "k_dict_counts", k_dict_counts, (unsigned)((nwords + 255) / 256), 256, 0, P.nulmap, H.dict_total,
+                    dict_prefix.as<uint32_t>(), nwords));
+    ZDWB_TRY(exclusive_scan_u32(ctx, dict_prefix.as<uint32_t>(), dict_prefix.as<uint32_t>(), nwords, d_total.as<uint32_t>()));
+    ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(h_entries, d_total.p, 4, cudaMemcpyDeviceToHost, st));
+  }
+
+  // ---- row starts: lanes per row by the width of the flag bytes, as in zdwb_decode_block
+  const uint32_t GL = (ctx->dec_group_lanes == 8 || ctx->dec_group_lanes == 16 || ctx->dec_group_lanes == 32)
+                          ? (uint32_t)ctx->dec_group_lanes
+                          : F <= 8 ? 8u : F <= 16 ? 16u : 32u;
+  DevBuf row_off;
+  uint64_t consumed_stream = 0;
+  if (nrows) ZDWB_TRY(dec_find_rows(ctx, D, GL, opts->at_end_of_file != 0, row_off, &consumed_stream));
+  out->consumed = D.rows_base + consumed_stream;
+
+  if (want_dict) {
+    ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));  // (the number of entries)
+    const uint64_t n = *h_entries;
+    DevBuf eb;
+    ZDWB_TRY(eb.alloc(ctx, (n + 1) * 8));
+    ZDWB_TRY(launch(ctx, "k_dict_entries", k_dict_entries, (unsigned)((nwords + 255) / 256), 256, 0, P.nulmap, H.dict_total,
+                    dict_prefix.as<uint32_t>(), nwords, eb.as<unsigned long long>()));
+    out->entry_off = static_cast<const uint64_t*>(eb.detach());
+    out->dict_entries = n;
+  }
+  if (nrows) {
+    // a column the block does not use holds its type's default in every row
+    for (uint32_t k = 0; k < K; ++k) {
+      const uint32_t c = opts->cols[k];
+      if (used_idx[c] < 0)
+        ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(values + (size_t)k * nrows, is_text_like(schema->types[c]) ? 0xff : 0, (size_t)nrows * 8, st));
+    }
+  }
+  if (nrows && !sel.empty()) {
+    // ---- strips of 32 rows: the value every used column holds where a strip begins, then one warp per strip
+    const uint32_t R = 32, nstrips = (nrows + R - 1) / R;
+    DevBuf cin, sval, shas, d_sel_u, d_sel_k;
+    ZDWB_TRY(cin.alloc(ctx, (size_t)nstrips * U * 8));
+    ZDWB_TRY(sval.alloc(ctx, (size_t)nstrips * U * 8));
+    ZDWB_TRY(shas.alloc(ctx, (size_t)nstrips * U));
+    const size_t smem_sum = (size_t)U * 4 + 16;
+    ZDWB_TRY(with_lanes(GL, [&](auto g) -> int {
+      auto k = k_dec_strip_summary<decltype(g)::value>;
+      ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      return launch(ctx, "k_dec_strip_summary", k, nstrips, DEC_THREADS, smem_sum, P, row_off.as<uint32_t>(), R, 0,
+                    (unsigned long long*)nullptr, sval.as<unsigned long long>(), shas.as<uint8_t>(), D.meta);
+    }));
+    ZDWB_TRY(carry_prefix(ctx, sval.as<unsigned long long>(), shas.as<uint8_t>(), nstrips, U, cin.as<unsigned long long>()));
+    ZDWB_TRY(upload(ctx, d_sel_u, sel_u));
+    ZDWB_TRY(upload(ctx, d_sel_k, sel_k));
+    ZDWB_TRY(launch(ctx, "k_dec_columns", k_dec_columns, (nstrips + DEC_WARPS - 1) / DEC_WARPS, DEC_THREADS, 0, P,
+                    row_off.as<uint32_t>(), cin.as<unsigned long long>(), d_sel_u.as<uint32_t>(), d_sel_k.as<uint32_t>(),
+                    (uint32_t)sel.size(), dict_prefix.as<uint32_t>(), values, D.meta));
+  }
+  DecMeta* hm = static_cast<DecMeta*>(ctx->meta_host);
+  ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hm, D.meta, sizeof(DecMeta), cudaMemcpyDeviceToHost, st));
+  ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  if (hm->err) {
+    ctx->err = "decode_columns: a text value's dictionary offset is not the start of an entry";
+    return ZDWB_ERR_CORRUPT;
+  }
+  out->values = reinterpret_cast<const int64_t*>(values);
   return ZDWB_OK;
 }
 
