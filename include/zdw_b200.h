@@ -19,6 +19,8 @@
  *        llutoa/lltoa :318-356, outputDefault :1224-1266) for all rows of the block
  *   zdwb_decode_columns (no counterpart in the reference) decodes a block into typed device columns instead
  *        of text: one int64 per cell, text as codes into the block's sorted dictionary
+ *   zdwb_merge_codes (no counterpart either) merges the dictionaries of many blocks into one sorted dictionary and
+ *        re-codes their codes into it
  *
  * Plain C types only; int status codes; no exceptions and no C++ types cross the boundary.  Outputs
  * are owned by the context and stay valid until the next call on the same context.  One context per
@@ -85,7 +87,8 @@ int zdwb_ctx_set_stream(zdwb_ctx* ctx, void* cuda_stream);
  * width), "dec_tile_bytes" (row-stream bytes per CTA in the row-boundary discovery).  Both: "copy_gate" (0/1, default
  * 1: host<->device copies of 8 MiB and more
  * take turns with those of the process's other contexts on the same device instead of sharing the link),
- * "kernel_timing" (0/1).  Returns ZDWB_ERR_BAD_ARG for unknown names. */
+ * "kernel_timing" (0/1).  Merge: "merge_max_refs" (most referenced entries zdwb_merge_codes accepts, default and
+ * ceiling 2^32 - 1; lower values let a test reach ZDWB_ERR_UNSUPPORTED).  Returns ZDWB_ERR_BAD_ARG for unknown names. */
 int zdwb_ctx_set_tuning(zdwb_ctx* ctx, const char* name, long long value);
 
 /* Number of kernels this context has launched so far (bench.py reports the delta as gpu_launches). */
@@ -261,6 +264,47 @@ typedef struct {
 
 int zdwb_decode_columns(zdwb_ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail,
                         const zdwb_columns_opts* opts, zdwb_columns_out* out);
+
+/* ---- merged dictionaries (ABI 5) -------------------------------------------------------------
+ * zdwb_merge_codes takes n_parts parts, each a dictionary laid out as zdwb_columns_out's (dict, entry_off) plus codes
+ * into it, and returns one dictionary for all of them and the codes re-coded into it:
+ *   - The merged dictionary holds exactly the distinct strings that at least one code references, in strictly
+ *     increasing bytewise order (memcmp over the shorter string, then the length: strcmp's order for strings without
+ *     NUL).  Strings that are only in an input dictionary, with no code pointing at them, are left out.  So every code
+ *     0..entries-1 occurs, codes compare like their strings, and two output codes are equal iff their strings are equal.
+ *   - out->codes holds the sum of the parts' n codes, the parts in order; -1 stays -1.
+ *   - The parts may come from any blocks, any columns and any files: the parts of one column over all blocks give that
+ *     column a file-wide dictionary; the parts of two columns give them one shared dictionary (what a join needs).
+ *   - The referenced entries of every part must be strictly increasing bytewise (a block's dictionary is).
+ * Outputs are device memory owned by the context and stay valid until its next call.  With no referenced entry, dict
+ * is NULL, entries and dict_bytes are 0 and entry_off holds the one offset 0; codes is NULL when n is 0.
+ * Errors (each checked before any string byte is read through the offsets involved; the context works normally at its
+ * next call):
+ *   ZDWB_ERR_BAD_ARG: n_parts > 0 with NULL parts; a part with n > 0 and NULL codes, or with entries > 0 and a NULL dict
+ *     or entry_off; a code < -1 or >= its part's entries; a referenced entry e whose offsets are not
+ *     entry_off[e] < entry_off[e+1] <= dict_bytes; a part whose referenced entries are not strictly increasing bytewise.
+ *   ZDWB_ERR_UNSUPPORTED: more than 2^32 - 1 referenced entries in total (counted once per part that references them).
+ * The input memory must hold its final contents when the call is made: the context's stream does not wait for other
+ * streams.  Device scratch: 88 bytes per referenced entry plus 4 bytes per input entry (DESIGN 4.6). */
+typedef struct {
+  const uint8_t*  dict;       /* device: a dictionary laid out as zdwb_columns_out.dict (NULL iff entries == 0) */
+  const uint64_t* entry_off;  /* device: entries + 1 offsets; entry i = dict[entry_off[i] .. entry_off[i+1] - 1) */
+  uint64_t entries;
+  uint64_t dict_bytes;
+  const int64_t*  codes;      /* device: n codes into this dictionary, -1 = no value */
+  uint64_t n;
+} zdwb_code_part;
+
+typedef struct {
+  const int64_t*  codes;      /* device: sum(n) codes, parts in order, into the merged dictionary; -1 stays -1 */
+  const uint8_t*  dict;       /* device: origin NUL byte, then every entry NUL-terminated (NULL iff entries == 0) */
+  const uint64_t* entry_off;  /* device: entries + 1 offsets, entry_off[entries] = dict_bytes */
+  uint64_t entries;
+  uint64_t dict_bytes;
+  uint64_t n;
+} zdwb_merge_out;
+
+int zdwb_merge_codes(zdwb_ctx* ctx, const zdwb_code_part* parts, uint32_t n_parts, zdwb_merge_out* out);
 
 /* ---- pinned host staging (used by the host classes and the end-to-end bench) ------------------ */
 void* zdwb_host_alloc(size_t bytes);   /* cudaHostAlloc'd (pinned, usable from every device) memory, NULL on failure */

@@ -4,7 +4,8 @@ The product is native: `libzdw_b200.so` (hand-written CUDA kernels behind the C 
 include/zdw_b200.h) plus the C++ host classes/CLIs under zdw_b200/host.  This Python package holds
 the ctypes binding of that ABI (capi: Context, used by the test-suite and bench.py) and a reader
 that decodes ZDW files into typed CUDA tensors (reader: read_header, read_columns; one ColumnBlock
-per block, decoded on the GPU by zdwb_decode_columns).  It contains no compute of its own and no
+per block, decoded on the GPU by zdwb_decode_columns; read_table: one ColumnTable per file, its text
+columns merged into file-wide dictionaries by zdwb_merge_codes).  It contains no compute of its own and no
 CPU fallback; torch is only imported by the columnar calls.
 """
 from .capi import (  # noqa: F401
@@ -12,11 +13,12 @@ from .capi import (  # noqa: F401
     Context,
     EncodedBlock,
     DecodedBlock,
+    MergedCodes,
     ZdwError,
     lib_path,
     load_library,
 )
-from .reader import FileHeader, read_columns, read_header  # noqa: F401
+from .reader import ColumnTable, FileHeader, read_columns, read_header, read_table  # noqa: F401
 
-__all__ = ["Context", "EncodedBlock", "DecodedBlock", "ColumnBlock", "ZdwError", "FileHeader", "lib_path", "load_library",
-           "read_columns", "read_header"]
+__all__ = ["Context", "EncodedBlock", "DecodedBlock", "ColumnBlock", "MergedCodes", "ZdwError", "FileHeader", "ColumnTable",
+           "lib_path", "load_library", "read_columns", "read_header", "read_table"]

@@ -18,7 +18,7 @@ STATUS_NAMES = {0: "OK", 1: "ERR_CUDA", 2: "ERR_OOM", 3: "ERR_WRONG_COLUMNS", 4:
 EXPORTED_SYMBOLS = [
     "zdwb_abi_version", "zdwb_device_count", "zdwb_ctx_create", "zdwb_ctx_destroy", "zdwb_last_error", "zdwb_ctx_set_stream",
     "zdwb_ctx_set_tuning", "zdwb_ctx_kernel_launches", "zdwb_ctx_kernel_times", "zdwb_encode_block", "zdwb_decode_block", "zdwb_host_alloc",
-    "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns",
+    "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns", "zdwb_merge_codes",
 ]
 
 
@@ -82,6 +82,16 @@ class _ColsOut(C.Structure):
                 ("is_last", C.c_uint8), ("reserved", C.c_uint8 * 3), ("ncols_used", C.c_uint32)]
 
 
+class _CodePart(C.Structure):
+    _fields_ = [("dict", C.c_void_p), ("entry_off", C.c_void_p), ("entries", C.c_uint64), ("dict_bytes", C.c_uint64),
+                ("codes", C.c_void_p), ("n", C.c_uint64)]
+
+
+class _MergeOut(C.Structure):
+    _fields_ = [("codes", C.c_void_p), ("dict", C.c_void_p), ("entry_off", C.c_void_p), ("entries", C.c_uint64),
+                ("dict_bytes", C.c_uint64), ("n", C.c_uint64)]
+
+
 _lib = None
 
 
@@ -121,6 +131,7 @@ def load_library():
                                     C.POINTER(_RowsOut)]
     L.zdwb_decode_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.c_void_p, C.c_size_t, C.POINTER(_ColOpts),
                                       C.POINTER(_ColsOut)]
+    L.zdwb_merge_codes.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.c_uint32, C.POINTER(_MergeOut)]
     L.zdwb_host_alloc.argtypes = [C.c_size_t]
     L.zdwb_host_alloc.restype = C.c_void_p
     L.zdwb_host_free.argtypes = [C.c_void_p]
@@ -161,6 +172,11 @@ class DecodedBlock:
     flag_counts: list | None = None
 
 
+# column types whose cells zdwb_decode_columns gives as dictionary codes (include/zdw_b200.h): VARCHAR, TEXT, DATETIME,
+# CHAR_2, DECIMAL, TINYTEXT, MEDIUMTEXT, LONGTEXT (the library's is_text_like, csrc/common.cuh)
+TEXT_LIKE_TYPES = frozenset({0, 1, 2, 3, 11, 16, 17, 18})
+
+
 @dataclass
 class ColumnBlock:
     """One block decoded into typed device columns (zdwb_decode_columns): row k of `values` is the k-th requested column.
@@ -184,10 +200,37 @@ class ColumnBlock:
 
     def strings(self, k: int) -> list:
         """The texts of row k of `values` (a text-like column) on the host: bytes per row, None for code -1."""
-        codes = self.values[k].cpu().tolist()
-        d = bytes(self.dict.cpu().numpy().tobytes()) if self.dict.numel() else b""
-        eo = self.entry_off.cpu().tolist()
-        return [None if c < 0 else d[eo[c]:eo[c + 1] - 1] for c in codes]
+        return _strings(self.values[k], self.dict, self.entry_off)
+
+
+def _strings(codes, dct, entry_off) -> list:
+    """Host texts of a 1-D code tensor into (dict, entry_off): bytes per code, None for -1."""
+    d = bytes(dct.cpu().numpy().tobytes()) if dct.numel() else b""
+    eo = entry_off.cpu().tolist()
+    return [None if c < 0 else d[eo[c]:eo[c + 1] - 1] for c in codes.cpu().tolist()]
+
+
+@dataclass
+class MergedCodes:
+    """The result of Context.merge_codes (zdwb_merge_codes).
+
+    codes      int64 CUDA tensor: the parts' codes, concatenated in order, into `dict` (-1 stays -1).
+    dict       uint8 CUDA tensor: origin NUL byte, then every entry NUL-terminated (empty when no code references one).
+    entry_off  int64 CUDA tensor of entries + 1 offsets: entry i is dict[entry_off[i] : entry_off[i + 1] - 1].
+    The entries are distinct, sorted bytewise, and each is referenced by a code: codes 0 .. entries - 1 all occur, they
+    compare like their strings, and two codes are equal iff their strings are.
+    """
+    codes: object
+    dict: object
+    entry_off: object
+
+    @property
+    def entries(self) -> int:
+        return self.entry_off.numel() - 1
+
+    def strings(self) -> list:
+        """The texts of `codes` on the host: bytes per code, None for -1."""
+        return _strings(self.codes, self.dict, self.entry_off)
 
 
 class _DeviceArray:
@@ -395,3 +438,37 @@ class Context:
             (out.dict or 0, (out.dict_bytes if out.dict else 0,), "|u1", torch.uint8),
             (out.entry_off or 0, (out.dict_entries + 1 if out.entry_off else 0,), "<i8", torch.int64)])
         return ColumnBlock(values, dct, eo, cols, out.nrows, out.consumed, bool(out.is_last), out.line_length, out.ncols_used)
+
+    # ------------------------------------------------------------------ merged dictionaries
+    def merge_codes(self, parts) -> MergedCodes:
+        """One sorted dictionary for codes into many (zdwb_merge_codes; see MergedCodes).  parts: a sequence of
+        (dict, entry_off, codes) CUDA tensors on the context's device, e.g. (blk.dict, blk.entry_off, blk.values[k]) of
+        ColumnBlocks; codes 1-D contiguous int64, entry_off int64 (or uint64) with entries + 1 offsets.  The tensors
+        must hold their final contents when the call is made (those of decode_columns do): the context's stream does not
+        wait for torch's.  The results are copies, complete when this returns, as with decode_columns."""
+        import torch
+
+        dev = self.device
+        arr = (_CodePart * max(len(parts), 1))()
+        for i, (dct, eo, codes) in enumerate(parts):
+            for name, t in (("dict", dct), ("entry_off", eo), ("codes", codes)):
+                if not t.is_cuda or t.device.index != dev or not t.is_contiguous():
+                    raise ValueError(f"merge_codes: part {i}: {name} must be a contiguous tensor on cuda:{dev}")
+            if codes.dtype != torch.int64 or codes.dim() != 1:
+                raise ValueError(f"merge_codes: part {i}: codes must be a 1-D int64 tensor")
+            if eo.dtype not in (torch.int64, torch.uint64) or dct.dtype != torch.uint8:
+                raise ValueError(f"merge_codes: part {i}: dict must be uint8 and entry_off int64")
+            entries = max(eo.numel() - 1, 0)
+            arr[i] = _CodePart(dct.data_ptr() if dct.numel() else None, eo.data_ptr() if eo.numel() else None, entries,
+                               dct.numel(), codes.data_ptr() if codes.numel() else None, codes.numel())
+        out = _MergeOut()
+        rc = self._L.zdwb_merge_codes(self._h, arr, len(parts), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=dev)
+        codes, dct, eo = _device_tensors(torch, dev, self._copy_stream, [
+            (out.codes or 0, (out.n,), "<i8", torch.int64),
+            (out.dict or 0, (out.dict_bytes,), "|u1", torch.uint8),
+            (out.entry_off or 0, (out.entries + 1,), "<i8", torch.int64)])
+        return MergedCodes(codes, dct, eo)

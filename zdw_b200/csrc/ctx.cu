@@ -7,7 +7,9 @@
 
 #include "common.cuh"
 
-struct zdwb_ctx : zdwb::Ctx {};
+struct zdwb_ctx : zdwb::Ctx {
+  long long merge_max_refs = 0xffffffffll;  // zdwb_merge_codes: most referenced entries of a call (tests lower it)
+};
 
 namespace zdwb {
 int encode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* tsv, size_t n, const zdwb_encode_opts* opts,
@@ -16,6 +18,7 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
                       zdwb_rows_out* out);
 int decode_columns_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_columns_opts* opts,
                         zdwb_columns_out* out);
+int merge_codes_impl(Ctx* ctx, const zdwb_code_part* parts, uint32_t n_parts, unsigned long long max_refs, zdwb_merge_out* out);
 }  // namespace zdwb
 
 using zdwb::Ctx;
@@ -171,6 +174,7 @@ int zdwb_ctx_set_tuning(zdwb_ctx* c, const char* name, long long value) {
     c->delta_bailed = false;
   } else if (!strcmp(name, "enc_p2_rows")) c->enc_p2_rows = value;
   else if (!strcmp(name, "enc_dtile")) c->enc_dtile = value;
+  else if (!strcmp(name, "merge_max_refs")) c->merge_max_refs = value < 0 ? 0 : value > 0xffffffffll ? 0xffffffffll : value;
   else if (!strcmp(name, "kernel_timing")) c->timing = value != 0;
   else return ZDWB_ERR_BAD_ARG;
   return ZDWB_OK;
@@ -280,6 +284,28 @@ int zdwb_decode_columns(zdwb_ctx* c, const zdwb_schema* schema, const void* zdw,
     return ZDWB_ERR_OOM;
   } catch (...) {
     c->err = "zdwb_decode_columns: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_merge_codes(zdwb_ctx* c, const zdwb_code_part* parts, uint32_t n_parts, zdwb_merge_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!out) {
+    c->err = "zdwb_merge_codes: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::merge_codes_impl(c, parts, n_parts, (unsigned long long)c->merge_max_refs, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_merge_codes: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_merge_codes: unexpected C++ exception";
     return ZDWB_ERR_CUDA;
   }
 }
