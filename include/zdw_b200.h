@@ -21,6 +21,8 @@
  *        of text: one int64 per cell, text as codes into the block's sorted dictionary
  *   zdwb_merge_codes (no counterpart either) merges the dictionaries of many blocks into one sorted dictionary and
  *        re-codes their codes into it
+ *   zdwb_render_columns (no counterpart either) renders typed device columns back to TSV rows, the input of
+ *        zdwb_encode_block: the way from columns back to a ZDW file
  *
  * Plain C types only; int status codes; no exceptions and no C++ types cross the boundary.  Outputs
  * are owned by the context and stay valid until the next call on the same context.  One context per
@@ -305,6 +307,39 @@ typedef struct {
 } zdwb_merge_out;
 
 int zdwb_merge_codes(zdwb_ctx* ctx, const zdwb_code_part* parts, uint32_t n_parts, zdwb_merge_out* out);
+
+/* ---- columns back to rows (ABI 5) ---------------------------------------------------------------
+ * zdwb_render_columns writes schema->ncols columns of n rows each (cols[k] is column k, of type schema->types[k]) as TSV
+ * rows: fields separated by '\t', every row ended by '\n'.  The text of every cell is the one that zdwb_encode_block (and
+ * convertDWfile) reads back as the same cell, so encoding the output gives a block whose zdwb_decode_columns cells are
+ * the input's (text-like cells as codes into that block's own dictionary).  cols[k] is laid out as a zdwb_merge_codes
+ * part: for a text-like column codes into (dict, entry_off, entries, dict_bytes), as zdwb_columns_out / zdwb_merge_out
+ * give them, -1 = no value; for any other column the int64 cells as zdwb_decode_columns gives them, and the dictionary
+ * fields are ignored (NULL / 0).  Columns may share a dictionary.  The cell texts:
+ *   text-like    code -1: empty (DECIMAL too: "0.000000000000" would encode as a dictionary string); code c: entry c
+ *   unsigned     the decimal of the uint64 bits
+ *   signed       the decimal of the int64 (INT64_MIN as "-9223372036854775808", not the decoder's lltoa text)
+ *   CHAR         0: empty; sx(b) with b not NUL, '\t', '\n', '\\': the byte b; '\\' + sx(b) * 256 with b not NUL: '\\' then b
+ *                (sx = signed-char extension, as the encoder computes a CHAR value)
+ * out->tsv is device memory in a buffer of the context that no other entry point re-uses (as zdwb_fd_to_device's): it
+ * stays valid until the next zdwb_render_columns call on the context, so it can be handed to zdwb_encode_block with
+ * input_on_device = 1.  Zero rows: ZDWB_OK with len 0.
+ * ZDWB_ERR_BAD_ARG (zdwb_last_error names the lowest (column, row) at fault and the rule): NULL arguments, zero columns,
+ *   columns of different n, a type the encoder does not know (4, 5: the VISID types); a code < -1 or >= entries; a
+ *   referenced entry whose offsets are not entry_off[e] < entry_off[e+1] <= dict_bytes, that is empty, holds a NUL or does
+ *   not end in one, holds a '\t' or '\n' not preceded by an odd run of backslashes, or ends in an odd run of backslashes
+ *   (the row reader would not give it back as one field); a CHAR value of none of the forms above; an empty cell in a
+ *   table of one column (the row "\n" would be skipped).  Entries no code references are not checked for content, and
+ *   nothing is read through an entry's offsets before they are checked.  ZDWB_ERR_UNSUPPORTED: 2^36 rows or 2^24
+ *   columns and more.  The context works normally at its next call.
+ * The input memory must hold its final contents when the call is made: the context's stream does not wait for other
+ * streams.  Device scratch: 8 bytes per row and 1 byte per entry of every distinct dictionary (DESIGN 4.7). */
+typedef struct {
+  const uint8_t* tsv;   /* device: the rows; fields separated by '\t', every row ended by '\n' */
+  uint64_t len;
+} zdwb_render_out;
+
+int zdwb_render_columns(zdwb_ctx* ctx, const zdwb_schema* schema, const zdwb_code_part* cols, zdwb_render_out* out);
 
 /* ---- pinned host staging (used by the host classes and the end-to-end bench) ------------------ */
 void* zdwb_host_alloc(size_t bytes);   /* cudaHostAlloc'd (pinned, usable from every device) memory, NULL on failure */

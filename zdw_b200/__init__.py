@@ -5,7 +5,9 @@ include/zdw_b200.h) plus the C++ host classes/CLIs under zdw_b200/host.  This Py
 the ctypes binding of that ABI (capi: Context, used by the test-suite and bench.py) and a reader
 that decodes ZDW files into typed CUDA tensors (reader: read_header, read_columns; one ColumnBlock
 per block, decoded on the GPU by zdwb_decode_columns; read_table: one ColumnTable per file, its text
-columns merged into file-wide dictionaries by zdwb_merge_codes).  It contains no compute of its own and no
+columns merged into file-wide dictionaries by zdwb_merge_codes) and a writer that goes the other way (writer:
+write_table renders a ColumnTable's blocks to TSV on the GPU with zdwb_render_columns and encodes them with
+zdwb_encode_block).  It contains no compute of its own and no
 CPU fallback; torch is only imported by the columnar calls.
 """
 from .capi import (  # noqa: F401
@@ -19,6 +21,8 @@ from .capi import (  # noqa: F401
     load_library,
 )
 from .reader import ColumnTable, FileHeader, read_columns, read_header, read_table  # noqa: F401
+from .writer import write_table  # noqa: F401
 
 __all__ = ["Context", "EncodedBlock", "DecodedBlock", "ColumnBlock", "MergedCodes", "ZdwError", "FileHeader", "ColumnTable",
-           "lib_path", "load_library", "read_columns", "read_header", "read_table"]
+           "lib_path", "load_library", "read_columns", "read_header", "read_table",
+           "write_table"]

@@ -19,6 +19,7 @@ EXPORTED_SYMBOLS = [
     "zdwb_abi_version", "zdwb_device_count", "zdwb_ctx_create", "zdwb_ctx_destroy", "zdwb_last_error", "zdwb_ctx_set_stream",
     "zdwb_ctx_set_tuning", "zdwb_ctx_kernel_launches", "zdwb_ctx_kernel_times", "zdwb_encode_block", "zdwb_decode_block", "zdwb_host_alloc",
     "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns", "zdwb_merge_codes",
+    "zdwb_render_columns",
 ]
 
 
@@ -92,6 +93,10 @@ class _MergeOut(C.Structure):
                 ("dict_bytes", C.c_uint64), ("n", C.c_uint64)]
 
 
+class _RenderOut(C.Structure):
+    _fields_ = [("tsv", C.c_void_p), ("len", C.c_uint64)]
+
+
 _lib = None
 
 
@@ -132,6 +137,7 @@ def load_library():
     L.zdwb_decode_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.c_void_p, C.c_size_t, C.POINTER(_ColOpts),
                                       C.POINTER(_ColsOut)]
     L.zdwb_merge_codes.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.c_uint32, C.POINTER(_MergeOut)]
+    L.zdwb_render_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.POINTER(_CodePart), C.POINTER(_RenderOut)]
     L.zdwb_host_alloc.argtypes = [C.c_size_t]
     L.zdwb_host_alloc.restype = C.c_void_p
     L.zdwb_host_free.argtypes = [C.c_void_p]
@@ -472,3 +478,46 @@ class Context:
             (out.dict or 0, (out.dict_bytes,), "|u1", torch.uint8),
             (out.entry_off or 0, (out.entries + 1,), "<i8", torch.int64)])
         return MergedCodes(codes, dct, eo)
+
+    # ------------------------------------------------------------------ columns back to rows
+    def render_columns(self, types, cells, dicts) -> tuple[int, int]:
+        """TSV rows of typed device columns (zdwb_render_columns; include/zdw_b200.h gives the text of every cell), which
+        encode_block(types, ptr, length, input_on_device=True) encodes back into the same cells.  types: the column
+        types; cells: a sequence of 1-D int64 CUDA tensors, or a 2-D one (row k = column k), on the context's device;
+        dicts: per column (dict, entry_off) for a text-like column (as ColumnTable.dicts holds them), None for the
+        others.  The tensors must hold their final contents when the call is made, as with merge_codes.  Returns
+        (device pointer, length) of the rows: a buffer of the context, valid until its next render_columns call."""
+        import torch
+
+        dev = self.device
+        if isinstance(cells, torch.Tensor) and cells.dim() == 2:
+            cells = list(cells)
+        if len(cells) != len(types) or len(dicts) != len(types):
+            raise ValueError(f"render_columns: {len(types)} types, {len(cells)} columns of cells and {len(dicts)} dicts")
+        arr = (_CodePart * max(len(types), 1))()
+        for k, (codes, dd) in enumerate(zip(cells, dicts)):
+            if not isinstance(codes, torch.Tensor) or not codes.is_cuda or codes.device.index != dev:
+                raise ValueError(f"render_columns: column {k}: cells must be a tensor on cuda:{dev}")
+            if codes.dtype != torch.int64 or codes.dim() != 1 or not codes.is_contiguous():
+                raise ValueError(f"render_columns: column {k}: cells must be a contiguous 1-D int64 tensor")
+            dptr = eptr = None
+            entries = nbytes = 0
+            if dd is not None:
+                dct, eo = dd
+                for name, t in (("dict", dct), ("entry_off", eo)):
+                    if not t.is_cuda or t.device.index != dev or not t.is_contiguous():
+                        raise ValueError(f"render_columns: column {k}: {name} must be a contiguous tensor on cuda:{dev}")
+                if eo.dtype not in (torch.int64, torch.uint64) or dct.dtype != torch.uint8:
+                    raise ValueError(f"render_columns: column {k}: dict must be uint8 and entry_off int64")
+                entries = max(eo.numel() - 1, 0)
+                nbytes = dct.numel()
+                dptr = dct.data_ptr() if nbytes else None
+                eptr = eo.data_ptr() if eo.numel() else None
+            arr[k] = _CodePart(dptr, eptr, entries, nbytes, codes.data_ptr() if codes.numel() else None, codes.numel())
+        tarr = (C.c_uint8 * max(len(types), 1))(*types)
+        sch = _Schema(len(types), C.cast(tarr, C.POINTER(C.c_uint8)))
+        out = _RenderOut()
+        rc = self._L.zdwb_render_columns(self._h, C.byref(sch), arr, C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        return int(out.tsv or 0), int(out.len)

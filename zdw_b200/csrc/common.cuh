@@ -689,6 +689,20 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 // orders the generic-proxy accesses of this thread before later async-proxy (bulk copy) accesses to shared memory
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
+// decimal digits of x (llutoa's text length)
+__device__ __forceinline__ uint32_t digits_u32(uint32_t x) {
+  return x < 10u ? 1u : x < 100u ? 2u : x < 1000u ? 3u : x < 10000u ? 4u : x < 100000u ? 5u : x < 1000000u ? 6u
+         : x < 10000000u ? 7u : x < 100000000u ? 8u : x < 1000000000u ? 9u : 10u;
+}
+__device__ __forceinline__ uint32_t digits_u64(unsigned long long v) {
+  if (v <= 0xffffffffull) return digits_u32((uint32_t)v);
+  if (v < 100000000000000ull) {  // < 10^14
+    return v < 10000000000ull ? 10u : v < 100000000000ull ? 11u : v < 1000000000000ull ? 12u : v < 10000000000000ull ? 13u : 14u;
+  }
+  return v < 1000000000000000ull ? 15u : v < 10000000000000000ull ? 16u : v < 100000000000000000ull ? 17u
+         : v < 1000000000000000000ull ? 18u : v < 10000000000000000000ull ? 19u : 20u;
+}
+
 // per-byte equality mask of a 32-bit word against a replicated byte: bit 7 of each byte lane set
 __device__ __forceinline__ uint32_t bytes_eq(uint32_t w, uint32_t rep) {
   uint32_t x = w ^ rep;

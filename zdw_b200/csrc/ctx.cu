@@ -9,6 +9,8 @@
 
 struct zdwb_ctx : zdwb::Ctx {
   long long merge_max_refs = 0xffffffffll;  // zdwb_merge_codes: most referenced entries of a call (tests lower it)
+  void* render_dev = nullptr;  // zdwb_render_columns' output (own allocation: it outlives the arena resets of later calls)
+  size_t render_dev_cap = 0;
 };
 
 namespace zdwb {
@@ -19,6 +21,8 @@ int decode_block_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size
 int decode_columns_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, size_t avail, const zdwb_columns_opts* opts,
                         zdwb_columns_out* out);
 int merge_codes_impl(Ctx* ctx, const zdwb_code_part* parts, uint32_t n_parts, unsigned long long max_refs, zdwb_merge_out* out);
+int render_columns_impl(Ctx* ctx, const zdwb_schema* schema, const zdwb_code_part* cols, void** buf, size_t* cap,
+                        zdwb_render_out* out);
 }  // namespace zdwb
 
 using zdwb::Ctx;
@@ -81,6 +85,7 @@ void zdwb_ctx_destroy(zdwb_ctx* c) {
   if (c->stage_host) cudaFreeHost(c->stage_host);
   zdwb::ring_destroy(c);
   if (c->fd_dev) cudaFree(c->fd_dev);
+  if (c->render_dev) cudaFree(c->render_dev);
   if (c->own_stream) cudaStreamDestroy(c->own_stream);
   delete c;
 }
@@ -306,6 +311,28 @@ int zdwb_merge_codes(zdwb_ctx* c, const zdwb_code_part* parts, uint32_t n_parts,
     return ZDWB_ERR_OOM;
   } catch (...) {
     c->err = "zdwb_merge_codes: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_render_columns(zdwb_ctx* c, const zdwb_schema* schema, const zdwb_code_part* cols, zdwb_render_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!schema || !cols || !out) {
+    c->err = "zdwb_render_columns: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::render_columns_impl(c, schema, cols, &c->render_dev, &c->render_dev_cap, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_render_columns: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_render_columns: unexpected C++ exception";
     return ZDWB_ERR_CUDA;
   }
 }
