@@ -23,6 +23,8 @@
  *        re-codes their codes into it
  *   zdwb_render_columns (no counterpart either) renders typed device columns back to TSV rows, the input of
  *        zdwb_encode_block: the way from columns back to a ZDW file
+ *   zdwb_match_like, zdwb_find_strings (no counterpart either) answer LIKE and string lookups over a sorted dictionary,
+ *        once per distinct string: the filters on text columns
  *
  * Plain C types only; int status codes; no exceptions and no C++ types cross the boundary.  Outputs
  * are owned by the context and stay valid until the next call on the same context.  One context per
@@ -340,6 +342,62 @@ typedef struct {
 } zdwb_render_out;
 
 int zdwb_render_columns(zdwb_ctx* ctx, const zdwb_schema* schema, const zdwb_code_part* cols, zdwb_render_out* out);
+
+/* ---- predicates over a dictionary (ABI 5) -------------------------------------------------------
+ * Both calls take a dictionary as a zdwb_code_part whose codes and n are ignored: a merged one (zdwb_merge_out) or a
+ * block's (zdwb_columns_out).  Entry i is dict[entry_off[i] .. entry_off[i+1] - 1).  A filter on a text column is then
+ * one pass over its distinct strings plus one gather of the per-entry answer by the codes.
+ *
+ * zdwb_match_like: SQL LIKE of every entry against opts->pattern, and of opts->null_text, the text that code -1 stands
+ *   for ("" for text columns, "0.000000000000" for DECIMAL).  out->flags holds entries + 1 bytes, 1 = match: one per
+ *   entry, the last one for null_text.  The whole entry is matched, bytewise, as it is stored (what unconvertDWfile prints
+ *   for the cell, TSV escapes included): '%' matches any run of bytes, the empty one too; '_' matches exactly one BYTE
+ *   (not one UTF-8 character); the escape byte followed by any byte matches that byte; every other byte matches itself.
+ *   With ignore_case the ASCII letters A-Z / a-z match either case (escaped ones too); no other byte is folded.
+ * zdwb_find_strings: for the n query strings in queries (query i = bytes[off[i] .. off[i+1]), device memory),
+ *   out->rank[i] is the number of entries bytewise less than query i (lower_bound, in [0, entries]) and out->found[i] is
+ *   1 iff entry rank[i] equals it.  The entries must be strictly increasing bytewise (memcmp over the shorter string, then
+ *   the length: the order of zdwb_merge_codes and of a block's dictionary); every entry is checked against the one
+ *   before it.  Queries may be unsorted, repeated, empty, and hold any byte.  rank and found are NULL when n is 0.
+ * Outputs are device memory owned by the context and stay valid until its next call.  The input memory must hold its
+ * final contents when the call is made: the context's stream does not wait for other streams.
+ * Errors (checked before anything is read through the offsets involved; zdwb_last_error names the lowest entry or query
+ * at fault; the context works normally at its next call):
+ *   ZDWB_ERR_BAD_ARG: a NULL dict, opts, queries or out; entries > 0 with a NULL dict or entry_off; a pattern or null_text
+ *     with a length and a NULL pointer; escape not in -1 .. 255; a pattern that ends in a lone escape byte; an entry whose
+ *     offsets are not entry_off[e] < entry_off[e+1] <= dict_bytes; (find) n > 0 with NULL off, bytes_len > 0 with NULL
+ *     bytes, an entry not greater than the one before it, a query whose offsets are not off[i] <= off[i+1] <= bytes_len.
+ *   ZDWB_ERR_UNSUPPORTED: a pattern of 2^32 - 1 bytes or more.
+ * Device scratch: match 2 bytes per pattern byte; find 16 bytes per entry (DESIGN 4.8). */
+typedef struct {
+  const uint8_t* pattern;    /* host memory */
+  uint64_t pattern_len;
+  const uint8_t* null_text;  /* host memory: the text of code -1 */
+  uint64_t null_text_len;
+  int32_t escape;            /* -1 = no escape byte, else 0 .. 255 */
+  int32_t ignore_case;       /* fold ASCII A-Z / a-z */
+} zdwb_like_opts;
+
+typedef struct {
+  const uint8_t* flags;      /* device: n bytes, 0 / 1; flags[entries] is null_text's */
+  uint64_t n;                /* entries + 1 */
+} zdwb_match_out;
+
+typedef struct {
+  const uint8_t* bytes;      /* device: the query strings back to back */
+  uint64_t bytes_len;
+  const uint64_t* off;       /* device: n + 1 offsets into bytes */
+  uint64_t n;
+} zdwb_strings;
+
+typedef struct {
+  const int64_t* rank;       /* device: n lower bounds */
+  const uint8_t* found;      /* device: n bytes, 1 iff entry rank[i] equals query i */
+  uint64_t n;
+} zdwb_find_out;
+
+int zdwb_match_like(zdwb_ctx* ctx, const zdwb_code_part* dict, const zdwb_like_opts* opts, zdwb_match_out* out);
+int zdwb_find_strings(zdwb_ctx* ctx, const zdwb_code_part* dict, const zdwb_strings* queries, zdwb_find_out* out);
 
 /* ---- pinned host staging (used by the host classes and the end-to-end bench) ------------------ */
 void* zdwb_host_alloc(size_t bytes);   /* cudaHostAlloc'd (pinned, usable from every device) memory, NULL on failure */

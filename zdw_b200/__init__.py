@@ -7,7 +7,8 @@ that decodes ZDW files into typed CUDA tensors (reader: read_header, read_column
 per block, decoded on the GPU by zdwb_decode_columns; read_table: one ColumnTable per file, its text
 columns merged into file-wide dictionaries by zdwb_merge_codes) and a writer that goes the other way (writer:
 write_table renders a ColumnTable's blocks to TSV on the GPU with zdwb_render_columns and encodes them with
-zdwb_encode_block).  It contains no compute of its own and no
+zdwb_encode_block) and filters on text columns (predicates: like, isin, between, answered once per dictionary entry by
+zdwb_match_like and zdwb_find_strings).  It contains no compute of its own and no
 CPU fallback; torch is only imported by the columnar calls.
 """
 from .capi import (  # noqa: F401
@@ -22,7 +23,8 @@ from .capi import (  # noqa: F401
 )
 from .reader import ColumnTable, FileHeader, read_columns, read_header, read_table  # noqa: F401
 from .writer import write_table  # noqa: F401
+from .predicates import between, isin, like  # noqa: F401
 
 __all__ = ["Context", "EncodedBlock", "DecodedBlock", "ColumnBlock", "MergedCodes", "ZdwError", "FileHeader", "ColumnTable",
            "lib_path", "load_library", "read_columns", "read_header", "read_table",
-           "write_table"]
+           "write_table", "like", "isin", "between"]

@@ -19,7 +19,7 @@ EXPORTED_SYMBOLS = [
     "zdwb_abi_version", "zdwb_device_count", "zdwb_ctx_create", "zdwb_ctx_destroy", "zdwb_last_error", "zdwb_ctx_set_stream",
     "zdwb_ctx_set_tuning", "zdwb_ctx_kernel_launches", "zdwb_ctx_kernel_times", "zdwb_encode_block", "zdwb_decode_block", "zdwb_host_alloc",
     "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns", "zdwb_merge_codes",
-    "zdwb_render_columns",
+    "zdwb_render_columns", "zdwb_match_like", "zdwb_find_strings",
 ]
 
 
@@ -97,6 +97,23 @@ class _RenderOut(C.Structure):
     _fields_ = [("tsv", C.c_void_p), ("len", C.c_uint64)]
 
 
+class _LikeOpts(C.Structure):
+    _fields_ = [("pattern", C.c_char_p), ("pattern_len", C.c_uint64), ("null_text", C.c_char_p), ("null_text_len", C.c_uint64),
+                ("escape", C.c_int32), ("ignore_case", C.c_int32)]
+
+
+class _MatchOut(C.Structure):
+    _fields_ = [("flags", C.c_void_p), ("n", C.c_uint64)]
+
+
+class _Strings(C.Structure):
+    _fields_ = [("bytes", C.c_void_p), ("bytes_len", C.c_uint64), ("off", C.c_void_p), ("n", C.c_uint64)]
+
+
+class _FindOut(C.Structure):
+    _fields_ = [("rank", C.c_void_p), ("found", C.c_void_p), ("n", C.c_uint64)]
+
+
 _lib = None
 
 
@@ -138,6 +155,8 @@ def load_library():
                                       C.POINTER(_ColsOut)]
     L.zdwb_merge_codes.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.c_uint32, C.POINTER(_MergeOut)]
     L.zdwb_render_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.POINTER(_CodePart), C.POINTER(_RenderOut)]
+    L.zdwb_match_like.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.POINTER(_LikeOpts), C.POINTER(_MatchOut)]
+    L.zdwb_find_strings.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.POINTER(_Strings), C.POINTER(_FindOut)]
     L.zdwb_host_alloc.argtypes = [C.c_size_t]
     L.zdwb_host_alloc.restype = C.c_void_p
     L.zdwb_host_free.argtypes = [C.c_void_p]
@@ -521,3 +540,66 @@ class Context:
         if rc:
             raise ZdwError(rc, self.last_error())
         return int(out.tsv or 0), int(out.len)
+
+    # ------------------------------------------------------------------ predicates over a dictionary
+    def _dict_part(self, who: str, dct, eo) -> _CodePart:
+        import torch
+        for name, t in (("dict", dct), ("entry_off", eo)):
+            if not isinstance(t, torch.Tensor) or not t.is_cuda or t.device.index != self.device or not t.is_contiguous():
+                raise ValueError(f"{who}: {name} must be a contiguous tensor on cuda:{self.device}")
+        if eo.dtype not in (torch.int64, torch.uint64) or dct.dtype != torch.uint8:
+            raise ValueError(f"{who}: dict must be uint8 and entry_off int64")
+        return _CodePart(dct.data_ptr() if dct.numel() else None, eo.data_ptr() if eo.numel() else None,
+                         max(eo.numel() - 1, 0), dct.numel(), None, 0)
+
+    def match_like(self, dct, entry_off, pattern: bytes, *, escape: bytes | None = b"\\", ignore_case=False,
+                   null_text: bytes = b""):
+        """SQL LIKE of every entry of a dictionary (zdwb_match_like; include/zdw_b200.h gives the rules): a bool CUDA
+        tensor of entries + 1 flags, the last one for `null_text`, the text of code -1.  So `flags[codes]` is the answer
+        per cell, code -1 included.  dct, entry_off: a dictionary as ColumnTable.dicts[k] or ColumnBlock.dict /
+        entry_off hold it, on the context's device, with their final contents (as with merge_codes).  escape: one byte,
+        or None for none.  The result is a copy, complete when this returns."""
+        import torch
+        part = self._dict_part("match_like", dct, entry_off)
+        if escape is not None and len(escape) != 1:
+            raise ValueError("match_like: escape must be one byte or None")
+        pattern, null_text = bytes(pattern), bytes(null_text)
+        o = _LikeOpts(pattern, len(pattern), null_text, len(null_text), -1 if escape is None else escape[0], int(bool(ignore_case)))
+        out = _MatchOut()
+        rc = self._L.zdwb_match_like(self._h, C.byref(part), C.byref(o), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=self.device)
+        (flags,) = _device_tensors(torch, self.device, self._copy_stream, [(out.flags or 0, (out.n,), "|u1", torch.uint8)])
+        return flags.view(torch.bool)
+
+    def find_strings(self, dct, entry_off, strings):
+        """lower_bound of every string of `strings` (a sequence of bytes) among the entries of a sorted dictionary
+        (zdwb_find_strings): (rank, found) CUDA tensors, rank int64 = the number of entries bytewise less than the string,
+        found bool = entry rank equals it.  The dictionary is taken as by match_like; the strings go to the device in one
+        buffer.  The results are copies, complete when this returns."""
+        import torch
+        dev = self.device
+        part = self._dict_part("find_strings", dct, entry_off)
+        import numpy as np
+        strings = [s if isinstance(s, bytes) else bytes(s) for s in strings]
+        offs = np.zeros(len(strings) + 1, dtype=np.int64)
+        np.cumsum(np.fromiter(map(len, strings), dtype=np.int64, count=len(strings)), out=offs[1:])
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=dev)
+        # the queries are uploaded on the copy stream and complete before the call: torch's current stream may be busy
+        with torch.cuda.stream(self._copy_stream):
+            blob = b"".join(strings)
+            qb = torch.frombuffer(bytearray(blob), dtype=torch.uint8).to(f"cuda:{dev}") if blob else \
+                torch.empty(0, dtype=torch.uint8, device=f"cuda:{dev}")
+            qo = torch.from_numpy(offs).to(f"cuda:{dev}")
+        self._copy_stream.synchronize()
+        q = _Strings(qb.data_ptr() if qb.numel() else None, qb.numel(), qo.data_ptr(), len(strings))
+        out = _FindOut()
+        rc = self._L.zdwb_find_strings(self._h, C.byref(part), C.byref(q), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        rank, found = _device_tensors(torch, dev, self._copy_stream, [
+            (out.rank or 0, (out.n,), "<i8", torch.int64), (out.found or 0, (out.n,), "|u1", torch.uint8)])
+        return rank, found.view(torch.bool)

@@ -703,6 +703,34 @@ __device__ __forceinline__ uint32_t digits_u64(unsigned long long v) {
          : v < 1000000000000000000ull ? 18u : v < 10000000000000000000ull ? 19u : 20u;
 }
 
+// a string in device memory (merge.cu, match.cu)
+struct Str {
+  const uint8_t* p;
+  unsigned long long len;
+};
+
+// bytes [off, off + 8) of s as a big-endian number, zero past len (the idea of sort.cu's prefix_key)
+__device__ __forceinline__ unsigned long long key8(const uint8_t* s, unsigned long long len, unsigned long long off) {
+  unsigned long long k = 0;
+#pragma unroll
+  for (uint32_t i = 0; i < 8; ++i) k = (k << 8) | (off + i < len ? (unsigned long long)__ldg(s + off + i) : 0ull);
+  return k;
+}
+
+// bytewise order (memcmp over the shorter, then the length); the keys hold bytes 0..15
+__device__ __forceinline__ int str_cmp(const ulonglong2& ka, const Str& a, const ulonglong2& kb, const Str& b) {
+  if (ka.x != kb.x) return ka.x < kb.x ? -1 : 1;
+  if (ka.y != kb.y) return ka.y < kb.y ? -1 : 1;
+  // 8 bytes at a time past the keys: a word that straddles the shorter length compares its zero padding with the
+  // longer string's bytes, which orders the pair as the length compare below would, or finds them equal
+  const unsigned long long m = a.len < b.len ? a.len : b.len;
+  for (unsigned long long i = 16; i < m; i += 8) {
+    const unsigned long long x = key8(a.p, a.len, i), y = key8(b.p, b.len, i);
+    if (x != y) return x < y ? -1 : 1;
+  }
+  return a.len < b.len ? -1 : a.len > b.len ? 1 : 0;
+}
+
 // per-byte equality mask of a 32-bit word against a replicated byte: bit 7 of each byte lane set
 __device__ __forceinline__ uint32_t bytes_eq(uint32_t w, uint32_t rep) {
   uint32_t x = w ^ rep;

@@ -23,6 +23,8 @@ int decode_columns_impl(Ctx* ctx, const zdwb_schema* schema, const void* zdw, si
 int merge_codes_impl(Ctx* ctx, const zdwb_code_part* parts, uint32_t n_parts, unsigned long long max_refs, zdwb_merge_out* out);
 int render_columns_impl(Ctx* ctx, const zdwb_schema* schema, const zdwb_code_part* cols, void** buf, size_t* cap,
                         zdwb_render_out* out);
+int match_like_impl(Ctx* ctx, const zdwb_code_part* dict, const zdwb_like_opts* opts, zdwb_match_out* out);
+int find_strings_impl(Ctx* ctx, const zdwb_code_part* dict, const zdwb_strings* queries, zdwb_find_out* out);
 }  // namespace zdwb
 
 using zdwb::Ctx;
@@ -333,6 +335,50 @@ int zdwb_render_columns(zdwb_ctx* c, const zdwb_schema* schema, const zdwb_code_
     return ZDWB_ERR_OOM;
   } catch (...) {
     c->err = "zdwb_render_columns: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_match_like(zdwb_ctx* c, const zdwb_code_part* dict, const zdwb_like_opts* opts, zdwb_match_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!opts || !out) {
+    c->err = "zdwb_match_like: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::match_like_impl(c, dict, opts, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_match_like: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_match_like: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_find_strings(zdwb_ctx* c, const zdwb_code_part* dict, const zdwb_strings* queries, zdwb_find_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!queries || !out) {
+    c->err = "zdwb_find_strings: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::find_strings_impl(c, dict, queries, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_find_strings: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_find_strings: unexpected C++ exception";
     return ZDWB_ERR_CUDA;
   }
 }

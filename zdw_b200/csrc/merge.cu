@@ -39,11 +39,6 @@ struct MergeMeta {
 };
 constexpr uint32_t MG_ERR_CODE = 1, MG_ERR_OFFSETS = 2, MG_ERR_ORDER = 4;
 
-struct Str {
-  const uint8_t* p;
-  unsigned long long len;
-};
-
 __device__ __forceinline__ void merge_fail(MergeMeta* meta, uint32_t bit, uint32_t part) {
   atomicOr(&meta->err, bit);
   atomicMin(&meta->bad_part, part);
@@ -59,28 +54,6 @@ __device__ __forceinline__ uint32_t last_le(const T* __restrict__ a, uint32_t n,
     else hi = mid;
   }
   return lo;
-}
-
-// bytes [off, off + 8) of s as a big-endian number, zero past len (the idea of sort.cu's prefix_key)
-__device__ __forceinline__ unsigned long long key8(const uint8_t* s, unsigned long long len, unsigned long long off) {
-  unsigned long long k = 0;
-#pragma unroll
-  for (uint32_t i = 0; i < 8; ++i) k = (k << 8) | (off + i < len ? (unsigned long long)__ldg(s + off + i) : 0ull);
-  return k;
-}
-
-// bytewise order (memcmp over the shorter, then the length); the keys hold bytes 0..15
-__device__ __forceinline__ int str_cmp(const ulonglong2& ka, const Str& a, const ulonglong2& kb, const Str& b) {
-  if (ka.x != kb.x) return ka.x < kb.x ? -1 : 1;
-  if (ka.y != kb.y) return ka.y < kb.y ? -1 : 1;
-  // 8 bytes at a time past the keys: a word that straddles the shorter length compares its zero padding with the
-  // longer string's bytes, which orders the pair as the length compare below would, or finds them equal
-  const unsigned long long m = a.len < b.len ? a.len : b.len;
-  for (unsigned long long i = 16; i < m; i += 8) {
-    const unsigned long long x = key8(a.p, a.len, i), y = key8(b.p, b.len, i);
-    if (x != y) return x < y ? -1 : 1;
-  }
-  return a.len < b.len ? -1 : a.len > b.len ? 1 : 0;
 }
 
 __device__ __forceinline__ unsigned long long grid_threads() { return (unsigned long long)gridDim.x * blockDim.x; }
