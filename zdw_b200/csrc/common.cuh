@@ -46,7 +46,9 @@ struct Ctx {
   long long enc_delta = -1;            // pass 1 variant: 1 = row-delta, 0 = general, -1 = by row width (encode.cu)
   long long enc_p2_rows = 0;           // rows per pass-2 tile (0 = automatic)
   long long enc_dtile = 0;             // bytes per row-delta tile (0 = automatic; a power of two >= 2048)
+  long long enc_census = -1;           // row-delta row census: 1 = always, 0 = skipped for every uncut block, -1 = automatic
   bool delta_bailed = false;           // a block of this context did not fit the row-delta pass: stop trying
+  bool census_fell_back = false;       // a census-free pass 1 of this context handed its block to the census
   unsigned long long last_row_bytes = 0;  // mean row length of the previous block
   unsigned long long last_records = 0;    // records the previous block's row-delta pass 1 produced (sizes the next arrays)
   // outputs owned by the context (valid until the next call)

@@ -181,6 +181,10 @@ int zdwb_ctx_set_tuning(zdwb_ctx* c, const char* name, long long value) {
     c->delta_bailed = false;
   } else if (!strcmp(name, "enc_p2_rows")) c->enc_p2_rows = value;
   else if (!strcmp(name, "enc_dtile")) c->enc_dtile = value;
+  else if (!strcmp(name, "enc_census")) {
+    c->enc_census = value;
+    c->census_fell_back = false;
+  }
   else if (!strcmp(name, "merge_max_refs")) c->merge_max_refs = value < 0 ? 0 : value > 0xffffffffll ? 0xffffffffll : value;
   else if (!strcmp(name, "kernel_timing")) c->timing = value != 0;
   else return ZDWB_ERR_BAD_ARG;

@@ -17,9 +17,10 @@
 //   k_col_stats, k_col_info, k_block_header   writeLookupColumnStats         ConvertToZDW.cpp:417-483, :839-842
 //   k_pass2, k_gather_tiles       writeBlockRows                 ConvertToZDW.cpp:486-606 + Dictionary::getOffset :53-59
 //
-// Data layout in HBM: the TSV block is read twice (census, pass 1); records are 12 B per NON-EMPTY field (most
-// fields of analytics-shaped data are empty and cost nothing beyond their delimiter byte); the string hash set keeps
-// (start, len) of the first occurrence inside the TSV - strings are never copied until the dictionary is emitted.
+// Data layout in HBM: the TSV block is read twice (census, pass 1; the census-free row-delta pass 1 reads it once);
+// records are 12 B per NON-EMPTY field (most fields of analytics-shaped data are empty and cost nothing beyond their
+// delimiter byte); the string hash set keeps (start, len) of the first occurrence inside the TSV - strings are never
+// copied until the dictionary is emitted.
 #include <algorithm>
 #include <vector>
 
@@ -67,6 +68,10 @@ struct EncMeta {
   uint32_t next_start;     // first byte of the row after it
   uint32_t spill_end;      // position + 1 of the delimiter that closes the last spilled column of that row
   uint32_t spill_row_len;  // length of that row incl. its terminator (0 = there is no complete row)
+  // census-free row-delta pass 1 (k_pass1d<true>): rows are numbered per tile, k_row_fixup makes the numbers global
+  uint32_t slot_overflow;  // a tile owns more rows than it has slots: the block is run again with the census
+  uint32_t pad2;
+  unsigned long long bad_slot;  // (tile << 32) | row of the tile, of the first malformed row (~0 = none)
 };
 
 // per tile: counts, then (after k_tile_scan) exclusive prefixes
@@ -1034,6 +1039,9 @@ struct D1Args {
   uint32_t* row_cnt;     // [nrows] records of row r; they start at P.row_rec[r]
   uint32_t* chg_start;   // [rec_cap] where the changed field of record k starts in the TSV ...
   uint32_t* chg_len;     // ... and its length; 0 = the record of a column that became empty (value 0)
+  // census-free mode only: row j of tile t goes to slot t * slot_cap + j of P.row_rec / row_cnt
+  uint32_t slot_cap;     // row slots per tile
+  uint32_t* tile_rows;   // [ntiles] complete rows that start in the tile
 };
 
 // Row census of the delta path: per tile the number of row terminators, the last row break and the last row start.
@@ -1431,6 +1439,41 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
   }
 }
 
+// Census-free mode: position + 1 of the last row start in front of t0 (a byte other than '\n' behind an unescaped
+// newline, or the buffer's first byte), which is what the census's prefix of rs_p1 holds for the tile; 0 = only blank
+// lines in front of t0.  The warp walks back from t0 a step at a time and looks at newlines only.  -1: no row starts
+// within 64 KiB plus a step, the delta path's row limit (the warp bails; the host runs the block with the census).
+__device__ __forceinline__ int64_t d1_ref_start_p1(const uint8_t* __restrict__ buf, int64_t t0, unsigned lane) {
+  uint32_t nl_behind = 1u;  // the byte behind the step is '\n' - or is t0, where a row start does not count
+  for (int64_t hi = t0; hi > 0; hi -= DSTEP) {
+    if (t0 - hi > 65536) return -1;
+    const int64_t p0 = hi - (int64_t)DSTEP + 32 * (int64_t)lane;  // (16-byte aligned in memory, as the tiles are)
+    uint32_t nl = 0;
+    if (p0 + 32 > 0) {
+      const uint4 v0 = p0 + 16 > 0 ? ldg_keep_u4(buf + p0) : make_uint4(0u, 0u, 0u, 0u);
+      const uint4 v1 = ldg_keep_u4(buf + p0 + 16);
+      if (chunk_has(v0, '\n') || chunk_has(v1, '\n'))
+        nl = mask32(v0, v1, '\n') & (p0 >= 0 ? 0xffffffffu : ~bits_below((uint32_t)-p0));
+    }
+    uint32_t behind = __shfl_down_sync(0xffffffffu, nl & 1u, 1);
+    if (lane == 31) behind = nl_behind;
+    nl_behind = __shfl_sync(0xffffffffu, nl & 1u, 0);
+    uint32_t brk = nl & ~((nl >> 1) | (behind << 31));  // newlines followed by a byte other than '\n'
+    for (uint32_t m = brk; m; m &= m - 1u) {  // escape parity: rare, walked byte by byte
+      const int i = __ffs(m) - 1;
+      if (odd_backslashes_before(buf, p0 + i)) brk &= ~(1u << i);
+    }
+    const int32_t best = __reduce_max_sync(0xffffffffu, brk ? (int32_t)(lane * 32u) + (31 - __clz(brk)) : -1);
+    if (best >= 0) return hi - (int64_t)DSTEP + best + 2;
+    if (hi <= (int64_t)DSTEP) return __ldg(buf) != (uint8_t)'\n' ? 1 : 0;  // the step holds the buffer's first byte
+  }
+  return 0;
+}
+
+// CF = census-free: no TileAgg prefix.  The warp finds its reference row itself (d1_ref_start_p1), numbers the rows it
+// owns from 0 into its tile's slots, and reports the last row break it saw; k_row_fixup makes the numbers global.  The
+// limit is the end of the buffer, and a row it cuts short is dropped (it is the unterminated tail).
+template <bool CF>
 __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
   __shared__ D1Warp sw[D1_WARPS];
   const P1Args& P = A.P;
@@ -1438,15 +1481,30 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
   const uint32_t tile = blockIdx.x * D1_WARPS + warp;
   if (tile >= A.ntiles) return;
   const int64_t t0 = P.lo + (int64_t)tile * A.tile_bytes;
-  if (t0 >= P.limit) return;
+  if (t0 >= P.limit) {
+    if (CF && lane == 0) A.tile_rows[tile] = 0u;
+    return;
+  }
   const int64_t tile_end = t0 + A.tile_bytes;
   D1Warp& W = sw[warp];
   const uint32_t* wlast = reinterpret_cast<const uint32_t*>(reinterpret_cast<uintptr_t>(P.buf + P.n - 1) & ~(uintptr_t)3);
-  const TileAgg pre = P.pre[tile];
+  TileAgg pre;
+  if (CF) {
+    const int64_t rs_p1 = d1_ref_start_p1(P.buf, t0, lane);
+    if (rs_p1 < 0) {
+      if (lane == 0) *reinterpret_cast<volatile uint32_t*>(&P.meta->delta_bail) = 1u;
+      return;
+    }
+    pre.rs_p1 = (uint32_t)rs_p1;
+    pre.rows = 0u;
+  } else {
+    pre = P.pre[tile];
+  }
   const uint32_t BW = (P.ncols + 31u) >> 5;
   // the row in front of the tile's first row (if there is one) is read as the reference the first row is compared with
   const bool have_prev = pre.rs_p1 != 0u;
   const int64_t scan_from = have_prev ? (int64_t)pre.rs_p1 - 1 : (t0 > 0 ? t0 : 0);
+  uint32_t last_nl_p1 = 0;  // CF: position + 1 of the last row break the lane saw
   for (uint32_t w = lane; w < BW; w += 32u) W.BM[0][w] = W.BM[1][w] = 0u;  // "the row before" of a block's first row is empty
   __syncwarp();
   const uint32_t tabs_per_row = P.ncols - 1u;
@@ -1481,7 +1539,7 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
       if (stop || sb >= P.limit || (!row_open && sb >= tile_end)) {
         // a row the block's limit cut short (the reference's interrupted row, SURVEY App. B-14): the columns in front
         // of the limit count for the dictionary and the column ranges, the row itself is not part of the block
-        if (row_open && !reference && n_ne) {
+        if (!CF && row_open && !reference && n_ne) {
           need_finish = final = true;
           fin_row = 0xffffffffu;
           continue;
@@ -1518,6 +1576,7 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
           }
         }
       }
+      if (CF && nl) last_nl_p1 = (uint32_t)(p0 + 32 - __clz(nl));
       const uint32_t fix = (first && p0 <= scan_from && p0 + 32 > scan_from) ? 1u << (scan_from - p0) : 0u;
       uint32_t prevnl = __shfl_up_sync(0xffffffffu, nl >> 31, 1);
       if (lane == 0) prevnl = c_nl;
@@ -1572,7 +1631,7 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
       row_open = true;
       reference = start_abs < t0;
       row_start = start_abs;
-      row_no = pre.rows + rows_seen;
+      row_no = CF ? rows_seen : pre.rows + rows_seen;
       n_ne = tabs = 0;
       cursor = pos;
       for (uint32_t w = lane; w < BW; w += 32u) W.BM[cur][w] = 0u;  // (filled while the fields are extracted)
@@ -1650,12 +1709,25 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
     // ---- the row is complete
     const int64_t term_abs = sb + seg_end;
     if (!reference) {
-      if (tabs != tabs_per_row) atomicMin(&P.meta->bad_row, row_no);  // ConvertToZDW.cpp:336-337
+      if (tabs != tabs_per_row) {  // ConvertToZDW.cpp:336-337
+        if (CF) {
+          if (lane == 0) atomicMin(&P.meta->bad_slot, ((unsigned long long)tile << 32) | row_no);
+        } else {
+          atomicMin(&P.meta->bad_row, row_no);
+        }
+      }
       max_line = max(max_line, (uint32_t)(term_abs - row_start + 1));
     }
-    if (term_abs >= t0) ++rows_seen;
-    need_finish = true;
     fin_row = row_no;
+    if (CF) {  // rows_seen counts the rows the tile owns
+      if (!reference) {
+        ++rows_seen;
+        fin_row = row_no < A.slot_cap ? tile * A.slot_cap + row_no : 0xffffffffu;
+      }
+    } else if (term_abs >= t0) {
+      ++rows_seen;
+    }
+    need_finish = true;
     cursor = seg_end + 1;
   }
   if (bail) {
@@ -1663,6 +1735,31 @@ __global__ void __launch_bounds__(D1_THREADS, 8) k_pass1d(const D1Args A) {
     return;
   }
   if (lane == 0 && max_line) atomicMax(&P.meta->max_line, max_line);
+  if (CF) {
+    last_nl_p1 = __reduce_max_sync(0xffffffffu, last_nl_p1);
+    if (lane == 0) {
+      A.tile_rows[tile] = rows_seen;
+      if (last_nl_p1) atomicMax(&P.meta->last_break_p1, last_nl_p1);
+      if (rows_seen > A.slot_cap) *reinterpret_cast<volatile uint32_t*>(&P.meta->slot_overflow) = 1u;
+    }
+  }
+}
+
+// Census-free mode, behind pass 1: the rows of tile t start at base[t] (an exclusive scan of tile_rows, whose total is
+// meta->tot_rows); the slots go to the global row_rec / row_cnt, and the first malformed row gets its global number.
+__global__ void k_row_fixup(const uint32_t* __restrict__ tile_rows, const uint32_t* __restrict__ base, uint32_t ntiles,
+                            uint32_t slot_cap, const uint32_t* __restrict__ slot_rec, const uint32_t* __restrict__ slot_cnt,
+                            uint32_t* __restrict__ row_rec, uint32_t* __restrict__ row_cnt, EncMeta* __restrict__ meta) {
+  if (meta->delta_bail || meta->slot_overflow) return;  // the block is run again: the counts may be incomplete
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i == 0 && meta->bad_slot != ~0ull) meta->bad_row = base[meta->bad_slot >> 32] + (uint32_t)meta->bad_slot;
+  const uint64_t tile = i / slot_cap;
+  if (tile >= ntiles) return;
+  const uint32_t j = (uint32_t)(i - tile * slot_cap);
+  if (j < tile_rows[tile]) {
+    row_rec[base[tile] + j] = slot_rec[i];
+    row_cnt[base[tile] + j] = slot_cnt[i];
+  }
 }
 
 // Second half of the row-delta pass 1: the value of every listed field (parseInput's strtoull / CHAR tuple /
@@ -2500,8 +2597,13 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
   ZDWB_TRY(types_d.alloc(ctx, ncols));
   EncMeta* meta = meta_d.as<EncMeta>();
   EncMeta* hmeta = static_cast<EncMeta*>(ctx->meta_host);
-  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(meta, 0, sizeof(EncMeta), st));
-  ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(&meta->bad_row, 0xff, 4, st));  // 0xffffffff = no malformed row
+  auto reset_meta = [&]() -> int {
+    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(meta, 0, sizeof(EncMeta), st));
+    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(&meta->bad_row, 0xff, 4, st));  // 0xffffffff = no malformed row
+    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(&meta->bad_slot, 0xff, 8, st));
+    return ZDWB_OK;
+  };
+  ZDWB_TRY(reset_meta());
   {
     void* pinned = stage_take(ctx, ncols);
     if (!pinned) {
@@ -2517,14 +2619,23 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
   const uint64_t DELTA_MIN_ROW_BYTES = 512;
   bool delta = !probe && ctx->enc_delta != 0 && ncols <= DELTA_MAX_COLS && n >= 64 &&
                (ctx->enc_delta == 1 || (!ctx->delta_bailed && (ctx->last_row_bytes == 0 || ctx->last_row_bytes >= DELTA_MIN_ROW_BYTES)));
+  // A delta block that is not cut (max_rows) can do without the row census: pass 1 finds every tile's reference row
+  // itself and numbers the tile's rows from 0 (k_pass1d<true>, then k_row_fixup), which saves a read of the TSV and a
+  // host round trip.  Automatic once a delta block of this context has shown how wide the rows are; the first block of
+  // a context, cut blocks and blocks whose tiles hold more rows than they have slots for take the census (and after such
+// a fall-back, the context's later blocks).
+  bool census_free = delta && opts->max_rows == 0 &&
+                     (ctx->enc_census == 0 || (ctx->enc_census < 0 && ctx->last_row_bytes >= DELTA_MIN_ROW_BYTES &&
+                                               !ctx->delta_bailed && ctx->last_records && !ctx->census_fell_back));
 
   DevBuf agg, colset, colmin, colmax, slots, rec_col, rec_val, row_rec, row_cnt, chg_start, chg_len, csize, cbase, used_idx, used_cols;
+  DevBuf slot_rec, slot_cnt, tile_rows, tile_base;
   HashTable ht{nullptr, 0};
   uint32_t nrows = 0;
   bool is_last = false;
   uint32_t spill_row_len = 0, tail_bytes = 0;
   uint64_t rows_total = 0, ne_total = 0;
-  for (;;) {  // at most twice: the delta variant may hand the block over to the general one
+  for (;;) {  // the census-free run may hand the block to the census, the delta variant to the general one
     // ---- census: per-tile counts and their prefix
     // (delta: a warp walks its tile row by row, so a small input is cut into smaller tiles - down to 8 KiB - until there
     // are about as many as warps fit on the GPU; every tile re-reads the row in front of it, which is why not smaller)
@@ -2538,72 +2649,97 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     const uint64_t span = (uint64_t)(-lo) + n;
     const uint32_t ntiles = (uint32_t)((span + tile_bytes - 1) / tile_bytes);
     const uint32_t tile_ctas = (ntiles + ENC_WARPS - 1) / ENC_WARPS;
-    ZDWB_TRY(agg.alloc(ctx, (size_t)ntiles * sizeof(TileAgg)));
-    if (delta)
-      ZDWB_TRY(launch(ctx, "k_row_census", k_row_census, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>()));
-    else
-      ZDWB_TRY(launch(ctx, "k_tile_count", k_tile_count, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, agg.as<TileAgg>()));
-    {
-      const uint32_t nparts = (ntiles + TS_THREADS - 1) / TS_THREADS;
-      DevBuf part;
-      ZDWB_TRY(part.alloc(ctx, (size_t)nparts * sizeof(TileAgg)));
-      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_local, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
-      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan, 1, TS_THREADS, 0, part.as<TileAgg>(), nparts, meta));
-      ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_add, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
+    // census-free: row slots per tile.  A valid row is at least ncols bytes (its tabs and terminator), so
+    // ceil(tile / ncols) always suffice; in automatic mode a quarter of the previous block's mean row bounds them for
+    // narrow schemas
+    uint32_t slot_cap = 0;
+    if (census_free) {
+      const uint64_t min_row = std::max<uint64_t>({(uint64_t)ncols, 2, ctx->enc_census < 0 ? ctx->last_row_bytes / 4 : 0});
+      slot_cap = (uint32_t)((tile_bytes + min_row - 1) / min_row);
+      if ((uint64_t)ntiles * slot_cap > (n >> 3) + (1u << 20)) census_free = false;  // too many slots: take the census
     }
-    ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
-    ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    rows_total = hmeta->tot_rows;
-    const uint64_t tail_start = hmeta->last_break_p1;  // first byte after the last row break
-    out->rows_in_buffer = rows_total;
-    if (rows_total == 0) {
-      out->tsv_consumed = opts->more_input_follows ? 0 : n;  // a window without a complete row: the caller widens it
-      return ZDWB_OK;  // "Empty data file -- nothing to process", ConvertToZDW.cpp:824-835
-    }
-    ctx->last_row_bytes = std::max<uint64_t>(1, tail_start / rows_total);
-    if (delta && ctx->enc_delta != 1 && ctx->last_row_bytes < DELTA_MIN_ROW_BYTES) {
-      delta = false;  // narrow rows: the general pass 1 (and its census)
-      continue;
-    }
-
-    const uint64_t nrows64 = (opts->max_rows && opts->max_rows < rows_total) ? opts->max_rows : rows_total;
-    nrows = (uint32_t)nrows64;
-    const bool took_all = nrows64 == rows_total;
-    is_last = took_all && !opts->more_input_follows;
-
-    // ---- block extent
-    uint64_t limit;  // bytes that belong to the block
-    spill_row_len = 0;  // the interrupted row was read in full before it was dropped: it counts for longestLine
-    tail_bytes = 0;
-    if (took_all) {
-      // the terminator of the last row is the last row break unless blank lines follow it; either way every
-      // delimiter in front of tail_start belongs to the block
-      limit = tail_start;
-      if (is_last) {
-        out->tsv_consumed = n;
-        tail_bytes = (uint32_t)(n - tail_start);
-      } else {
-        out->tsv_consumed = tail_start;  // the unterminated tail belongs to the next window
+    uint64_t limit = n;  // bytes that belong to the block (census-free: pass 1 drops a row the buffer's end cuts short)
+    // The block's rows and extent from the window's totals in hmeta (census: before pass 1; census-free: after it, and
+    // never cut).  *next: 0 = go on, 1 = the window holds no complete row, 2 = narrow rows: the general variant.
+    auto settle = [&](int* next) -> int {
+      *next = 0;
+      rows_total = hmeta->tot_rows;
+      const uint64_t tail_start = hmeta->last_break_p1;  // first byte after the last row break
+      out->rows_in_buffer = rows_total;
+      if (rows_total == 0) {
+        out->tsv_consumed = opts->more_input_follows ? 0 : n;  // a window without a complete row: the caller widens it
+        *next = 1;
+        return ZDWB_OK;  // "Empty data file -- nothing to process", ConvertToZDW.cpp:824-835
       }
-    } else {
-      ZDWB_TRY(launch(ctx, "k_find_cut", k_find_cut, 1, 32, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>(), nrows - 1, meta));
-      ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
-      ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-      limit = hmeta->cut_end_p1;
-      out->tsv_consumed = hmeta->next_start;
-      {
-        // the row behind the block has been read in full when the block is closed - the row buffer has grown with it
-        // (getnextrow.cpp:57-65), so its length counts for longestLine - and its first spill_cols columns have been parsed
-        ZDWB_TRY(launch(ctx, "k_find_spill", k_find_spill, 1, 1, 0, buf, n, hmeta->next_start, opts->spill_cols, meta));
+      ctx->last_row_bytes = std::max<uint64_t>(1, tail_start / rows_total);
+      if (delta && ctx->enc_delta != 1 && ctx->last_row_bytes < DELTA_MIN_ROW_BYTES) {
+        *next = 2;  // narrow rows: the general pass 1 (and its census)
+        return ZDWB_OK;
+      }
+
+      const uint64_t nrows64 = (opts->max_rows && opts->max_rows < rows_total) ? opts->max_rows : rows_total;
+      nrows = (uint32_t)nrows64;
+      const bool took_all = nrows64 == rows_total;
+      is_last = took_all && !opts->more_input_follows;
+
+      // ---- block extent
+      spill_row_len = 0;  // the interrupted row was read in full before it was dropped: it counts for longestLine
+      tail_bytes = 0;
+      if (took_all) {
+        // the terminator of the last row is the last row break unless blank lines follow it; either way every
+        // delimiter in front of tail_start belongs to the block
+        limit = tail_start;
+        if (is_last) {
+          out->tsv_consumed = n;
+          tail_bytes = (uint32_t)(n - tail_start);
+        } else {
+          out->tsv_consumed = tail_start;  // the unterminated tail belongs to the next window
+        }
+      } else {
+        ZDWB_TRY(launch(ctx, "k_find_cut", k_find_cut, 1, 32, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>(), nrows - 1, meta));
         ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
         ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        if (hmeta->spill_row_len) {
-          if (opts->spill_cols) limit = hmeta->spill_end;  // pass 1 takes every field whose closing delimiter lies in front of this
-          spill_row_len = hmeta->spill_row_len;
+        limit = hmeta->cut_end_p1;
+        out->tsv_consumed = hmeta->next_start;
+        {
+          // the row behind the block has been read in full when the block is closed - the row buffer has grown with it
+          // (getnextrow.cpp:57-65), so its length counts for longestLine - and its first spill_cols columns have been parsed
+          ZDWB_TRY(launch(ctx, "k_find_spill", k_find_spill, 1, 1, 0, buf, n, hmeta->next_start, opts->spill_cols, meta));
+          ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
+          ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+          if (hmeta->spill_row_len) {
+            if (opts->spill_cols) limit = hmeta->spill_end;  // pass 1 takes every field whose closing delimiter lies in front of this
+            spill_row_len = hmeta->spill_row_len;
+          }
         }
       }
+      out->nrows = nrows;
+      return ZDWB_OK;
+    };
+    if (!census_free) {
+      ZDWB_TRY(agg.alloc(ctx, (size_t)ntiles * sizeof(TileAgg)));
+      if (delta)
+        ZDWB_TRY(launch(ctx, "k_row_census", k_row_census, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, tile_bytes, agg.as<TileAgg>()));
+      else
+        ZDWB_TRY(launch(ctx, "k_tile_count", k_tile_count, tile_ctas, ENC_THREADS, 0, buf, n, lo, ntiles, agg.as<TileAgg>()));
+      {
+        const uint32_t nparts = (ntiles + TS_THREADS - 1) / TS_THREADS;
+        DevBuf part;
+        ZDWB_TRY(part.alloc(ctx, (size_t)nparts * sizeof(TileAgg)));
+        ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_local, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
+        ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan, 1, TS_THREADS, 0, part.as<TileAgg>(), nparts, meta));
+        ZDWB_TRY(launch(ctx, "k_tile_scan", k_tile_scan_add, nparts, TS_THREADS, 0, agg.as<TileAgg>(), ntiles, part.as<TileAgg>()));
+      }
+      ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
+      ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+      int next;
+      ZDWB_TRY(settle(&next));
+      if (next == 1) return ZDWB_OK;
+      if (next == 2) {
+        delta = false;
+        continue;
+      }
     }
-    out->nrows = nrows;
 
     // ---- pass 1 (retry with a larger hash set / larger record arrays when they fill up)
     ZDWB_TRY(colset.alloc(ctx, (size_t)ncols * 4));
@@ -2615,13 +2751,21 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ZDWB_TRY(used_cols.alloc(ctx, (size_t)ncols * 4));
     ne_total = hmeta->tot_ne;  // (general variant only: the delta census does not count fields)
     uint64_t rec_cap = 0;
+    const uint64_t nslots = (uint64_t)ntiles * slot_cap;
     if (delta) {
       // a row's records = its changed fields + the columns that became empty; sized from the previous block of the
       // file (blocks look alike) or from the bytes, and grown on overflow
       rec_cap = std::max<uint64_t>({ctx->last_records + ctx->last_records / 2, limit / 16, (uint64_t)1 << 16});
       rec_cap = std::min<uint64_t>(rec_cap, limit + 64);
-      ZDWB_TRY(row_rec.alloc(ctx, (size_t)(nrows + 2) * 4));
-      ZDWB_TRY(row_cnt.alloc(ctx, (size_t)(nrows + 2) * 4));
+      const uint64_t rows_cap = census_free ? nslots : nrows;
+      ZDWB_TRY(row_rec.alloc(ctx, (size_t)(rows_cap + 2) * 4));
+      ZDWB_TRY(row_cnt.alloc(ctx, (size_t)(rows_cap + 2) * 4));
+      if (census_free) {
+        ZDWB_TRY(slot_rec.alloc(ctx, (size_t)nslots * 4));
+        ZDWB_TRY(slot_cnt.alloc(ctx, (size_t)nslots * 4));
+        ZDWB_TRY(tile_rows.alloc(ctx, (size_t)ntiles * 4));
+        ZDWB_TRY(tile_base.alloc(ctx, (size_t)ntiles * 4));
+      }
     } else {
       rec_cap = ne_total;
       ZDWB_TRY(row_rec.alloc(ctx, (size_t)(rows_total + 2) * 4));
@@ -2666,24 +2810,36 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       A.colmax = colmax.as<unsigned long long>();
       A.rec_col = rec_col.as<uint32_t>();
       A.rec_val = rec_val.as<unsigned long long>();
-      A.row_rec = row_rec.as<uint32_t>();
+      A.row_rec = census_free ? slot_rec.as<uint32_t>() : row_rec.as<uint32_t>();
       A.meta = meta;
       if (delta) {
         D1Args D;
         D.P = A;
         D.ntiles = p1_tiles;
         D.tile_bytes = tile_bytes;
-        D.nrows = nrows;
+        D.nrows = census_free ? (uint32_t)nslots : nrows;
         D.rec_cap = (uint32_t)rec_cap;
-        D.row_cnt = row_cnt.as<uint32_t>();
+        D.row_cnt = census_free ? slot_cnt.as<uint32_t>() : row_cnt.as<uint32_t>();
         D.chg_start = chg_start.as<uint32_t>();
         D.chg_len = chg_len.as<uint32_t>();
-        ZDWB_TRY(launch(ctx, "k_pass1d", k_pass1d, (p1_tiles + D1_WARPS - 1) / D1_WARPS, D1_THREADS, 0, D));
+        D.slot_cap = slot_cap;
+        D.tile_rows = tile_rows.as<uint32_t>();
+        const uint32_t d1_ctas = (p1_tiles + D1_WARPS - 1) / D1_WARPS;
+        if (census_free)
+          ZDWB_TRY(launch(ctx, "k_pass1d", k_pass1d<true>, d1_ctas, D1_THREADS, 0, D));
+        else
+          ZDWB_TRY(launch(ctx, "k_pass1d", k_pass1d<false>, d1_ctas, D1_THREADS, 0, D));
         D1List L;
         L.start = chg_start.as<uint32_t>();
         L.len = chg_len.as<uint32_t>();
         L.col = rec_col.as<uint32_t>();
         ZDWB_TRY(launch(ctx, "k_pass1d_values", k_pass1d_values, ctx->sm_count * 4, ENC_THREADS, 0, A, L, (uint32_t)rec_cap));
+        if (census_free) {  // global row numbers; their total comes back with pass 1's read-back
+          ZDWB_TRY(exclusive_scan_u32(ctx, tile_rows.as<uint32_t>(), tile_base.as<uint32_t>(), p1_tiles, &meta->tot_rows));
+          ZDWB_TRY(launch(ctx, "k_row_fixup", k_row_fixup, (unsigned)((nslots + 255) / 256), 256, 0, tile_rows.as<uint32_t>(),
+                          tile_base.as<uint32_t>(), p1_tiles, slot_cap, slot_rec.as<uint32_t>(), slot_cnt.as<uint32_t>(),
+                          row_rec.as<uint32_t>(), row_cnt.as<uint32_t>(), meta));
+        }
       } else {
         ZDWB_TRY(launch(ctx, "k_pass1", k_pass1, (p1_tiles + ENC_WARPS - 1) / ENC_WARPS, ENC_THREADS, 0, A));
       }
@@ -2697,7 +2853,8 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
         bailed = true;
         break;
       }
-      if (hmeta->bad_row < nrows) break;
+      if (hmeta->slot_overflow) break;
+      if (hmeta->bad_row < (census_free ? hmeta->tot_rows : nrows)) break;
       const bool ht_full = hmeta->ht_overflow || hmeta->n_unique * 2 > cap;
       const bool rec_full = hmeta->rec_overflow != 0;
       if (!ht_full && !rec_full) break;
@@ -2728,12 +2885,29 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(meta, hmeta, sizeof(EncMeta), cudaMemcpyHostToDevice, st));
       ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
     }
+    if (census_free) {
+      int next = 0;
+      if (bailed || hmeta->slot_overflow) {
+        // A tile holds more rows than its slots, or a warp gave up: no row starts within the delta path's row limit
+        // in front of its tile (a long run of blank lines, say), or a row runs past the limit (possibly the dropped
+        // tail).  The census decides this block - it bails only where the row-delta pass cannot take the block - and
+        // the context's later blocks take the census too, so that such a file does not run pass 1 twice a block.
+        census_free = false;
+        ctx->census_fell_back = true;
+      } else {
+        ZDWB_TRY(settle(&next));
+        if (next == 1) return ZDWB_OK;
+        if (next == 0) break;
+        delta = census_free = false;
+      }
+      ZDWB_TRY(reset_meta());
+      continue;
+    }
     if (!bailed) break;
     // a row with more non-empty fields (or bytes) than a warp's lists hold: the whole block takes the general path
-    delta = false;
+    delta = census_free = false;
     ctx->delta_bailed = true;
-    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(meta, 0, sizeof(EncMeta), st));
-    ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(&meta->bad_row, 0xff, 4, st));
+    ZDWB_TRY(reset_meta());
   }
   if (hmeta->bad_row < nrows) {
     out->bad_row = hmeta->bad_row + 1;  // "Row %u had the problem": one past the last good row, ConvertToZDW.cpp:811
