@@ -83,8 +83,9 @@ int zdwb_ctx_set_stream(zdwb_ctx* ctx, void* cuda_stream);
 
 /* Tuning / test knobs (name = value); every default is what the measurements in DESIGN.md picked.  Encode:
  * "enc_delta" (pass-1 variant: 1 = row-delta, 0 = general, -1 = by row width), "enc_dtile" (bytes per row-delta tile, a
- * power of two >= 2048; 0 = by input size), "enc_p2_rows" (rows per pass-2 tile, 0 = automatic), "small_sort_max"
- * (largest dictionary ranked by the tile-sort path instead of the radix sort), "sort_radix_items" (records per thread
+ * power of two >= 2048; 0 = by input size), "enc_p2_rows" (rows per pass-2 tile of the general path, 0 = automatic;
+ * the row-delta path writes every row from its own records and has no tiles), "small_sort_max" (largest dictionary
+ * ranked by the tile-sort path instead of the radix sort), "sort_radix_items" (records per thread
  * in the radix passes: 4 or 16, 0 = by size), "ht_initial_log2" (first-try size of the string hash set).  Decode:
  * "dec_delta" (0/1: rows of wide schemas are assembled from the row before), "dec_strip_rows" (rows per strip of the row
  * kernels, 0 = automatic), "dec_group_lanes" (lanes per row in the narrow-schema kernels: 8, 16, 32, 0 = by schema

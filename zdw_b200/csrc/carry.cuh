@@ -1,6 +1,5 @@
 // carry.cuh -- "last explicit value per column" carried across strips of rows (used by the decoder for the
-// reference's columnVal[] state, UnconvertFromZDW.cpp:985-986,1349-1453, and by the encoder's row-delta pass 2 for the
-// previous-row values of ConvertToZDW.cpp:504-505,532,548,567).
+// reference's columnVal[] state, UnconvertFromZDW.cpp:985-986,1349-1453).
 //
 // Input: for every strip s and used column u, shas[s*U+u] = the strip holds an explicit value for the column and
 // sval[s*U+u] = the last one.  Output: cin[s*U+u] = the value the column has where strip s begins (0 at block start).

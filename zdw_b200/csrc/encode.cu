@@ -16,6 +16,7 @@
 //                                 Dictionary::write              dictionary.cpp:76-111
 //   k_col_stats, k_col_info, k_block_header   writeLookupColumnStats         ConvertToZDW.cpp:417-483, :839-842
 //   k_pass2, k_gather_tiles       writeBlockRows                 ConvertToZDW.cpp:486-606 + Dictionary::getOffset :53-59
+//   k_p2d_rowlen, k_p2d_emit      the same for the row-delta path, from each row's own records
 //
 // Data layout in HBM: the TSV block is read twice (census, pass 1; the census-free row-delta pass 1 reads it once);
 // records are 12 B per NON-EMPTY field (most fields of analytics-shaped data are empty and cost nothing beyond their
@@ -25,7 +26,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "carry.cuh"
 
 namespace zdwb {
 
@@ -38,6 +38,8 @@ constexpr uint32_t STEP = 512;            // bytes per warp step (32 lanes x 16 
 constexpr uint32_t HT_MAX_PROBE = 2048;
 constexpr uint32_t SHORT_MAX = 16;        // texts up to this length are hashed / compared by one lane, straight-line
 constexpr uint32_t REC_EMPTY = 0xffffffffu;
+// row-delta records: rec_col bit 31 = the value equals the row before's (no repeat flag); columns are < 4096 there
+constexpr uint32_t REC_SAME = 1u << 31;
 
 struct EncMeta {
   uint32_t bad_row;        // first row whose field count != schema (0xffffffff = none)
@@ -786,31 +788,48 @@ __device__ __forceinline__ void p1_process(const P1Args& A, const uint32_t* wlas
   const bool live = valid && len != 0u;
   const bool text = is_text_like(t);
   if (BIAS == 0u && valid && len == 0u) A.rec_col[ord] = REC_EMPTY;  // -t turned the field into an empty one (or the row is malformed)
-  if (live && !text) {
-    unsigned long long v1, v2;
-    if (len <= NUM_FAST_MAX || t == ZDWB_CHAR) {
-      uint32_t x[5];
-      short_words<5>(A.buf + start, len, wlast, x);
-      if (t == ZDWB_CHAR) {
-        // sign-extended first byte (+ second byte * 256): min/max rule ConvertToZDW.cpp:358-361 (second byte only
-        // after a backslash), pass-2 rule :543-547 (always); bytes past the field read as NUL (x is masked)
-        const long long b0 = (long long)(int8_t)(x[0] & 0xffu);
-        const long long b1 = len > 1 ? (long long)((int32_t)(int8_t)((x[0] >> 8) & 0xffu) * 256) : 0ll;
-        v1 = (unsigned long long)(b0 + ((x[0] & 0xffu) == (uint32_t)'\\' ? b1 : 0ll));
-        v2 = (unsigned long long)(b0 + b1);
-      } else {
-        // strtoull (:385,564): an optional sign in front of the digits ('-' negates modulo 2^64; with a sign at most
-        // 19 digits are left, which cannot overflow); anything else - white space, junk - takes the exact byte walk
-        if (!fast_number(x, len, &v1)) v1 = parse_u64_field(A.buf + start, len);
-        v2 = v1;
+  // The row-delta path (BIAS 1) also takes the "became empty" records (len 0), and parses the field the column had in
+  // the row before as well - k_pass1d left its place in rec_val - so that the record can say whether the value changed
+  if (!text && (BIAS == 0u ? live : valid)) {
+    unsigned long long v1 = 0, v2 = 0, old = 0;
+    const unsigned long long prev = BIAS ? A.rec_val[ord] : 0ull;
+#pragma unroll 1
+    for (uint32_t h = 0; h < (BIAS ? 2u : 1u); ++h) {
+      const uint32_t fs = h ? (uint32_t)(prev >> 32) : start, fl = h ? (uint32_t)prev : len;
+      unsigned long long a = 0, b = 0;
+      if (fl && (fl <= NUM_FAST_MAX || t == ZDWB_CHAR)) {
+        uint32_t x[5];
+        short_words<5>(A.buf + fs, fl, wlast, x);
+        if (t == ZDWB_CHAR) {
+          // sign-extended first byte (+ second byte * 256): min/max rule ConvertToZDW.cpp:358-361 (second byte only
+          // after a backslash), pass-2 rule :543-547 (always); bytes past the field read as NUL (x is masked)
+          const long long b0 = (long long)(int8_t)(x[0] & 0xffu);
+          const long long b1 = fl > 1 ? (long long)((int32_t)(int8_t)((x[0] >> 8) & 0xffu) * 256) : 0ll;
+          a = (unsigned long long)(b0 + ((x[0] & 0xffu) == (uint32_t)'\\' ? b1 : 0ll));
+          b = (unsigned long long)(b0 + b1);
+        } else {
+          // strtoull (:385,564): an optional sign in front of the digits ('-' negates modulo 2^64; with a sign at most
+          // 19 digits are left, which cannot overflow); anything else - white space, junk - takes the exact byte walk
+          if (!fast_number(x, fl, &a)) a = parse_u64_field(A.buf + fs, fl);
+          b = a;
+        }
+      } else if (fl) {  // a number of more than 20 characters
+        a = b = parse_u64_field(A.buf + fs, fl);
       }
-    } else {  // a number of more than 20 characters
-      v1 = v2 = parse_u64_field(A.buf + start, len);
+      if (h) {
+        old = b;
+      } else {
+        v1 = a;
+        v2 = b;
+      }
     }
-    A.rec_col[ord] = col;
+    // (pass 2's flag is mapped(v2) != mapped(old), mapped(v) = v ? v - base : 0.  That is v2 != old: subtracting the
+    // base is injective, and a non-zero v2 never equals the base - DESIGN 3 shows it for CHAR cells too)
+    A.rec_col[ord] = BIAS && v2 == old ? col | REC_SAME : col;
     A.rec_val[ord] = v2;
     note_column_value(A, col, v1);
   }
+  if (BIAS != 0u && valid && text && len == 0u) A.rec_val[ord] = 0ull;  // a text column became empty: value 0, flag set
   const bool is_text = live && text;
   uint32_t waiting[2];
   waiting[0] = side_push(Q[0], is_text && len <= SHORT_MAX, start, len, col, ord);
@@ -1036,7 +1055,8 @@ struct D1Args {
   uint32_t tile_bytes;   // DTILE, or a smaller power of two when the input is too small to fill the GPU with DTILE tiles
   uint32_t nrows;        // rows of the block: the spilled row beyond it has records but no row entry
   uint32_t rec_cap;      // capacity of the record arrays
-  uint32_t* row_cnt;     // [nrows] records of row r; they start at P.row_rec[r]
+  uint32_t* row_cnt;     // [nrows] records of row r (low 16 bits; they start at P.row_rec[r]), the first (high 16 bits)
+                         // of which are its "became empty" records: two runs, each in column order
   uint32_t* chg_start;   // [rec_cap] where the changed field of record k starts in the TSV ...
   uint32_t* chg_len;     // ... and its length; 0 = the record of a column that became empty (value 0)
   // census-free mode only: row j of tile t goes to slot t * slot_cap + j of P.row_rec / row_cnt
@@ -1256,6 +1276,16 @@ __device__ __forceinline__ bool warp_differ(const uint8_t* __restrict__ a, const
   return false;
 }
 
+// Where column `col` of the row before (lists of `prv`) lies in the TSV: (start << 32) | len, 0 = it was empty.  Every
+// record carries this in its rec_val until k_pass1d_values has compared the two values and put the new one there.
+__device__ __forceinline__ unsigned long long d1_prev_field(const D1Warp& W, uint32_t prv, uint32_t col, int64_t prev_start) {
+  const uint32_t pw = W.BM[prv][col >> 5], bit = col & 31u;
+  if (!((pw >> bit) & 1u)) return 0ull;
+  const uint32_t j = (uint32_t)W.PF[prv][col >> 5] + (uint32_t)__popc(pw & bits_below(bit));
+  const uint32_t ps = W.S[prv][j];
+  return ((unsigned long long)(uint32_t)(prev_start + ps) << 32) | ((uint32_t)W.E[prv][j] - ps);
+}
+
 // The open row is complete (n fields in the lists of `cur`, their columns' bits in BM[cur], set while they were
 // extracted): rank prefix of the bitmap; unless it is the reference row,
 // compare with the row before (lists of cur ^ 1), hand out the records and queue the changed fields.
@@ -1395,10 +1425,10 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
   }
   if (r < A.nrows && lane == 0) {
     P.row_rec[r] = base;
-    A.row_cnt[r] = drop ? 0u : cnt;
+    A.row_cnt[r] = drop ? 0u : cnt | (nte << 16);
   }
   if (drop || !cnt) return;
-  // ---- "became empty" records: (column, value 0)
+  // ---- "became empty" records: (column, the field it had in the row before)
   if (nte) {
     uint32_t run = 0;
     for (uint32_t w0 = 0; w0 < BW; w0 += 32u) {
@@ -1416,7 +1446,7 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
         const uint32_t bit = (uint32_t)__ffs(x) - 1u;
         x &= x - 1u;
         P.rec_col[at] = w * 32u + bit;
-        P.rec_val[at] = 0ull;
+        P.rec_val[at] = d1_prev_field(W, prv, w * 32u + bit, prev_start);
         A.chg_len[at] = 0u;
         ++at;
       }
@@ -1430,8 +1460,9 @@ __device__ __forceinline__ void d1_finish_row(const D1Args& A, const uint32_t* w
     if (!m) continue;
     const uint32_t k = k0 + lane;
     if ((m >> lane) & 1u) {
-      const uint32_t s = W.S[cur][k], d = at + (uint32_t)__popc(m & lanemask_lt());
-      P.rec_col[d] = W.C[k];
+      const uint32_t s = W.S[cur][k], d = at + (uint32_t)__popc(m & lanemask_lt()), col = W.C[k];
+      P.rec_col[d] = col;
+      P.rec_val[d] = d1_prev_field(W, prv, col, prev_start);
       A.chg_start[d] = (uint32_t)(row_start + s);
       A.chg_len[d] = (uint32_t)W.E[cur][k] - s;
     }
@@ -2107,226 +2138,120 @@ __global__ void __launch_bounds__(ENC_THREADS)
 }
 
 // ---------------------------------------------------------------------------------------------
-// pass 2, row-delta variant: the records of a row name only the columns whose field changed against the row before
-// (value 0 = the field became empty; a text's value is its hash-set slot + 1).  A tile of R rows therefore needs the
-// value every used column has where the tile begins: k_p2d_summary reports the last record of every column inside a
-// tile, the k_carry_* kernels (carry.cuh) turn that into the carried-in values, and k_pass2d fills the value matrix
-// forward row by row before flags and value bytes are produced exactly as in k_pass2 (ConvertToZDW.cpp:486-606).
+// pass 2, row-delta variant: the records of a row are exactly the columns whose field changed against the row before,
+// and k_pass1d_values has already decided for each whether the VALUE changed (rec_col without REC_SAME: the reference's
+// flag, ConvertToZDW.cpp:532,548,567).  A row's bytes therefore follow from its own records: k_p2d_rowlen sums the
+// sizes of the flagged columns (before pass 1's read-back, so the exact output size comes back with it), k_p2d_emit
+// writes flags and value bytes straight to the row's place in the output.  A row's records are two runs in column
+// order - the "became empty" ones, then the changed fields - and every value goes behind the sizes of the records of
+// both runs with a smaller column.
 // ---------------------------------------------------------------------------------------------
-struct P2DArgs {
-  const uint32_t* rec_col;
-  const unsigned long long* rec_val;
-  const uint32_t* row_rec;   // [nrows] first record of the row
-  const uint32_t* row_cnt;   // [nrows]
-  uint32_t nrows, R, U, nflag;
-  const ColInfo* cinfo;
-  const uint32_t* slot_off;
-  const uint32_t* used_cols;
-  const uint8_t* csize;
+// value a record stands for in the row stream: dictionary offset / number minus the column's base (0 stays 0)
+__device__ __forceinline__ unsigned long long record_value(const ColInfo& ci, const uint32_t* __restrict__ slot_off,
+                                                           unsigned long long v) {
+  if (v == 0ull) return 0ull;
+  return ci.text ? (unsigned long long)__ldg(slot_off + (uint32_t)(v - 1ull)) : v - ci.base;  // :548,566; Dictionary::getOffset
+}
+
+// one warp per row: row_off[r] = nflag + the sizes of the flagged records' columns (csize is 0 for a column the block
+// does not use).  rows_cap rows are written, those at or past the block's row count with 0, so that an exclusive scan
+// over all of them gives the row offsets and the total; census-free, the row count is only known on the device.
+__global__ void __launch_bounds__(ENC_THREADS)
+    k_p2d_rowlen(const uint32_t* __restrict__ rec_col, const uint32_t* __restrict__ row_rec, const uint32_t* __restrict__ row_cnt,
+                 uint32_t rows_cap, bool census_free, const uint8_t* __restrict__ csize, const EncMeta* __restrict__ meta,
+                 uint64_t* __restrict__ row_off) {
+  // Pass 1 runs again, or the general one: row_off stays unwritten, and the scan behind this kernel leaves a
+  // meaningless meta->rows_bytes, which the host reads only from a run of pass 1 that went through
+  if (meta->delta_bail || meta->rec_overflow || meta->slot_overflow) return;
+  const unsigned lane = lane_id();
+  const uint32_t nrows = census_free ? min(meta->tot_rows, rows_cap) : rows_cap, nflag = meta->nflag;
+  for (uint32_t r = blockIdx.x * ENC_WARPS + (threadIdx.x >> 5); r < rows_cap; r += gridDim.x * ENC_WARPS) {
+    uint32_t acc = 0;
+    if (r < nrows) {
+      const uint32_t k0 = row_rec[r], cnt = row_cnt[r] & 0xffffu;
+      for (uint32_t i = lane; i < cnt; i += 32u) {
+        const uint32_t c = rec_col[k0 + i];
+        if (!(c & REC_SAME)) acc += csize[c];
+      }
+      acc = nflag + __reduce_add_sync(0xffffffffu, acc);
+    }
+    if (lane == 0) row_off[r] = acc;
+  }
+}
+
+struct P2DWarp {                // (16-bit prefixes: a row's value bytes are at most 2 * DCAP * 8; 8 CTAs fit an SM)
+  uint16_t col[2 * DCAP];      // the row's records: column
+  uint16_t pre[2 * DCAP + 1];  // ... value bytes of the records in front of it (record order)
+  uint32_t flags[DBW];         // the row's flag bytes: bit u = used column u
 };
 
-// value a record stands for in the row stream: dictionary offset / number minus the column's base (0 stays 0)
-__device__ __forceinline__ unsigned long long record_value(const P2DArgs& A, const ColInfo& ci, unsigned long long v) {
-  if (v == 0ull) return 0ull;
-  return ci.text ? (unsigned long long)__ldg(A.slot_off + (uint32_t)(v - 1ull)) : v - ci.base;  // :548,566; Dictionary::getOffset
-}
-
-// shared by both kernels: record ranges of the tile's rows; roff[j] = records in front of row j of the tile
-__device__ __forceinline__ void p2d_load_ranges(const P2DArgs& A, uint32_t r0, uint32_t Rn, uint32_t* rstart, uint32_t* roff) {
-  for (uint32_t j = threadIdx.x; j < Rn; j += ENC_THREADS) {
-    rstart[j] = A.row_rec[r0 + j];
-    roff[j + 1] = A.row_cnt[r0 + j];
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
+__global__ void __launch_bounds__(ENC_THREADS)
+    k_p2d_emit(const uint32_t* __restrict__ rec_col, const unsigned long long* __restrict__ rec_val,
+               const uint32_t* __restrict__ row_rec, const uint32_t* __restrict__ row_cnt, const uint64_t* __restrict__ row_off,
+               uint32_t nrows, uint32_t nflag, const ColInfo* __restrict__ cinfo, const uint8_t* __restrict__ csize,
+               const uint32_t* __restrict__ slot_off, uint8_t* __restrict__ rows_out) {
+  __shared__ P2DWarp sw[ENC_WARPS];
+  const unsigned lane = lane_id();
+  P2DWarp& W = sw[threadIdx.x >> 5];
+  const uint32_t nfw = (nflag + 3u) >> 2;
+  for (uint32_t r = blockIdx.x * ENC_WARPS + (threadIdx.x >> 5); r < nrows; r += gridDim.x * ENC_WARPS) {
+    const uint32_t k0 = row_rec[r], cw = row_cnt[r], cnt = cw & 0xffffu, nte = cw >> 16;
+    uint8_t* orow = rows_out + row_off[r];
+    for (uint32_t w = lane; w < nfw; w += 32u) W.flags[w] = 0u;
+    __syncwarp();
+    // ---- columns, value sizes and flags of the records
     uint32_t run = 0;
-    roff[0] = 0;
-    for (uint32_t j = 0; j < Rn; ++j) {
-      run += roff[j + 1];
-      roff[j + 1] = run;
-    }
-  }
-  __syncthreads();
-}
-__device__ __forceinline__ uint32_t p2d_row_of(const uint32_t* roff, uint32_t Rn, uint32_t idx) {
-  uint32_t a = 0, b = Rn;  // last a with roff[a] <= idx
-  while (b - a > 1) {
-    const uint32_t m = (a + b) >> 1;
-    if (roff[m] <= idx) a = m;
-    else b = m;
-  }
-  return a;
-}
-
-__global__ void __launch_bounds__(ENC_THREADS)
-    k_p2d_summary(const P2DArgs A, unsigned long long* __restrict__ sval, uint8_t* __restrict__ shas) {
-  extern __shared__ __align__(16) uint8_t dsm[];
-  int32_t* last_row = reinterpret_cast<int32_t*>(dsm);          // [U]
-  uint32_t* rstart = reinterpret_cast<uint32_t*>(last_row + A.U);  // [R]
-  uint32_t* roff = rstart + A.R;                                 // [R + 1]
-  const uint32_t tile = blockIdx.x, r0 = tile * A.R, Rn = min(A.nrows - r0, A.R);
-  for (uint32_t u = threadIdx.x; u < A.U; u += ENC_THREADS) last_row[u] = -1;
-  p2d_load_ranges(A, r0, Rn, rstart, roff);
-  const uint32_t tot = roff[Rn];
-  for (uint32_t idx = threadIdx.x; idx < tot; idx += ENC_THREADS) {
-    const uint32_t j = p2d_row_of(roff, Rn, idx);
-    const uint32_t col = A.rec_col[rstart[j] + (idx - roff[j])];
-    const int32_t u = __ldg(&A.cinfo[col].u);
-    if (u >= 0) atomicMax(&last_row[u], (int32_t)j);
-  }
-  __syncthreads();
-  for (uint32_t idx = threadIdx.x; idx < tot; idx += ENC_THREADS) {
-    const uint32_t j = p2d_row_of(roff, Rn, idx);
-    const uint32_t k = rstart[j] + (idx - roff[j]);
-    const uint32_t col = A.rec_col[k];
-    const uint4 q = __ldg(reinterpret_cast<const uint4*>(A.cinfo + col));
-    ColInfo ci;
-    ci.base = (unsigned long long)q.x | ((unsigned long long)q.y << 32);
-    ci.u = (int32_t)q.z;
-    ci.text = q.w;
-    if (ci.u >= 0 && last_row[ci.u] == (int32_t)j) sval[(size_t)tile * A.U + (uint32_t)ci.u] = record_value(A, ci, A.rec_val[k]);
-  }
-  for (uint32_t u = threadIdx.x; u < A.U; u += ENC_THREADS) shas[(size_t)tile * A.U + u] = last_row[u] >= 0 ? 1 : 0;
-}
-
-__global__ void __launch_bounds__(ENC_THREADS)
-    k_pass2d(const P2DArgs A, const unsigned long long* __restrict__ cin, uint64_t tile_cap, uint8_t* __restrict__ staging,
-             uint64_t* __restrict__ tile_bytes) {
-  extern __shared__ __align__(16) uint8_t dsm[];
-  // dynamic smem: nval[(R+1)*U] u64 | mark[(R+1)*MW] u32 | rowoff[R+1] | rstart[R] | roff[R+1] | usz[U] u8
-  const uint32_t U = A.U, R = A.R, MW = (U + 31u) >> 5, nflag = A.nflag;
-  unsigned long long* nval = reinterpret_cast<unsigned long long*>(dsm);
-  uint32_t* mark = reinterpret_cast<uint32_t*>(nval + (size_t)(R + 1) * U);
-  uint32_t* rowoff = mark + (size_t)(R + 1) * MW;
-  uint32_t* rstart = rowoff + R + 1;
-  uint32_t* roff = rstart + R;
-  uint8_t* usz = reinterpret_cast<uint8_t*>(roff + R + 1);
-  const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t tile = blockIdx.x, r0 = tile * R, Rn = min(A.nrows - r0, R);
-
-  for (uint32_t u = tid; u < U; u += ENC_THREADS) {
-    nval[u] = cin ? cin[(size_t)tile * U + u] : 0ull;  // the row in front of the tile (all empty at block start, :504-505)
-    usz[u] = A.csize[A.used_cols[u]];
-  }
-  for (uint32_t k = tid; k < (R + 1) * MW; k += ENC_THREADS) mark[k] = 0u;
-  p2d_load_ranges(A, r0, Rn, rstart, roff);
-
-  // ---- the records of the tile's rows: value into the matrix, mark bit set
-  {
-    const uint32_t tot = roff[Rn];
-    constexpr int NR = 4;
-    for (uint32_t ib = tid; ib < tot; ib += NR * ENC_THREADS) {
-      uint32_t row[NR], col[NR];
-      unsigned long long v[NR];
-      ColInfo ci[NR];
-#pragma unroll
-      for (int q = 0; q < NR; ++q) {
-        const uint32_t idx = ib + (uint32_t)q * ENC_THREADS;
-        row[q] = 0;
-        col[q] = REC_EMPTY;
-        v[q] = 0ull;
-        if (idx < tot) {
-          row[q] = p2d_row_of(roff, Rn, idx);
-          const uint32_t k = rstart[row[q]] + (idx - roff[row[q]]);
-          col[q] = A.rec_col[k];
-          v[q] = A.rec_val[k];
+    for (uint32_t i0 = 0; i0 < cnt; i0 += 32u) {
+      const uint32_t i = i0 + lane;
+      uint32_t sz = 0;
+      if (i < cnt) {
+        const uint32_t c = rec_col[k0 + i], col = c & ~REC_SAME;
+        W.col[i] = (uint16_t)col;
+        if (!(c & REC_SAME)) {
+          sz = csize[col];
+          if (sz) {
+            const uint32_t u = (uint32_t)__ldg(&cinfo[col].u);
+            atomicOr(&W.flags[u >> 5], 1u << (u & 31u));
+          }
         }
       }
-#pragma unroll
-      for (int q = 0; q < NR; ++q) {
-        ci[q].u = -1;
-        ci[q].text = 0;
-        ci[q].base = 0;
-        if (col[q] != REC_EMPTY) {
-          const uint4 w = __ldg(reinterpret_cast<const uint4*>(A.cinfo + col[q]));
-          ci[q].base = (unsigned long long)w.x | ((unsigned long long)w.y << 32);
-          ci[q].u = (int32_t)w.z;
-          ci[q].text = w.w;
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < NR; ++q) {
-        if (ci[q].u < 0) continue;
-        const uint32_t u = (uint32_t)ci[q].u;
-        nval[(size_t)(row[q] + 1) * U + u] = record_value(A, ci[q], v[q]);
-        atomicOr(&mark[(size_t)(row[q] + 1) * MW + (u >> 5)], 1u << (u & 31u));
-      }
-    }
-  }
-  __syncthreads();
-  // ---- a column without a record keeps the value of the row before
-  for (uint32_t u = tid; u < U; u += ENC_THREADS) {
-    unsigned long long v = nval[u];
-    for (uint32_t j = 1; j <= Rn; ++j) {
-      if ((mark[(size_t)j * MW + (u >> 5)] >> (u & 31u)) & 1u) v = nval[(size_t)j * U + u];
-      else nval[(size_t)j * U + u] = v;
-    }
-  }
-  __syncthreads();
-
-  // ---- encoded length of every row: nflag + sum of the sizes of the changed columns
-  for (uint32_t j = warp; j < Rn; j += ENC_WARPS) {
-    const unsigned long long* cur = nval + (size_t)(j + 1) * U;
-    const unsigned long long* prv = nval + (size_t)j * U;
-    uint32_t acc = 0;
-    for (uint32_t u = lane; u < U; u += 32)
-      if (cur[u] != prv[u]) acc += usz[u];
-    acc = __reduce_add_sync(0xffffffffu, acc);
-    if (lane == 0) rowoff[j] = nflag + acc;
-  }
-  __syncthreads();
-  if (warp == 0) {
-    uint32_t run = 0;
-    for (uint32_t j0 = 0; j0 < Rn; j0 += 32) {
-      const uint32_t j = j0 + lane;
-      const uint32_t v = j < Rn ? rowoff[j] : 0u;
-      uint32_t inc = v;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= (unsigned)o) inc += t;
-      }
-      if (j < Rn) rowoff[j] = run + inc - v;
-      run += __shfl_sync(0xffffffffu, inc, 31);
-    }
-    if (lane == 0) {
-      rowoff[Rn] = run;
-      tile_bytes[tile] = run;
-    }
-  }
-  __syncthreads();
-  uint8_t* tile_out = staging + (uint64_t)tile * tile_cap;
-
-  // ---- emit: flag bytes, then the low columnSize bytes of every changed value (little-endian)
-  for (uint32_t j = warp; j < Rn; j += ENC_WARPS) {
-    const unsigned long long* cur = nval + (size_t)(j + 1) * U;
-    const unsigned long long* prv = nval + (size_t)j * U;
-    uint8_t* orow = tile_out + rowoff[j];
-    uint32_t voff = nflag;
-    for (uint32_t ub = 0; ub < U; ub += 32) {
-      const uint32_t u = ub + lane;
-      unsigned long long v = 0;
-      bool flag = false;
-      if (u < U) {
-        v = cur[u];
-        flag = v != prv[u];
-      }
-      const unsigned bal = __ballot_sync(0xffffffffu, flag);
-      if (lane < 4 && (ub >> 3) + lane < nflag) orow[(ub >> 3) + lane] = (uint8_t)(bal >> (8 * lane));
-      const uint32_t sz = flag ? usz[u] : 0u;
       uint32_t inc = sz;
 #pragma unroll
       for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
+        const uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
         if (lane >= (unsigned)o) inc += t;
       }
-      const uint32_t tot = __shfl_sync(0xffffffffu, inc, 31);
-      if (flag) {
-        uint8_t* d = orow + voff + inc - sz;
-        for (uint32_t b = 0; b < sz; ++b) d[b] = (uint8_t)(v >> (8 * b));
-      }
-      voff += tot;
+      if (i < cnt) W.pre[i] = (uint16_t)(run + inc - sz);
+      run += __shfl_sync(0xffffffffu, inc, 31);
     }
+    if (lane == 0) W.pre[cnt] = (uint16_t)run;
+    __syncwarp();
+    for (uint32_t b = lane; b < nflag; b += 32u) orow[b] = (uint8_t)(W.flags[b >> 2] >> (8u * (b & 3u)));
+    // ---- value bytes (low csize bytes, little-endian): behind the flagged records of its own run in front of it and
+    // those of the other run with a smaller column (a column is in at most one of the runs)
+    for (uint32_t i = lane; i < cnt; i += 32u) {
+      const uint32_t sz = (uint32_t)W.pre[i + 1] - W.pre[i];
+      if (!sz) continue;
+      const uint32_t col = W.col[i];
+      const bool first = i < nte;
+      const uint32_t ob = first ? nte : 0u, oe = first ? cnt : nte;
+      uint32_t lo = ob, hi = oe;  // first record of the other run whose column is not smaller
+      while (lo < hi) {
+        const uint32_t m = (lo + hi) >> 1;
+        if (W.col[m] < col) lo = m + 1;
+        else hi = m;
+      }
+      const uint32_t own = first ? (uint32_t)W.pre[i] : (uint32_t)W.pre[i] - W.pre[nte];
+      const uint4 q = __ldg(reinterpret_cast<const uint4*>(cinfo + col));
+      ColInfo ci;
+      ci.base = (unsigned long long)q.x | ((unsigned long long)q.y << 32);
+      ci.u = (int32_t)q.z;
+      ci.text = q.w;
+      const unsigned long long v = record_value(ci, slot_off, rec_val[k0 + i]);
+      uint8_t* d = orow + nflag + own + ((uint32_t)W.pre[lo] - W.pre[ob]);
+      for (uint32_t b = 0; b < sz; ++b) d[b] = (uint8_t)(v >> (8u * b));
+    }
+    __syncwarp();  // the next row refills the lists
   }
 }
 
@@ -2629,7 +2554,7 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
                                                !ctx->delta_bailed && ctx->last_records && !ctx->census_fell_back));
 
   DevBuf agg, colset, colmin, colmax, slots, rec_col, rec_val, row_rec, row_cnt, chg_start, chg_len, csize, cbase, used_idx, used_cols;
-  DevBuf slot_rec, slot_cnt, tile_rows, tile_base;
+  DevBuf slot_rec, slot_cnt, tile_rows, tile_base, row_off;
   HashTable ht{nullptr, 0};
   uint32_t nrows = 0;
   bool is_last = false;
@@ -2752,14 +2677,15 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ne_total = hmeta->tot_ne;  // (general variant only: the delta census does not count fields)
     uint64_t rec_cap = 0;
     const uint64_t nslots = (uint64_t)ntiles * slot_cap;
+    const uint64_t rows_cap = census_free ? nslots : nrows;  // (delta: rows pass 1 can number)
     if (delta) {
       // a row's records = its changed fields + the columns that became empty; sized from the previous block of the
       // file (blocks look alike) or from the bytes, and grown on overflow
       rec_cap = std::max<uint64_t>({ctx->last_records + ctx->last_records / 2, limit / 16, (uint64_t)1 << 16});
       rec_cap = std::min<uint64_t>(rec_cap, limit + 64);
-      const uint64_t rows_cap = census_free ? nslots : nrows;
       ZDWB_TRY(row_rec.alloc(ctx, (size_t)(rows_cap + 2) * 4));
       ZDWB_TRY(row_cnt.alloc(ctx, (size_t)(rows_cap + 2) * 4));
+      ZDWB_TRY(row_off.alloc(ctx, (size_t)(rows_cap + 2) * 8));
       if (census_free) {
         ZDWB_TRY(slot_rec.alloc(ctx, (size_t)nslots * 4));
         ZDWB_TRY(slot_cnt.alloc(ctx, (size_t)nslots * 4));
@@ -2847,6 +2773,13 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
       ZDWB_TRY(launch(ctx, "k_col_stats", k_col_stats, 1, ENC_THREADS, 0, types_d.as<uint8_t>(), ncols, colset.as<uint32_t>(),
                       colmin.as<unsigned long long>(), colmax.as<unsigned long long>(), csize.as<uint8_t>(),
                       cbase.as<unsigned long long>(), used_idx.as<int32_t>(), used_cols.as<uint32_t>(), meta));
+      if (delta) {  // the rows' places in the row stream; their total (the exact output size) comes back with the read-back
+        const unsigned ctas = (unsigned)std::min<uint64_t>((rows_cap + ENC_WARPS - 1) / ENC_WARPS, (uint64_t)ctx->sm_count * 16);
+        ZDWB_TRY(launch(ctx, "k_p2d_rowlen", k_p2d_rowlen, ctas, ENC_THREADS, 0, rec_col.as<uint32_t>(), row_rec.as<uint32_t>(),
+                        row_cnt.as<uint32_t>(), (uint32_t)rows_cap, census_free, csize.as<uint8_t>(), meta, row_off.as<uint64_t>()));
+        ZDWB_TRY(exclusive_scan_u64(ctx, row_off.as<uint64_t>(), row_off.as<uint64_t>(), rows_cap,
+                                    reinterpret_cast<uint64_t*>(&meta->rows_bytes)));
+      }
       ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(hmeta, meta, sizeof(EncMeta), cudaMemcpyDeviceToHost, st));
       ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
       if (hmeta->delta_bail) {
@@ -2983,26 +2916,28 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
                     offs.as<uint32_t>(), nu, slot_off.as<uint32_t>()));
   }
 
-  // ---- pass 2 into the staging buffer
-  uint64_t rows_bytes = 0;
+  // ---- pass 2.  Row-delta: the row offsets are known already (k_p2d_rowlen), the rows are written into the output
+  // below.  General: into the staging buffer, packed once every tile's length is known.
+  uint64_t rows_bytes = delta ? hmeta->rows_bytes : 0;
   DevBuf staging, tile_bytes, tile_off, rows_total_d, colinfo;
   uint32_t tiles2 = 0;
   uint64_t tile_cap = 0;
   if (U > 0) {
+    ZDWB_TRY(colinfo.alloc(ctx, (size_t)ncols * sizeof(ColInfo)));
+    ZDWB_TRY(launch(ctx, "k_col_info", k_col_info, (ncols + 255) / 256, 256, 0, types_d.as<uint8_t>(), used_idx.as<int32_t>(),
+                    cbase.as<unsigned long long>(), ncols, colinfo.as<ColInfo>()));
+  }
+  if (U > 0 && !delta) {
     // rows per CTA: bounded by the shared-memory value matrix ((R+1) * U * 8 bytes) and a record-count target
     if ((uint64_t)U * 8 * 2 + 1024 > 180 * 1024) {
       ctx->err = "encode: more than 11400 used columns in one block are not supported";
       return ZDWB_ERR_UNSUPPORTED;
     }
     const uint64_t smem_budget = 64 * 1024;
-    const uint32_t MW = (U + 31) / 32;
-    const uint64_t row_smem = (uint64_t)U * 8 + (delta ? (uint64_t)MW * 4 : 0);
-    const uint64_t by_smem = std::max<uint64_t>(2, smem_budget / row_smem);
-    const uint64_t recs = delta ? hmeta->rec_count : ne_total;
-    const uint64_t rec_per_row = std::max<uint64_t>(1, recs / std::max<uint64_t>(delta ? nrows : rows_total, 1));
+    const uint64_t by_smem = std::max<uint64_t>(2, smem_budget / ((uint64_t)U * 8));
+    const uint64_t rec_per_row = std::max<uint64_t>(1, ne_total / std::max<uint64_t>(rows_total, 1));
     uint32_t rpc2 = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1, 4096 / rec_per_row), 1024);
     rpc2 = (uint32_t)std::min<uint64_t>(rpc2, by_smem - 1);
-    if (delta) rpc2 = std::min<uint32_t>(rpc2, 16);  // measured on C4: 16-row tiles (6 CTAs per SM) beat 30-row ones
     if (ctx->enc_p2_rows > 0) rpc2 = (uint32_t)std::min<uint64_t>((uint64_t)ctx->enc_p2_rows, by_smem - 1);
     tiles2 = (nrows + rpc2 - 1) / rpc2;
     tile_cap = (((uint64_t)rpc2 * hmeta->max_row_bytes) + 15) & ~15ull;
@@ -3010,46 +2945,11 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
     ZDWB_TRY(tile_bytes.alloc(ctx, (size_t)tiles2 * 8));
     ZDWB_TRY(tile_off.alloc(ctx, (size_t)tiles2 * 8));
     ZDWB_TRY(rows_total_d.alloc(ctx, 8));
-    ZDWB_TRY(colinfo.alloc(ctx, (size_t)ncols * sizeof(ColInfo)));
-    ZDWB_TRY(launch(ctx, "k_col_info", k_col_info, (ncols + 255) / 256, 256, 0, types_d.as<uint8_t>(), used_idx.as<int32_t>(),
-                    cbase.as<unsigned long long>(), ncols, colinfo.as<ColInfo>()));
-    if (delta) {
-      P2DArgs A2;
-      A2.rec_col = rec_col.as<uint32_t>();
-      A2.rec_val = rec_val.as<unsigned long long>();
-      A2.row_rec = row_rec.as<uint32_t>();
-      A2.row_cnt = row_cnt.as<uint32_t>();
-      A2.nrows = nrows;
-      A2.R = rpc2;
-      A2.U = U;
-      A2.nflag = nflag;
-      A2.cinfo = colinfo.as<ColInfo>();
-      A2.slot_off = slot_off.as<uint32_t>();
-      A2.used_cols = used_cols.as<uint32_t>();
-      A2.csize = csize.as<uint8_t>();
-      // the value every used column has where a tile begins
-      DevBuf cin, sval, shas;
-      if (tiles2 > 1) {
-        ZDWB_TRY(cin.alloc(ctx, (size_t)tiles2 * U * 8));
-        ZDWB_TRY(sval.alloc(ctx, (size_t)tiles2 * U * 8));
-        ZDWB_TRY(shas.alloc(ctx, (size_t)tiles2 * U));
-        const size_t smem_sum = (size_t)U * 4 + (size_t)(2 * rpc2 + 1) * 4 + 16;
-        ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_p2d_summary, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-        ZDWB_TRY(launch(ctx, "k_p2d_summary", k_p2d_summary, tiles2, ENC_THREADS, smem_sum, A2, sval.as<unsigned long long>(),
-                        shas.as<uint8_t>()));
-        ZDWB_TRY(carry_prefix(ctx, sval.as<unsigned long long>(), shas.as<uint8_t>(), tiles2, U, cin.as<unsigned long long>()));
-      }
-      const size_t smem = (size_t)(rpc2 + 1) * U * 8 + (size_t)(rpc2 + 1) * MW * 4 + (size_t)(3 * rpc2 + 3) * 4 + U + 16;
-      ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_pass2d, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-      ZDWB_TRY(launch(ctx, "k_pass2d", k_pass2d, tiles2, ENC_THREADS, smem, A2, tiles2 > 1 ? cin.as<unsigned long long>() : nullptr,
-                      tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>()));
-    } else {
-      const size_t smem = (size_t)(rpc2 + 1) * U * 8 + (size_t)(rpc2 + 1) * 4 + (size_t)(rpc2 + 2) * 4 + U + 16;
-      ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_pass2, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
-      ZDWB_TRY(launch(ctx, "k_pass2", k_pass2, tiles2, ENC_THREADS, smem, rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
-                      row_rec.as<uint32_t>(), nrows, rpc2, colinfo.as<ColInfo>(), slot_off.as<uint32_t>(), used_cols.as<uint32_t>(),
-                      csize.as<uint8_t>(), U, nflag, tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>()));
-    }
+    const size_t smem = (size_t)(rpc2 + 1) * U * 8 + (size_t)(rpc2 + 1) * 4 + (size_t)(rpc2 + 2) * 4 + U + 16;
+    ZDWB_CUDA_TRY(ctx, cudaFuncSetAttribute(k_pass2, cudaFuncAttributeMaxDynamicSharedMemorySize, 190 * 1024));
+    ZDWB_TRY(launch(ctx, "k_pass2", k_pass2, tiles2, ENC_THREADS, smem, rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
+                    row_rec.as<uint32_t>(), nrows, rpc2, colinfo.as<ColInfo>(), slot_off.as<uint32_t>(), used_cols.as<uint32_t>(),
+                    csize.as<uint8_t>(), U, nflag, tile_cap, staging.as<uint8_t>(), tile_bytes.as<uint64_t>()));
     ZDWB_TRY(exclusive_scan_u64(ctx, tile_bytes.as<uint64_t>(), tile_off.as<uint64_t>(), tiles2, rows_total_d.as<uint64_t>()));
     ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(ctx->meta_host) + 1024, rows_total_d.p, 8, cudaMemcpyDeviceToHost, st));
     ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(st));
@@ -3074,6 +2974,12 @@ static int encode_block_run(Ctx* ctx, const zdwb_schema* schema, const void* tsv
   if (tiles2)
     ZDWB_TRY(launch(ctx, "k_gather_tiles", k_gather_tiles, tiles2, ENC_THREADS, 0, staging.as<uint8_t>(), tile_cap,
                     tile_off.as<uint64_t>(), tile_bytes.as<uint64_t>(), outp + rows_base));
+  if (delta && rows_bytes) {
+    const unsigned ctas = (unsigned)std::min<uint64_t>((nrows + ENC_WARPS - 1) / ENC_WARPS, (uint64_t)ctx->sm_count * 16);
+    ZDWB_TRY(launch(ctx, "k_p2d_emit", k_p2d_emit, ctas, ENC_THREADS, 0, rec_col.as<uint32_t>(), rec_val.as<unsigned long long>(),
+                    row_rec.as<uint32_t>(), row_cnt.as<uint32_t>(), row_off.as<uint64_t>(), nrows, nflag, colinfo.as<ColInfo>(),
+                    csize.as<uint8_t>(), slot_off.as<uint32_t>(), outp + rows_base));
+  }
 
   const size_t total_len = (size_t)(rows_base + rows_bytes);
   out->len = total_len;
