@@ -25,6 +25,8 @@
  *        zdwb_encode_block: the way from columns back to a ZDW file
  *   zdwb_match_like, zdwb_find_strings (no counterpart either) answer LIKE and string lookups over a sorted dictionary,
  *        once per distinct string: the filters on text columns
+ *   zdwb_parse_numbers, zdwb_format_numbers (no counterpart either) read DATETIME and DECIMAL dictionary strings as
+ *        numbers and write numbers back as a sorted dictionary
  *
  * Plain C types only; int status codes; no exceptions and no C++ types cross the boundary.  Outputs
  * are owned by the context and stay valid until the next call on the same context.  One context per
@@ -399,6 +401,63 @@ typedef struct {
 
 int zdwb_match_like(zdwb_ctx* ctx, const zdwb_code_part* dict, const zdwb_like_opts* opts, zdwb_match_out* out);
 int zdwb_find_strings(zdwb_ctx* ctx, const zdwb_code_part* dict, const zdwb_strings* queries, zdwb_find_out* out);
+
+/* ---- numbers from and to text (ABI 5) -----------------------------------------------------------
+ * ZDW stores DATETIME and DECIMAL cells as dictionary strings.  These two calls turn a dictionary into numbers, once per
+ * distinct string, and numbers back into a dictionary, so that torch can compute on time and money columns.
+ *
+ * zdwb_parse_numbers: the number of every entry of `dict` (taken as by zdwb_match_like: codes and n are ignored) and of
+ *   opts->null_text, the text of code -1 ("" for text columns, "0.000000000000" for DECIMAL, as zdwb_like_opts).  Every
+ *   text is parsed as it is stored, bytewise: no white space is allowed and nothing is trimmed.  out->values[e] is the
+ *   number and out->ok[e] is 1 when the text is in the grammar and its number fits, else both are 0.  The last element is
+ *   null_text's.
+ *   DATETIME: "YYYY-MM-DD HH:MM:SS", optionally followed by '.' and 1 to 6 digits, or "YYYY-MM-DD" alone (midnight).
+ *     Every field has exactly the digits shown.  Dates run from 0001-01-01 to 9999-12-31 on the proleptic Gregorian
+ *     calendar; hours are 0-23, minutes and seconds 0-59; no time zone is applied.  So "0000-00-00 00:00:00",
+ *     "24:00:00" and "1900-02-29" are not ok.  The value is microseconds since 1970-01-01 00:00:00 (negative before).
+ *   DECIMAL of scale s = opts->digits: [+-]?(D+(\.D*)?|\.D+) with D an ASCII digit; no exponent.  The value is the number
+ *     times 10^s and must be exact (fraction digits past the s-th are '0') and lie in [INT64_MIN, INT64_MAX].  Leading
+ *     zeros and trailing fraction zeros never overflow.  Scale 0 reads the integers a VARCHAR column holds.
+ * zdwb_format_numbers: the inverse, for n values that are strictly increasing (as torch.unique returns them; every value
+ *   is checked against the one before it).  out is a dictionary laid out as zdwb_merge_out's: dense, entries strictly
+ *   increasing bytewise, out->codes[i] the code of values[i]'s text, out->n = n.  So (codes, dict, entry_off) is a row of a
+ *   ColumnTable and its dictionary, fit for zdwb_render_columns, zdwb_match_like, zdwb_find_strings and zdwb_merge_codes.
+ *   DATETIME: "YYYY-MM-DD HH:MM:SS", then '.' and exactly opts->digits fraction digits when digits > 0.
+ *   DECIMAL: an optional '-', the integer digits without leading zeros ("0" when the integer part is zero), then '.' and
+ *     exactly opts->digits digits when digits > 0.  INT64_MIN is written as every other value is.
+ *   Parsing a formatted text with the same opts gives the value back.  With n == 0: dict and codes are NULL, entries and
+ *   dict_bytes 0, and entry_off holds the one offset 0.
+ * Outputs are device memory owned by the context and stay valid until its next call.  The input memory must hold its
+ * final contents when the call is made: the context's stream does not wait for other streams.
+ * Errors (checked before anything is read through the offsets involved; zdwb_last_error names the lowest entry or value at
+ * fault; the context works normally at its next call):
+ *   ZDWB_ERR_BAD_ARG: NULL arguments; a kind that is neither ZDWB_NUM_DATETIME nor ZDWB_NUM_DECIMAL; digits outside 0..18
+ *     (DECIMAL) or, in format, 0..6 (DATETIME); null_text_len > 0 with a NULL null_text; entries > 0 with a NULL dict or
+ *     entry_off; (parse) an entry whose offsets are not entry_off[e] < entry_off[e+1] <= dict_bytes; (format) n > 0 with
+ *     NULL values, a value not greater than the one before it, a DATETIME outside 0001-01-01 00:00:00 ..
+ *     9999-12-31 23:59:59.999999 or not a multiple of 10^(6 - digits) microseconds.
+ *   ZDWB_ERR_UNSUPPORTED: (format) texts of 2^32 bytes or more in all, each counted with its NUL terminator (the limit of
+ *     the string sort).
+ * Device scratch: parse null_text_len + 24 bytes; format 20 bytes per value, the texts with their terminators, and the
+ * string sort's own: 40 bytes per value, plus up to 20 per value still tied after the first 8 bytes (DESIGN 4.9). */
+enum { ZDWB_NUM_DATETIME = 0, ZDWB_NUM_DECIMAL = 1 };
+
+typedef struct {
+  int32_t kind;              /* ZDWB_NUM_DATETIME or ZDWB_NUM_DECIMAL */
+  int32_t digits;            /* DECIMAL: the scale, 0..18.  DATETIME: ignored by parse; format: fraction digits, 0..6 */
+  const uint8_t* null_text;  /* parse only, host memory: the text of code -1 */
+  uint64_t null_text_len;
+} zdwb_number_opts;
+
+typedef struct {
+  const int64_t* values;     /* device: n numbers; values[entries] is null_text's */
+  const uint8_t* ok;         /* device: n bytes, 1 = the text is in the grammar and its number fits */
+  uint64_t n;                /* entries + 1 */
+} zdwb_parse_out;
+
+int zdwb_parse_numbers(zdwb_ctx* ctx, const zdwb_code_part* dict, const zdwb_number_opts* opts, zdwb_parse_out* out);
+int zdwb_format_numbers(zdwb_ctx* ctx, const int64_t* values, uint64_t n, const zdwb_number_opts* opts,
+                        zdwb_merge_out* out);
 
 /* ---- pinned host staging (used by the host classes and the end-to-end bench) ------------------ */
 void* zdwb_host_alloc(size_t bytes);   /* cudaHostAlloc'd (pinned, usable from every device) memory, NULL on failure */

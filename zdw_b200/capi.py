@@ -19,8 +19,11 @@ EXPORTED_SYMBOLS = [
     "zdwb_abi_version", "zdwb_device_count", "zdwb_ctx_create", "zdwb_ctx_destroy", "zdwb_last_error", "zdwb_ctx_set_stream",
     "zdwb_ctx_set_tuning", "zdwb_ctx_kernel_launches", "zdwb_ctx_kernel_times", "zdwb_encode_block", "zdwb_decode_block", "zdwb_host_alloc",
     "zdwb_host_free", "zdwb_fd_to_device", "zdwb_device_to_fd", "zdwb_decode_columns", "zdwb_merge_codes",
-    "zdwb_render_columns", "zdwb_match_like", "zdwb_find_strings",
+    "zdwb_render_columns", "zdwb_match_like", "zdwb_find_strings", "zdwb_parse_numbers", "zdwb_format_numbers",
 ]
+
+# zdwb_number_opts.kind
+NUM_DATETIME, NUM_DECIMAL = 0, 1
 
 
 class ZdwError(RuntimeError):
@@ -114,6 +117,14 @@ class _FindOut(C.Structure):
     _fields_ = [("rank", C.c_void_p), ("found", C.c_void_p), ("n", C.c_uint64)]
 
 
+class _NumberOpts(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("digits", C.c_int32), ("null_text", C.c_char_p), ("null_text_len", C.c_uint64)]
+
+
+class _ParseOut(C.Structure):
+    _fields_ = [("values", C.c_void_p), ("ok", C.c_void_p), ("n", C.c_uint64)]
+
+
 _lib = None
 
 
@@ -157,6 +168,8 @@ def load_library():
     L.zdwb_render_columns.argtypes = [C.c_void_p, C.POINTER(_Schema), C.POINTER(_CodePart), C.POINTER(_RenderOut)]
     L.zdwb_match_like.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.POINTER(_LikeOpts), C.POINTER(_MatchOut)]
     L.zdwb_find_strings.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.POINTER(_Strings), C.POINTER(_FindOut)]
+    L.zdwb_parse_numbers.argtypes = [C.c_void_p, C.POINTER(_CodePart), C.POINTER(_NumberOpts), C.POINTER(_ParseOut)]
+    L.zdwb_format_numbers.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(_NumberOpts), C.POINTER(_MergeOut)]
     L.zdwb_host_alloc.argtypes = [C.c_size_t]
     L.zdwb_host_alloc.restype = C.c_void_p
     L.zdwb_host_free.argtypes = [C.c_void_p]
@@ -603,3 +616,51 @@ class Context:
         rank, found = _device_tensors(torch, dev, self._copy_stream, [
             (out.rank or 0, (out.n,), "<i8", torch.int64), (out.found or 0, (out.n,), "|u1", torch.uint8)])
         return rank, found.view(torch.bool)
+
+    # ------------------------------------------------------------------ numbers from and to text
+    def parse_numbers(self, dct, entry_off, kind: int, *, digits: int = 0, null_text: bytes = b""):
+        """The number of every entry of a dictionary (zdwb_parse_numbers; include/zdw_b200.h gives the grammars): kind
+        NUM_DATETIME gives microseconds since 1970-01-01, NUM_DECIMAL the number times 10^digits.  Returns (values, ok)
+        CUDA tensors of entries + 1 elements, int64 and bool, the last one for `null_text`, the text of code -1; ok is
+        False (and the value 0) where the text is not in the grammar or its number does not fit.  So `values[codes]` is
+        the answer per cell, code -1 included.  The dictionary is taken as by match_like.  The results are copies,
+        complete when this returns."""
+        import torch
+        part = self._dict_part("parse_numbers", dct, entry_off)
+        null_text = bytes(null_text)
+        o = _NumberOpts(int(kind), int(digits), null_text, len(null_text))
+        out = _ParseOut()
+        rc = self._L.zdwb_parse_numbers(self._h, C.byref(part), C.byref(o), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=self.device)
+        values, ok = _device_tensors(torch, self.device, self._copy_stream, [
+            (out.values or 0, (out.n,), "<i8", torch.int64), (out.ok or 0, (out.n,), "|u1", torch.uint8)])
+        return values, ok.view(torch.bool)
+
+    def format_numbers(self, values, kind: int, *, digits: int = 0) -> MergedCodes:
+        """Strictly increasing numbers (a 1-D int64 CUDA tensor on the context's device, e.g. torch.unique's output, with
+        its final contents) as a dictionary (zdwb_format_numbers): kind NUM_DATETIME writes microseconds since 1970-01-01
+        as "YYYY-MM-DD HH:MM:SS" plus `digits` (0..6) fraction digits, NUM_DECIMAL writes v / 10^digits (0..18) with
+        exactly `digits` fraction digits.  Returns MergedCodes: codes[i] is the code of values[i]'s text in the dense,
+        bytewise sorted dictionary.  The results are copies, complete when this returns."""
+        import torch
+        dev = self.device
+        if not isinstance(values, torch.Tensor) or not values.is_cuda or values.device.index != dev:
+            raise ValueError(f"format_numbers: values must be a tensor on cuda:{dev}")
+        if values.dtype != torch.int64 or values.dim() != 1 or not values.is_contiguous():
+            raise ValueError("format_numbers: values must be a contiguous 1-D int64 tensor")
+        o = _NumberOpts(int(kind), int(digits), None, 0)
+        out = _MergeOut()
+        rc = self._L.zdwb_format_numbers(self._h, C.c_void_p(values.data_ptr() if values.numel() else None), values.numel(),
+                                         C.byref(o), C.byref(out))
+        if rc:
+            raise ZdwError(rc, self.last_error())
+        if self._copy_stream is None:
+            self._copy_stream = torch.cuda.Stream(device=dev)
+        codes, dct, eo = _device_tensors(torch, dev, self._copy_stream, [
+            (out.codes or 0, (out.n,), "<i8", torch.int64),
+            (out.dict or 0, (out.dict_bytes,), "|u1", torch.uint8),
+            (out.entry_off or 0, (out.entries + 1,), "<i8", torch.int64)])
+        return MergedCodes(codes, dct, eo)

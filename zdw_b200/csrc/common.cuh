@@ -818,6 +818,45 @@ __device__ __forceinline__ uint64_t block_exclusive_scan64(uint64_t v, uint64_t*
 #endif  // __CUDACC__
 
 // ---------------------------------------------------------------------------------------------
+// host side of the calls over one dictionary (match.cu, numbers.cu)
+// ---------------------------------------------------------------------------------------------
+// n host bytes into a fresh device buffer (16 bytes of slack), through the pinned staging arena
+inline int upload_host(Ctx* ctx, DevBuf& d, const void* src, size_t n, const char* who) {
+  ZDWB_TRY(d.alloc(ctx, n + 16));
+  if (!n) return ZDWB_OK;
+  void* pinned = stage_take(ctx, n);
+  if (!pinned) {
+    ctx->err = std::string(who) + ": pinned staging allocation failed";
+    return ZDWB_ERR_OOM;
+  }
+  memcpy(pinned, src, n);
+  ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(d.p, pinned, n, cudaMemcpyHostToDevice, ctx->stream));
+  return ZDWB_OK;
+}
+
+// the pointer rules of a dictionary given as a zdwb_code_part (its offsets are checked on the device)
+inline int check_dict(Ctx* ctx, const zdwb_code_part* d, const char* who) {
+  if (!d) {
+    ctx->err = std::string(who) + ": dict is NULL";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (d->entries > 0 && (!d->dict || !d->entry_off)) {
+    ctx->err = std::string(who) + ": entries > 0 with a NULL dict or entry_off";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  return ZDWB_OK;
+}
+
+// the call's one host round trip: a small device struct (fault words, totals) copied out once the stream has finished
+template <typename T>
+int read_back(Ctx* ctx, const void* dev, T* h) {
+  ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->meta_host, dev, sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
+  ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  memcpy(h, ctx->meta_host, sizeof(T));
+  return ZDWB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
 // generic device-wide primitives (scan.cu / sort.cu)
 // ---------------------------------------------------------------------------------------------
 // out[i] = sum(in[0..i)), i in [0,n); total (device pointer, may be null) = sum(in[0..n)).  in == out allowed.

@@ -25,6 +25,8 @@ int render_columns_impl(Ctx* ctx, const zdwb_schema* schema, const zdwb_code_par
                         zdwb_render_out* out);
 int match_like_impl(Ctx* ctx, const zdwb_code_part* dict, const zdwb_like_opts* opts, zdwb_match_out* out);
 int find_strings_impl(Ctx* ctx, const zdwb_code_part* dict, const zdwb_strings* queries, zdwb_find_out* out);
+int parse_numbers_impl(Ctx* ctx, const zdwb_code_part* dict, const zdwb_number_opts* opts, zdwb_parse_out* out);
+int format_numbers_impl(Ctx* ctx, const int64_t* values, uint64_t n, const zdwb_number_opts* opts, zdwb_merge_out* out);
 }  // namespace zdwb
 
 using zdwb::Ctx;
@@ -383,6 +385,50 @@ int zdwb_find_strings(zdwb_ctx* c, const zdwb_code_part* dict, const zdwb_string
     return ZDWB_ERR_OOM;
   } catch (...) {
     c->err = "zdwb_find_strings: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_parse_numbers(zdwb_ctx* c, const zdwb_code_part* dict, const zdwb_number_opts* opts, zdwb_parse_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!opts || !out) {
+    c->err = "zdwb_parse_numbers: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::parse_numbers_impl(c, dict, opts, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_parse_numbers: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_parse_numbers: unexpected C++ exception";
+    return ZDWB_ERR_CUDA;
+  }
+}
+
+int zdwb_format_numbers(zdwb_ctx* c, const int64_t* values, uint64_t n, const zdwb_number_opts* opts, zdwb_merge_out* out) {
+  if (!c) return ZDWB_ERR_BAD_ARG;
+  c->err.clear();
+  if (!opts || !out) {
+    c->err = "zdwb_format_numbers: null argument";
+    return ZDWB_ERR_BAD_ARG;
+  }
+  if (cudaSetDevice(c->device) != cudaSuccess) {
+    c->err = "cudaSetDevice failed";
+    return ZDWB_ERR_NO_DEVICE;
+  }
+  try {
+    return zdwb::format_numbers_impl(c, values, n, opts, out);
+  } catch (const std::bad_alloc&) {
+    c->err = "zdwb_format_numbers: out of host memory";
+    return ZDWB_ERR_OOM;
+  } catch (...) {
+    c->err = "zdwb_format_numbers: unexpected C++ exception";
     return ZDWB_ERR_CUDA;
   }
 }

@@ -168,39 +168,6 @@ unsigned grid_for(const Ctx* ctx, unsigned long long threads) {
   return (unsigned)std::max<unsigned long long>(1, std::min(want, cap));
 }
 
-int match_upload(Ctx* ctx, DevBuf& d, const void* src, size_t n, const char* who) {
-  ZDWB_TRY(d.alloc(ctx, n + 16));
-  if (!n) return ZDWB_OK;
-  void* pinned = stage_take(ctx, n);
-  if (!pinned) {
-    ctx->err = std::string(who) + ": pinned staging allocation failed";
-    return ZDWB_ERR_OOM;
-  }
-  memcpy(pinned, src, n);
-  ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(d.p, pinned, n, cudaMemcpyHostToDevice, ctx->stream));
-  return ZDWB_OK;
-}
-
-int check_dict(Ctx* ctx, const zdwb_code_part* d, const char* who) {
-  if (!d) {
-    ctx->err = std::string(who) + ": dict is NULL";
-    return ZDWB_ERR_BAD_ARG;
-  }
-  if (d->entries > 0 && (!d->dict || !d->entry_off)) {
-    ctx->err = std::string(who) + ": entries > 0 with a NULL dict or entry_off";
-    return ZDWB_ERR_BAD_ARG;
-  }
-  return ZDWB_OK;
-}
-
-template <typename T>
-int read_back(Ctx* ctx, const void* dev, T* h) {
-  ZDWB_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->meta_host, dev, sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
-  ZDWB_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  memcpy(h, ctx->meta_host, sizeof(T));
-  return ZDWB_OK;
-}
-
 }  // namespace
 
 int match_like_impl(Ctx* ctx, const zdwb_code_part* d, const zdwb_like_opts* o, zdwb_match_out* out) {
@@ -243,9 +210,9 @@ int match_like_impl(Ctx* ctx, const zdwb_code_part* d, const zdwb_like_opts* o, 
   ZDWB_TRY(call_begin(ctx));
   const unsigned long long E = d->entries;
   DevBuf d_el, d_seg, d_null, d_bad;
-  ZDWB_TRY(match_upload(ctx, d_el, el.data(), el.size() * 2, who));
-  ZDWB_TRY(match_upload(ctx, d_seg, seg.data(), seg.size() * 4, who));
-  ZDWB_TRY(match_upload(ctx, d_null, o->null_text, o->null_text_len, who));
+  ZDWB_TRY(upload_host(ctx, d_el, el.data(), el.size() * 2, who));
+  ZDWB_TRY(upload_host(ctx, d_seg, seg.data(), seg.size() * 4, who));
+  ZDWB_TRY(upload_host(ctx, d_null, o->null_text, o->null_text_len, who));
   ZDWB_TRY(d_bad.alloc(ctx, 8));
   ZDWB_CUDA_TRY(ctx, cudaMemsetAsync(d_bad.p, 0xff, 8, ctx->stream));
   uint8_t* flags;
